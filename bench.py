@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- headline benchmark of the render path (BASELINE.json: Mrays/s and frame time).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4|c4b|c2|...] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--config c4|c4b|c2|...] [--impl ours|reference] [--dump-outputs DIR]
 
 A step = one frame of the workload.  The workload is the frame BASELINE.json's metric and north star are quoted on
 (configs[3]): the great grand stellated 120-cell {5/2,3,3} as a CompositeScene over the reference's own k-d tree
@@ -312,14 +312,56 @@ class Workload:
         self.ds.set_camera(self.cam_o, self.cam_a)
         self.ds.render(self.fmt, self.pageable)
 
+    def _pixels(self, packed):
+        return np.asarray(packed, np.uint8).reshape(self.h, self.fmt.pitch)[:, :self.w * 3].reshape(self.h, self.w, 3).copy()
+
+    def device_frame(self):
+        """rank 0: the frame step_device left in GPU memory, as (height, width, 3) uint8; None on the other ranks"""
+        from ntracer_b200.dist import PeerFrameRenderer
+        if self.rank != 0:
+            return None
+        if isinstance(self.dr, PeerFrameRenderer):
+            buf = np.zeros(self.fmt.pitch * self.h, np.uint8)
+            self.dr.frame.download(self.fmt, buf, self.dr.stream.cuda_stream)
+            self.dr.stream.synchronize()
+            return self._pixels(buf)
+        frame = self.dr.frame_on_device()
+        self.dr.stream.synchronize()
+        return self._pixels(frame.cpu().numpy())
+
+    def e2e_frame(self):
+        """rank 0: the frame step_e2e copied into host memory; None on the other ranks"""
+        if self.rank != 0:
+            return None
+        return self._pixels(self.host_frame.numpy() if self.world == 1 else self.dr.host.numpy())
+
     def close(self):
         if hasattr(self.dr, 'close'):
             self.dr.close()
         self.ds.close()
 
 
-def timed(wl, steps, warmup, flush, barrier):
-    """-> (device ms per step, e2e ms per step, launches), each the MAX over ranks of the per-rank totals"""
+# --dump-outputs: frames with more pixels than this are written as a fixed, seeded sample of their pixels (every run picks
+# the same pixels), so that the dump of a 4K headline frame and its secondaries stays far below 64 MB
+DUMP_SAMPLE_PIXELS = 1 << 19
+DUMP_SEED = 20240601
+
+
+def dump_outputs(directory, frames):
+    """frames: {name: (height, width, 3) uint8} -> directory/<name>.npy in float32, 0..255: the whole frame
+    (height, width, 3), or [DUMP_SAMPLE_PIXELS, 3] pixels at the seeded sample of flat pixel indices, in increasing order."""
+    os.makedirs(directory, exist_ok=True)
+    for name, px in frames.items():
+        h, w, _ = px.shape
+        if h * w > DUMP_SAMPLE_PIXELS:
+            idx = np.sort(np.random.default_rng(DUMP_SEED).choice(h * w, DUMP_SAMPLE_PIXELS, replace=False))
+            px = px.reshape(h * w, 3)[idx]
+        np.save(os.path.join(directory, name + '.npy'), px.astype(np.float32))
+
+
+def timed(wl, steps, warmup, flush, barrier, keep=False):
+    """-> (device ms per step, e2e ms per step, launches), each the MAX over ranks of the per-rank totals.
+    keep: also store the frames of the last device step and the last e2e step in wl.kept (rank 0; outside the timing)"""
     import torch
     import torch.distributed as dist
     for _ in range(warmup):
@@ -333,6 +375,8 @@ def timed(wl, steps, warmup, flush, barrier):
         barrier()
         dev_ms.append(wl.step_device())
     barrier()
+    if keep:
+        wl.kept = {'frame': wl.device_frame()}
     e2e_s = []
     for _ in range(steps):
         flush.zero_()
@@ -341,6 +385,8 @@ def timed(wl, steps, warmup, flush, barrier):
         wl.step_e2e()
         e2e_s.append(time.perf_counter() - t)
     barrier()
+    if keep:
+        wl.kept['frame_e2e'] = wl.e2e_frame()
     launches = wl.ds.launch_count() - launches0
     wl.pageable_ms = None
     if wl.world == 1:                   # BlockingRenderer.render is handed a bytearray: the same frames into pageable memory
@@ -371,7 +417,15 @@ def main():
     ap.add_argument('--no-secondary', action='store_true', help='skip the secondary workloads (c4b, c2) reported beside the headline one')
     ap.add_argument('--stream-frames', type=int, default=160,
                     help='frames of the rotating-camera loop (polytope.py --benchmark); 0 = skip that leg')
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help='after the timed steps, write the frames of the last device step and the last e2e step of every timed '
+                         'workload to DIR/<config>_frame.npy and DIR/<config>_frame_e2e.npy (float32; frames over %d pixels as '
+                         'a fixed seeded sample of their pixels)' % DUMP_SAMPLE_PIXELS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes the frames of --impl ours')
     args.warmup = max(args.warmup, 3)
 
     rank = int(os.environ.get('RANK', '0'))
@@ -444,22 +498,27 @@ def main():
     sampler = ClockSampler(local_rank) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms_per_step, e2e_ms, launches, dev_ms = timed(wl, args.steps, args.warmup, flush, barrier)
+    keep = bool(args.dump_outputs)
+    ms_per_step, e2e_ms, launches, dev_ms = timed(wl, args.steps, args.warmup, flush, barrier, keep)
     clocks = sampler.stop() if sampler else None
+    outputs = {'%s_%s' % (args.config, k): v for k, v in wl.kept.items()} if keep else {}
 
-    # the secondary workloads, measured the same way with fewer steps: BASELINE.json spells config 4's symbol {5/2,5,3}
+    # the secondary workloads, measured the same way: BASELINE.json spells config 4's symbol {5/2,5,3}
     # (c4b) while naming the {5/2,3,3} polytope (c4, the headline); c2 is the round-1 headline
     secondary = {}
     if not args.no_secondary and args.config == 'c4':
         for name in ('c4b', 'c2'):
             w2 = Workload(name, rank, local_rank, world)
-            k = max(3, min(args.steps, 10))
-            d2, e2, l2, _ = timed(w2, k, 3, flush, barrier)
-            secondary[name] = {'workload': w2.desc, 'width': w2.w, 'height': w2.h, 'rays_per_frame': w2.rays, 'steps': k,
+            d2, e2, l2, _ = timed(w2, args.steps, 3, flush, barrier, keep)
+            if keep:
+                outputs.update(('%s_%s' % (name, kk), v) for kk, v in w2.kept.items())
+            secondary[name] = {'workload': w2.desc, 'width': w2.w, 'height': w2.h, 'rays_per_frame': w2.rays, 'steps': args.steps,
                                'ms_per_step': d2, 'value': w2.rays / (d2 * 1e-3) / 1e6, 'unit': 'Mrays/s',
                                'e2e_ms_per_step': e2, 'e2e_value': w2.rays / (e2 * 1e-3) / 1e6, 'frames_per_s': 1e3 / d2,
                                'gpu_launches': l2}
             w2.close()
+    if keep and rank == 0:
+        dump_outputs(args.dump_outputs, outputs)
 
     ds = wl.ds
 

@@ -42,6 +42,9 @@ torch.tensor = lambda *a, **k: _real_tensor(*a, **{kk: vv for kk, vv in k.items(
 torch.Tensor.pin_memory = lambda self: self
 
 from ntracer_b200 import backend, dist as ntd
+def _fill(buf):                                      # a fixed pattern of bytes stands in for the frame
+    b = np.frombuffer(buf, np.uint8)
+    b[:] = np.arange(b.size) %% 251
 class FakeScene:
     def __init__(self, sc, device=-1): self.sc, self.n, self.open = sc, 0, {}
     def render_float(self, w, h): self.w, self.h = w, h; return np.zeros((h, w, 3), np.float32)
@@ -50,7 +53,7 @@ class FakeScene:
                 'simplex_tests': 7, 'solid_tests': 0, 'shaded_hits': 3, 'queue_overflows': 0}
     def set_camera(self, o, a): pass
     def set_instrumented(self, on): pass
-    def render(self, fmt, dest=None): self.n += 1; return dest
+    def render(self, fmt, dest=None): self.n += 1; _fill(dest); return dest
     def render_device(self, *a, **k): self.n += 1
     def render_begin(self, fmt, dest):
         self.n += 1
@@ -62,7 +65,9 @@ class FakeScene:
 backend.DeviceScene = FakeScene
 backend.measure_fp32_peak = lambda dev=0: 64.5
 class FakeDR:
-    def __init__(self, ds, fmt, group=None): self.ds, self.stream = ds, _Stream()
+    def __init__(self, ds, fmt, group=None):
+        self.ds, self.stream = ds, _Stream()
+        self.frame = types.SimpleNamespace(download=lambda fmt, buf, stream=0: _fill(buf))
     def render_strip(self): self.ds.render_device()
     def render(self): self.ds.render_device()
     def gather(self): pass
@@ -134,6 +139,32 @@ def test_watchdog_prints_the_line_when_a_late_leg_hangs():
     for k in ('value', 'e2e', 'roofline', 'clocks', 'gpu_launches'):
         assert k in line
     assert out.returncode == 0
+
+
+def test_dump_outputs_writes_the_frames_of_the_last_timed_steps(tmp_path):
+    line, out = run_stubbed(['--config', 'c1', '--steps', '2', '--no-cpu-baseline', '--stream-frames', '0',
+                             '--dump-outputs', str(tmp_path / 'out')])
+    assert line['steps'] == 2 and line['gpu_launches'] == 2 * 2
+    w, h = 640, 480
+    want = (np.arange(h * w * 3) % 251).reshape(h, w, 3).astype(np.float32)
+    assert sorted(os.listdir(tmp_path / 'out')) == ['c1_frame.npy', 'c1_frame_e2e.npy']
+    for name in ('c1_frame', 'c1_frame_e2e'):
+        got = np.load(tmp_path / 'out' / (name + '.npy'))
+        assert got.dtype == np.float32 and np.array_equal(got, want), name
+
+
+def test_dump_outputs_samples_big_frames_the_same_pixels_every_time(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    big = np.random.default_rng(0).integers(0, 256, (2160, 3840, 3), dtype=np.uint8)
+    bench.dump_outputs(str(tmp_path / 'a'), {'big': big, 'small': big[:90, :160]})
+    bench.dump_outputs(str(tmp_path / 'b'), {'big': big})
+    a = np.load(tmp_path / 'a' / 'big.npy')
+    assert a.dtype == np.float32 and a.shape == (bench.DUMP_SAMPLE_PIXELS, 3)
+    assert np.array_equal(a, np.load(tmp_path / 'b' / 'big.npy'))
+    assert np.array_equal(np.load(tmp_path / 'a' / 'small.npy'), big[:90, :160].astype(np.float32))
+    # the default workload dumps six 4K-sized frames (c4, c4b, c2; device and e2e path each)
+    assert 6 * os.path.getsize(tmp_path / 'a' / 'big.npy') <= 64e6
 
 
 def test_reference_arm_line():

@@ -1,8 +1,8 @@
 """ntracer_b200.pygame_render (the reference's lib/ntracer/pygame_render.py on this backend) without pygame: a small
 stand-in module provides what the front end touches (Surface queries, the event queue, the quit hook).  The channel
-lists are compared with the reference's own channels_from_surface run on the same stand-in (when /root/reference is
-here) and with values recorded from it; the renderer is driven end to end on the emulated device of
-tests/test_facade_emulated.py (CPU tier: Python side of the C ABI)."""
+lists are compared with values recorded from the reference's own channels_from_surface and, when NTRACER_REFERENCE
+names the reference's source tree, with that function run on the same stand-in; the renderer is driven end to end on
+the emulated device of tests/test_facade_emulated.py (CPU tier: Python side of the C ABI)."""
 import importlib
 import os
 import sys
@@ -12,7 +12,7 @@ import types
 import numpy as np
 import pytest
 
-REF = '/root/reference/lib/ntracer/pygame_render.py'
+REF = os.path.join(os.environ['NTRACER_REFERENCE'], 'lib', 'ntracer', 'pygame_render.py') if os.environ.get('NTRACER_REFERENCE') else None
 
 
 class FakeSurface:
@@ -78,7 +78,7 @@ def _tuples(channels):
 def test_channels_from_surface(fake_pygame):
     pg, mod = fake_pygame
     ref_fn = None
-    if os.path.exists(REF):
+    if REF and os.path.exists(REF):
         # the reference's own function, executed on the same stand-in (its `ntracer.render.Channel` replaced by a recorder)
         class Chan:
             def __init__(self, bit_size, f_r, f_g, f_b, f_c=0):
