@@ -119,7 +119,7 @@ typedef struct ntr_image_format {
 
 /* Ray / work counters of the last render (SURVEY.md section 8d "ray counting"). */
 typedef struct ntr_counters {
-    uint64_t primary_rays;          /* W*H */
+    uint64_t primary_rays;          /* W*H, times s*s for a supersampling factor s (ntr_scene_set_supersampling) */
     uint64_t reflection_rays;       /* recursive ray_color calls, src/tracer.hpp:1843 */
     uint64_t shadow_rays;           /* light_reaches calls, src/tracer.hpp:1787,1811 */
     uint64_t node_steps;            /* kd_branch visits (only filled by instrumented renders) */
@@ -152,6 +152,20 @@ NTR_API int ntr_scene_set_camera(ntr_scene *scene, const float *origin, const fl
  * background, ambient, lights) without touching geometry.  Replaces the set_* mutators
  * (src/ntracer_body.hpp:833-933). */
 NTR_API int ntr_scene_set_params(ntr_scene *scene, const ntr_scene_desc *desc);
+/* Supersampled anti-aliasing (no counterpart in the reference, which traces one ray through the corner of every pixel).
+ * factor s in 1..NTR_MAX_SUPERSAMPLING, default 1; anything else -> NTR_ERR_VALUE.  Host state like the camera: read when
+ * a frame is enqueued (ntr_render_begin captures it with the camera).  s = 1 is the plain renderer, byte for byte.
+ * With s > 1 the float colour of output pixel (x, y) of a W x H frame is the box-filtered mean of the s x s pixels
+ * (s*x + i, s*y + j) of the sW x sH view, summed j-major, i-minor: each sample's colour is computed exactly as
+ * ntr_render_float(sW, sH) computes that pixel, with every contribution weighted by 1/(s*s), and added to the pixel's sum;
+ * the sum is then packed as usual (the mean is taken before clamping).  For s in {2, 4, 8} and frames without reflections
+ * the result is bit-identical to that mean of the big view.  ntr_render, ntr_render_device, ntr_render_begin/end,
+ * ntr_render_float, ntr_calculate_color and ntr_group_render* honour it; ntr_primary_hit_ids, ntr_trace_rays* and
+ * ntr_occludes_rays are per-ray hooks and ignore it.  Counters: primary_rays = s*s per pixel, the others are those of the
+ * big view.  The wavefront queues of reflective scenes hold up to s*s times the bounces of a plain frame: their memory
+ * grows with s*s (see README). */
+#define NTR_MAX_SUPERSAMPLING 8
+NTR_API int ntr_scene_set_supersampling(ntr_scene *scene, int factor);
 
 /* ---- the hot path ---------------------------------------------------------------------------- */
 /* Renders one frame into a HOST buffer: replaces worker_draw + process_pixel for all tiles
@@ -223,6 +237,8 @@ NTR_API void ntr_group_destroy(ntr_group *group);
 NTR_API int ntr_group_size(ntr_group *group);
 NTR_API int ntr_group_set_camera(ntr_group *group, const float *origin, const float *axes);
 NTR_API int ntr_group_set_params(ntr_group *group, const ntr_scene_desc *desc);
+/* ntr_scene_set_supersampling for every device of the group. */
+NTR_API int ntr_group_set_supersampling(ntr_group *group, int factor);
 /* ntr_render over the group: host destination, same contract (NTR_ERR_ABORTED after ntr_group_abort). */
 NTR_API int ntr_group_render(ntr_group *group, const ntr_image_format *fmt, void *dst, size_t dst_len);
 /* The same frame left in device memory: *dev_frame_out receives the frame buffer on the first device (pitch*height

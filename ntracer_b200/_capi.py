@@ -16,6 +16,7 @@ REF_SIMPLEX, REF_BATCH, REF_SOLID = 0, 1, 2
 SCENE_BOX, SCENE_COMPOSITE = 0, 1
 
 NTR_OK = 0
+NTR_MAX_SUPERSAMPLING = 8
 NTR_ERR_VALUE, NTR_ERR_MEMORY, NTR_ERR_RUNTIME, NTR_ERR_NO_DEVICE, NTR_ERR_ABORTED = -1, -2, -3, -4, -5
 
 
@@ -197,6 +198,7 @@ def load():
         'ntr_scene_destroy': (None, [vp]),
         'ntr_scene_set_camera': (C.c_int, [vp, vp, vp]),
         'ntr_scene_set_params': (C.c_int, [vp, C.POINTER(SceneDesc)]),
+        'ntr_scene_set_supersampling': (C.c_int, [vp, i32]),
         'ntr_render': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t]),
         'ntr_render_device': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t, vp, i32, i32, i32]),
         'ntr_render_begin': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t, C.POINTER(C.c_uint64)]),
@@ -225,6 +227,7 @@ def load():
         'ntr_group_size': (C.c_int, [vp]),
         'ntr_group_set_camera': (C.c_int, [vp, vp, vp]),
         'ntr_group_set_params': (C.c_int, [vp, C.POINTER(SceneDesc)]),
+        'ntr_group_set_supersampling': (C.c_int, [vp, i32]),
         'ntr_group_render': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t]),
         'ntr_group_render_device': (C.c_int, [vp, C.POINTER(ImageFormat), C.POINTER(vp)]),
         'ntr_group_abort': (C.c_int, [vp]),
@@ -248,12 +251,13 @@ def load():
 
 EXPORTED_SYMBOLS = (
     'ntr_abi_version', 'ntr_last_error', 'ntr_device_count', 'ntr_scene_create', 'ntr_scene_destroy',
-    'ntr_scene_set_camera', 'ntr_scene_set_params', 'ntr_render', 'ntr_render_device', 'ntr_render_begin',
+    'ntr_scene_set_camera', 'ntr_scene_set_params', 'ntr_scene_set_supersampling', 'ntr_render', 'ntr_render_device', 'ntr_render_begin',
     'ntr_render_end', 'ntr_render_float',
     'ntr_calculate_color', 'ntr_primary_hit_ids', 'ntr_trace_rays', 'ntr_trace_rays_hits', 'ntr_occludes_rays', 'ntr_abort',
     'ntr_get_counters', 'ntr_set_instrumented', 'ntr_last_kernel_ms', 'ntr_launch_count',
     'ntr_measure_fp32_peak', 'ntr_simplex_from_points', 'ntr_build_kdtree', 'ntr_build_kdtree_culled', 'ntr_free', 'ntr_group_items',
     'ntr_group_create', 'ntr_group_destroy', 'ntr_group_size', 'ntr_group_set_camera', 'ntr_group_set_params',
+    'ntr_group_set_supersampling',
     'ntr_group_render', 'ntr_group_render_device', 'ntr_group_abort', 'ntr_group_get_counters',
     'ntr_group_last_kernel_ms', 'ntr_group_launch_count',
     'ntr_frame_alloc', 'ntr_frame_free', 'ntr_frame_export', 'ntr_frame_import', 'ntr_frame_release',

@@ -26,6 +26,7 @@ class DeviceScene:
         self.kind = int(scene['kind'])
         self._scene = scene
         self._open = {}
+        self.supersampling = 1
         desc, keep = _capi.make_desc(scene)
         _capi.check(self._lib.ntr_scene_create(C.byref(desc), device, C.byref(self._h)))
         if 'cam_origin' in scene and 'cam_axes' in scene:
@@ -62,6 +63,11 @@ class DeviceScene:
 
     def set_instrumented(self, on):
         _capi.check(self._lib.ntr_set_instrumented(self._h, int(bool(on))))
+
+    def set_supersampling(self, factor):
+        """Anti-aliasing: every pixel becomes the mean of factor x factor samples (1..8; 1 = one ray per pixel)."""
+        _capi.check(self._lib.ntr_scene_set_supersampling(self._h, int(factor)))
+        self.supersampling = int(factor)
 
     # ---- the hot path ----
     def render(self, fmt, dest=None):
@@ -189,6 +195,7 @@ class DeviceGroup:
         devs = None if devices is None else (C.c_int * len(devices))(*[int(d) for d in devices])
         _capi.check(self._lib.ntr_group_create(C.byref(desc), len(devices) if devices is not None else int(n), devs, C.byref(self._h)))
         self.size = int(self._lib.ntr_group_size(self._h))
+        self.supersampling = 1
         if 'cam_origin' in scene and 'cam_axes' in scene:
             self.set_camera(scene['cam_origin'], scene['cam_axes'])
 
@@ -213,6 +220,10 @@ class DeviceGroup:
     def set_params(self, scene):
         desc, keep = _capi.make_desc(scene)
         _capi.check(self._lib.ntr_group_set_params(self._h, C.byref(desc)))
+
+    def set_supersampling(self, factor):
+        _capi.check(self._lib.ntr_group_set_supersampling(self._h, int(factor)))
+        self.supersampling = int(factor)
 
     def render(self, fmt, dest=None):
         need = fmt.pitch * fmt.height

@@ -150,6 +150,7 @@ struct ntr_scene {
     int n_pass_ev = 0;
     bool pass_timing = false;
     ntr_counters counters{};
+    int ss = 1;                         // supersampling factor (ntr_scene_set_supersampling), read when a frame is enqueued
     // pageable destinations (what BlockingRenderer.render is handed: a bytearray): frames cross PCIe into this pinned
     // staging buffer in row chunks, and the host copies chunk k into the caller's buffer while chunk k+1 is in flight
     unsigned char *h_stage = nullptr; size_t h_stage_cap = 0;
@@ -157,7 +158,7 @@ struct ntr_scene {
     uint32_t *h_ctl = nullptr;              // pinned read-back of the control block and the counters (frame_readback)
     unsigned long long *h_cnt = nullptr;
     uint64_t launches = 0;
-    int grid_blocks[16] = {};
+    int grid_blocks[32] = {};          // per variant flags (NTR_F_SS included)
     // NTR_F_WIDE builds (96 registers, 5 CTAs per SM): for frames sharded over 4 or more GPUs, whose passes all end in a few
     // long rays (measured, config 4: 1/4 share 20.9 -> 19.9 ms, 1/8 share 15.2 -> 14.4 ms; 1/2 share and whole frames lose
     // 2..12 %).  Picking the build per pass from pass times measured on the second and third frame of a view gained another
@@ -357,7 +358,13 @@ struct RenderTarget {
     float *dists = nullptr;
 };
 
+// Supersampling factor of a frame: the hit-id hook traces one ray per pixel whatever the scene's factor
+int frame_ss(const ntr_scene *sc, int out_mode) { return out_mode == NTR_OUT_IDS ? 1 : sc->ss; }
+
 // Enqueues every kernel of one frame on `st`.  view = (width,height), window = (x0,y0,w,h).
+// A supersampled frame (factor ss > 1) traces the ss-times-larger view: FrameDev describes that view, while the window,
+// the tile grid and every output stay in output pixels (slabs, tile-row interleaving, compact strips and the 1x1 window of
+// ntr_calculate_color work unchanged).
 int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0, int y0, int win_w, int win_h,
                   const ntr_image_format *fmt, const RenderTarget &tgt, int tile_row_first, int tile_row_step,
                   int compact, bool *used_passes) {
@@ -367,10 +374,12 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         CUDA_TRY(cudaStreamWaitEvent(st, sc->frame_done[sc->ctl_slot], 0));
     FrameDev f;
     memset(&f, 0, sizeof f);
-    f.width = width; f.height = height;
+    const int ss = frame_ss(sc, tgt.out_mode);
+    f.ss = ss;
+    f.width = width * ss; f.height = height * ss;
     // flat_origin_ray_source::set_params (tracer.hpp:65-69)
-    f.half_w = (float)width / 2.0f;
-    f.half_h = (float)height / 2.0f;
+    f.half_w = (float)f.width / 2.0f;
+    f.half_h = (float)f.height / 2.0f;
     f.fovI = tanf(sc->dev.fov / 2) / f.half_w;
     f.x0 = x0; f.y0 = y0; f.win_w = win_w; f.win_h = win_h;
     f.tiles_x = (win_w + NTR_TILE - 1) / NTR_TILE;
@@ -403,9 +412,12 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         f.out_mode = NTR_OUT_ACCUM;
     }
     if (passes) {
-        // each pass can emit at most (1 + transparent layers) rays per input ray; start with 2 rays per pixel
+        // each pass can emit at most (1 + transparent layers) rays per input ray; start with 2 rays per traced sample
+        // (ss*ss per pixel; capped at 2^26 records -- 4 GB per queue in 4 dimensions -- unless a plain frame needs more)
         // and let the overflow check regrow (ntr_counters.queue_overflows)
-        const uint64_t want = sc->queue_init ? sc->queue_init : std::max<uint64_t>((uint64_t)npix * 2, 1u << 16);
+        const uint64_t plain = (uint64_t)npix * 2;
+        const uint64_t want = sc->queue_init ? sc->queue_init
+                                             : std::max<uint64_t>(std::min<uint64_t>(plain * ss * ss, std::max<uint64_t>(plain, 1ull << 26)), 1u << 16);
         if (sc->queue_capacity < want) {
             int rc = ensure_queues(sc, (uint32_t)std::min<uint64_t>(want, 0x7FFFFFFFu));
             if (rc) return rc;
@@ -414,7 +426,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
 
     // ---- tile schedule: reuse the order measured on the previous frame of the same geometry ----
     const size_t n_tiles = (size_t)(f.out_rows ? (compact ? f.out_rows / NTR_TILE : (f.tiles_y - tile_row_first + f.tile_row_step - 1) / f.tile_row_step) : 0) * f.tiles_x;
-    const long long key = ((((long long)win_w * 65536 + win_h) * 64 + tile_row_first) * 64 + f.tile_row_step) * 4 + x0 % 2 * 2 + y0 % 2;
+    const long long key = (((((long long)win_w * 65536 + win_h) * 64 + tile_row_first) * 64 + f.tile_row_step) * 4 + x0 % 2 * 2 + y0 % 2) * 8 + (ss - 1);
     // measured: the cost-sorted schedule pays when the frame is sharded over GPUs (8 GPUs, config 2: strip render
     // 0.258 -> 0.203 ms) -- each rank then has only ~2 blocks per warp and the tail matters -- but costs ~8 % on a
     // whole frame on one GPU (loss of row-major locality + the cost bookkeeping), so it is used for sharded renders --
@@ -471,7 +483,8 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     const bool wide_ok = sc->wide_mode != 0 && composite && passes && (flags & NTR_F_GENERAL) && sc->dev.dim <= 5 && sc->max_leaf >= 256;
     const uint32_t wide_now = wide_ok && (sc->wide_mode == 1 || f.tile_row_step >= 4) ? 0xFFFFFFFFu : 0u;
     auto wide_for = [&](int pass) { return (wide_now >> pass) & 1u ? (int)NTR_F_WIDE : 0; };
-    const int pflags = primary_flags | wide_for(0);
+    // a supersampled primary pass runs the per-lane, non-wide NTR_F_SS build whatever NTR_WARP / NTR_WIDE say (kernels.cuh)
+    const int pflags = ss > 1 ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_SS : primary_flags | wide_for(0);
     const KernelSet *ks = sc->kset(pflags);
     const int grid = grid_for(sc, pflags);
     const uint32_t rec4 = 2 + 2 * ((sc->dev.dim + 3) / 4);
@@ -638,12 +651,13 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
     }
     if (sc->h_abort[sc->abort_idx]) return fail(NTR_ERR_ABORTED, "render aborted");
     const uint64_t overflows = sc->counters.queue_overflows;
-    sc->counters.primary_rays = (uint64_t)j.win_w * j.win_h;
+    const uint64_t spp = (uint64_t)frame_ss(sc, j.tgt.out_mode) * frame_ss(sc, j.tgt.out_mode);
+    sc->counters.primary_rays = (uint64_t)j.win_w * j.win_h * spp;
     if (j.trs > 1) {
         const int tiles_y = (j.win_h + NTR_TILE - 1) / NTR_TILE;
         uint64_t rows = 0;
         for (int ty = j.trf; ty < tiles_y; ty += j.trs) rows += std::min(NTR_TILE, j.win_h - ty * NTR_TILE);
-        sc->counters.primary_rays = rows * (uint64_t)j.win_w;
+        sc->counters.primary_rays = rows * (uint64_t)j.win_w * spp;
     }
     sc->counters.reflection_rays = h_cnt[1]; sc->counters.shadow_rays = h_cnt[2]; sc->counters.node_steps = h_cnt[3];
     sc->counters.simplex_tests = h_cnt[4]; sc->counters.solid_tests = h_cnt[5]; sc->counters.shaded_hits = h_cnt[6];
@@ -771,7 +785,7 @@ int run_frame_slabs(ntr_scene *sc, const ntr_image_format *fmt, unsigned char *d
     const uint64_t overflows = sc->counters.queue_overflows;
     sc->counters = ntr_counters{};
     sc->counters.queue_overflows = overflows;
-    sc->counters.primary_rays = (uint64_t)fmt->width * fmt->height;
+    sc->counters.primary_rays = (uint64_t)fmt->width * fmt->height * sc->ss * sc->ss;
     for (int i = 0; i < S; ++i) {
         sc->counters.reflection_rays += h_cnt[i * 8 + 1]; sc->counters.shadow_rays += h_cnt[i * 8 + 2];
         sc->counters.shaded_hits += h_cnt[i * 8 + 6]; sc->counters.truncated_hit_lists += h_cnt[i * 8 + 7];
@@ -1055,6 +1069,14 @@ NTR_API int ntr_scene_set_camera(ntr_scene *sc, const float *origin, const float
     return NTR_OK;
 }
 
+NTR_API int ntr_scene_set_supersampling(ntr_scene *sc, int factor) {
+    if (!sc) return fail(NTR_ERR_VALUE, "scene is NULL");
+    if (factor < 1 || factor > NTR_MAX_SUPERSAMPLING) return fail(NTR_ERR_VALUE, "the supersampling factor must be between 1 and %d", NTR_MAX_SUPERSAMPLING);
+    if (sc->busy) return fail(NTR_ERR_RUNTIME, "the scene is locked while rendering");
+    sc->ss = factor;
+    return NTR_OK;
+}
+
 NTR_API int ntr_scene_set_params(ntr_scene *sc, const ntr_scene_desc *desc) {
     if (!sc || !desc) return fail(NTR_ERR_VALUE, "NULL argument");
     if (sc->busy) return fail(NTR_ERR_RUNTIME, "the scene is locked while rendering");
@@ -1098,7 +1120,7 @@ NTR_API int ntr_render_device(ntr_scene *sc, const ntr_image_format *fmt, void *
         CUDA_TRY(cudaEventRecord(sc->ev1, st));
         sc->timing_valid = true;
         sc->counters = ntr_counters{};
-        sc->counters.primary_rays = (uint64_t)fmt->width * fmt->height;
+        sc->counters.primary_rays = (uint64_t)fmt->width * fmt->height * sc->ss * sc->ss;
         return NTR_OK;
     }
     // wavefront passes: synchronous on `st` (the queue-overflow check needs the counters back)
@@ -1200,7 +1222,7 @@ NTR_API int ntr_render_begin(ntr_scene *sc, const ntr_image_format *fmt, void *d
         cudaEventRecord(sc->ev1, sc->stream);
         sc->timing_valid = rc == NTR_OK;
         sc->counters = ntr_counters{};
-        sc->counters.primary_rays = (uint64_t)fmt->width * fmt->height;
+        sc->counters.primary_rays = (uint64_t)fmt->width * fmt->height * sc->ss * sc->ss;
     } else {
         // wavefront passes need their counters back between passes: traced synchronously, only the copy overlaps
         rc = run_frame_sync(sc, fmt->width, fmt->height, 0, 0, fmt->width, fmt->height, fmt, tgt, 0, 1, 0, sc->stream);
@@ -1614,6 +1636,12 @@ NTR_API int ntr_group_set_camera(ntr_group *g, const float *origin, const float 
 NTR_API int ntr_group_set_params(ntr_group *g, const ntr_scene_desc *desc) {
     if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
     for (ntr_scene *sc : g->sc) { const int rc = ntr_scene_set_params(sc, desc); if (rc) return rc; }
+    return NTR_OK;
+}
+
+NTR_API int ntr_group_set_supersampling(ntr_group *g, int factor) {
+    if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
+    for (ntr_scene *sc : g->sc) { const int rc = ntr_scene_set_supersampling(sc, factor); if (rc) return rc; }
     return NTR_OK;
 }
 

@@ -34,8 +34,10 @@ enum : int {
     NTR_F_COUNT = 2,        // instrumented: node/primitive counters (never used for timing)
     NTR_F_WARP = 4,         // render_pass_kernel only: the warp-synchronous per-ray path (trace_warp.cuh), chosen for scenes
                             // with big leaves; otherwise every lane traces for itself (trace_core.cuh)
-    NTR_F_WIDE = 8          // render_pass_kernel only, general variant in 3..5 dimensions: 96 registers / 5 CTAs per SM instead of
+    NTR_F_WIDE = 8,         // render_pass_kernel only, general variant in 3..5 dimensions: 96 registers / 5 CTAs per SM instead of
                             // 64 / 8 -- no spills, fewer warps: the build for passes that end in a few long rays (kernels.cuh)
+    NTR_F_SS = 16           // render_pass_kernel only, per-lane form: the primary pass of a supersampled frame (FrameDev::ss > 1),
+                            // every lane traces the ss x ss samples of its pixel one after the other (trace_core.cuh: ss_pixel_color)
 };
 
 struct SceneDev {
@@ -96,6 +98,8 @@ struct FrameDev {
     int32_t *ids;                   // NTR_OUT_IDS
     float *dists;
     FormatDev fmt;
+    int ss;                         // supersampling factor: width / height / half_w / half_h / fovI describe the ss-times-larger
+                                    // view, the window and tile grid stay in output pixels (1: plain frame)
 };
 
 // One deferred ray of the wavefront (a reflection bounce): 16-byte aligned record.

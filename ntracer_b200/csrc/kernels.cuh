@@ -150,7 +150,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
 
     // One loop serves both kinds of pass so that the per-ray code (ray_color and everything it inlines) exists
     // exactly once in the kernel: only the work fetch and the epilogue differ.
-    const bool primary = q.in == nullptr;
+    const bool primary = (FLAGS & NTR_F_SS) != 0 || q.in == nullptr;       // NTR_F_SS builds only run primary passes
     const int my_rows = f.tile_row_first < f.tiles_y
                             ? (f.tiles_y - f.tile_row_first + f.tile_row_step - 1) / f.tile_row_step : 0;
     uint32_t total = (uint32_t)my_rows * (uint32_t)f.tiles_x * NTR_BLOCKS_PER_TILE;
@@ -227,9 +227,16 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
             out_row0 = f.compact ? (tyi * NTR_TILE + (by - ty * NTR_TILE)) : by;
             pix = (uint32_t)(out_row0 + (lane >> 3)) * (uint32_t)f.win_w + (uint32_t)px;
             if (inside) {
-                primary_ray<DT>(s, cam, f, f.x0 + px, f.y0 + py, o, dir);
-                if (s.kind == NTR_SCENE_BOX) box_color<DT>(s, o, dir, acc, &prim);
-                else active = true;
+                if constexpr ((FLAGS & NTR_F_SS) != 0) {
+                    // supersampled frame: the lane traces the ss x ss samples of its pixel right here, one after the other
+                    // (the loop count is the same for every lane); their bounces go to the next pass already weighted
+                    QueueEmit<DT> emit{q, ctl, pix, f.out_mode == NTR_OUT_ACCUM};
+                    ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT)>(s, cam, f, f.x0 + px, f.y0 + py, acc, emit, cnt, &ms);
+                } else {
+                    primary_ray<DT>(s, cam, f, f.x0 + px, f.y0 + py, o, dir);
+                    if (s.kind == NTR_SCENE_BOX) box_color<DT>(s, o, dir, acc, &prim);
+                    else active = true;
+                }
             }
         } else {
             const uint32_t idx = b + lane;
@@ -262,7 +269,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
         // warp-synchronous form (trace_warp.cuh: all 32 lanes enter, `active` says who has a ray; rays park at big leaves
         // and the warp splits them over its lanes when enough lanes are idle) wins where single rays walk leaves of
         // hundreds of items (config 4: 58.4 -> 49.9 ms, its 1/8-frame share 26.3 -> 19.9 ms).
-        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE);      // the per-ray code knows nothing of the switches
+        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE | NTR_F_SS);      // the per-ray code knows nothing of the switches
         if constexpr ((FLAGS & NTR_F_WARP) != 0) {
             if (s.kind != NTR_SCENE_BOX) {          // warp-uniform
                 if (!active) {
@@ -272,7 +279,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
                 QueueEmit<DT> emit{q, ctl, pix, !primary || f.out_mode == NTR_OUT_ACCUM};
                 ray_color_warp<DT, RF>(s, active, o, dir, depth, skip, w, acc, emit, cnt, &prim, done_ctr, &ms);
             }
-        } else if (active) {
+        } else if ((FLAGS & NTR_F_SS) == 0 && active) {
             QueueEmit<DT> emit{q, ctl, pix, !primary || f.out_mode == NTR_OUT_ACCUM};
             ray_color<DT, RF>(s, active, o, dir, depth, skip, w, acc, emit, cnt, &prim, &ms);
         }
@@ -430,8 +437,9 @@ template <int DT, int FLAGS> struct Launch {
     }
 };
 
-// defined in kern_d*.cu: variant index = FLAGS (0..15; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
-// everywhere else the index falls back to the build without it)
+// defined in kern_d*.cu: variant index = FLAGS (0..31; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
+// everywhere else the index falls back to the build without it; NTR_F_SS builds exist in the per-lane, non-wide form only,
+// so NTR_F_SS overrides NTR_F_WARP and NTR_F_WIDE)
 const KernelSet *kernel_set_d3(int flags);
 const KernelSet *kernel_set_d4(int flags);
 const KernelSet *kernel_set_d5(int flags);
@@ -442,8 +450,13 @@ const KernelSet *kernel_set_d9(int flags);
 const KernelSet *kernel_set_d10(int flags);
 const KernelSet *kernel_set_dn(int flags);
 
+#define NTR_SS_SETS(DT)                                                                                 \
+        static const KernelSet ss[4] = {Launch<DT, NTR_F_SS>::get(), Launch<DT, 1 | NTR_F_SS>::get(),   \
+                                        Launch<DT, 2 | NTR_F_SS>::get(), Launch<DT, 3 | NTR_F_SS>::get()}; \
+        if (flags & NTR_F_SS) return &ss[flags & 3];
 #define NTR_INSTANTIATE_DIM(NAME, DT)                                                                   \
     const KernelSet *NAME(int flags) {                                                                  \
+        NTR_SS_SETS(DT)                                                                                 \
         static const KernelSet sets[8] = {Launch<DT, 0>::get(), Launch<DT, 1>::get(), Launch<DT, 2>::get(), \
                                           Launch<DT, 3>::get(), Launch<DT, 4>::get(), Launch<DT, 5>::get(), \
                                           Launch<DT, 6>::get(), Launch<DT, 7>::get()};                  \
@@ -451,6 +464,7 @@ const KernelSet *kernel_set_dn(int flags);
     }
 #define NTR_INSTANTIATE_DIM_WIDE(NAME, DT)                                                              \
     const KernelSet *NAME(int flags) {                                                                  \
+        NTR_SS_SETS(DT)                                                                                 \
         static const KernelSet sets[8] = {Launch<DT, 0>::get(), Launch<DT, 1>::get(), Launch<DT, 2>::get(), \
                                           Launch<DT, 3>::get(), Launch<DT, 4>::get(), Launch<DT, 5>::get(), \
                                           Launch<DT, 6>::get(), Launch<DT, 7>::get()};                  \

@@ -1508,6 +1508,53 @@ NTR_HD void box_color(const SceneDev &s, const float *o, const float *dir, float
     if (primary_out) { primary_out->dist = 0; primary_out->ref = NTR_NONE_REF; primary_out->lane = -1; }
 }
 
+// ---- supersampling (ntr_scene_set_supersampling; no counterpart in the reference) ----------------------------------
+// Output pixel (x, y) of a frame with factor ss = f.ss > 1 is the box-filtered mean of pixels (ss*x + i, ss*y + j) of the
+// ss-times-larger view that f describes, summed j-major, i-minor.  Every sample is traced from zero exactly as the big
+// view's pixel, with weight 1/ss^2 from the start, so its bounces (emitted to the next pass with that weight) need nothing
+// special.  Scaling by a power of two is exact and no decision of the per-ray code reads the weight: for ss in {2, 4, 8}
+// the per-sample colours are the big view's times 1/ss^2 and their sum is the big view's float32 sequential box sum times
+// 1/ss^2, bit for bit.  The sum is added without contraction so that it cannot fuse with the last product of a sample.
+NTR_HD float add_rn(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fadd_rn(a, b);
+#else
+    return a + b;
+#endif
+}
+NTR_HD float mul_rn(float a, float b) {
+#if defined(__CUDA_ARCH__)
+    return __fmul_rn(a, b);
+#else
+    return a * b;
+#endif
+}
+
+// colour of output pixel (x, y) of a supersampled frame into sum[3]; samples go to the (per-lane) ray_color
+template <int DT, int FLAGS, typename EMIT>
+NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, float *sum,
+                           EMIT &emit, Counters &cnt, MailboxStore *ms) {
+    constexpr int CAP = DimCap<DT>::value;
+    const int ss = f.ss;
+    const float wt = 1.0f / (float)(ss * ss);
+    const float w[3] = {wt, wt, wt};
+    const Skip none = {NTR_NONE_REF, 0};
+    sum[0] = 0.0f; sum[1] = 0.0f; sum[2] = 0.0f;
+    for (int k = 0; k < ss * ss; ++k) {
+        const int j = k / ss, i = k - j * ss;
+        float o[CAP], dir[CAP];
+        float c[3] = {0.0f, 0.0f, 0.0f};
+        primary_ray<DT>(s, cam, f, ss * x + i, ss * y + j, o, dir);
+        if (s.kind == NTR_SCENE_BOX) {
+            box_color<DT>(s, o, dir, c, nullptr);                  // assigns the colour: weight it here
+            c[0] = mul_rn(c[0], wt); c[1] = mul_rn(c[1], wt); c[2] = mul_rn(c[2], wt);
+        } else {
+            ray_color<DT, FLAGS>(s, true, o, dir, 0, none, w, c, emit, cnt, nullptr, ms);
+        }
+        sum[0] = add_rn(sum[0], c[0]); sum[1] = add_rn(sum[1], c[1]); sum[2] = add_rn(sum[2], c[2]);
+    }
+}
+
 // ---- pixel packing ------------------------------------------------------------------------------------
 // process_pixel::operator() (reference src/render.cpp:421-462): channel = clamp(f_r*r+f_g*g+f_b*b+f_c,0,1);
 // integer channels lround(v * double(2^bits-1)), float channels raw IEEE bits; bits appended MSB-first into

@@ -9,6 +9,7 @@ Same names, argument meaning and error behaviour as the reference; the arithmeti
 not the hot path.  The dimension is a run-time attribute like in the reference's generic module.
 """
 import math
+import numbers
 
 import numpy as np
 
@@ -965,6 +966,8 @@ class _LightList(list):
 
 
 class _SceneBase(Scene):
+    supersampling = 1           # class-level default: scenes pickled before the attribute existed load with it
+
     def __init__(self, dimension):
         self.locked = 0
         self.fov = 0.8
@@ -996,6 +999,19 @@ class _SceneBase(Scene):
         self._check_unlocked()
         self.fov = float(fov)
 
+    def set_supersampling(self, factor):
+        """Anti-aliasing (no counterpart in the reference, which traces one ray through the corner of every pixel): every
+        pixel of a frame becomes the mean of factor x factor samples on an ordered grid over the pixel, i.e. the box-filtered
+        factor-times-larger frame.  factor is an integer from 1 to 8; 1 (the default) is one ray per pixel.  Every renderer
+        and calculate_color honour it.  A frame costs about factor ** 2 times the rays, and the device memory that holds the
+        reflection rays of a frame grows with factor ** 2 as well."""
+        self._check_unlocked()
+        if isinstance(factor, bool) or not isinstance(factor, numbers.Integral):
+            raise TypeError('the supersampling factor must be an integer')
+        if not 1 <= factor <= _capi.NTR_MAX_SUPERSAMPLING:
+            raise ValueError('the supersampling factor must be between 1 and %d' % _capi.NTR_MAX_SUPERSAMPLING)
+        self.supersampling = int(factor)
+
     # ---- backend ----
     def _device_scene(self):
         raise NotImplementedError
@@ -1015,6 +1031,8 @@ class _SceneBase(Scene):
                 grp.set_params(self._scene_dict())
             dev = grp
         dev.set_camera(self._cam._origin, self._cam._axes)
+        if getattr(dev, 'supersampling', 1) != self.supersampling:
+            dev.set_supersampling(self.supersampling)
         return dev
 
     def calculate_color(self, x, y, width, height):
