@@ -166,6 +166,26 @@ NTR_API int ntr_scene_set_params(ntr_scene *scene, const ntr_scene_desc *desc);
  * grows with s*s (see README). */
 #define NTR_MAX_SUPERSAMPLING 8
 NTR_API int ntr_scene_set_supersampling(ntr_scene *scene, int factor);
+/* Adaptive supersampling: trace the s x s samples only where a pixel's corner colours disagree.  threshold t < 0 (the
+ * default) is off: the full supersampling above, byte for byte; NaN or +inf -> NTR_ERR_VALUE.  Host state like the factor,
+ * ignored at factor 1 (the same kernels and launches as without it).  With s > 1 and t >= 0, c(x, y) is the plain 1-spp
+ * float colour of view pixel (x, y) (what factor 1 gives); pixel (x, y) is refined iff, for some channel k,
+ * max c_k(p) - min c_k(p) > t over p in {(x, y), (x+1, y), (x, y+1), (x+1, y+1)} intersected with the VIEW (float32, RGB,
+ * before packing).  A refined pixel's float colour is that of full supersampling at factor s, any other pixel's is c(x, y);
+ * then the frame is packed as usual.  Without reflection passes both parts are bit-identical to the full-SS and the plain
+ * frame; with them every pixel stays within 1 LSB, and the mask may differ where a pixel's contrast lies within float
+ * rounding of t (the bounce passes add with float atomics).  Counters: primary_rays = traced plain pixels (the window's own
+ * pixels and the halo of corner pixels a sharded render or a calculate_color window needs beyond them) + refined pixels *
+ * s*s; the others are summed over everything traced.  Every path that honours the factor honours the threshold
+ * (ntr_render_begin captures it with the camera); the per-ray hooks ignore it.  Adaptive frames are traced synchronously
+ * like frames with reflection passes. */
+NTR_API int ntr_scene_set_supersampling_threshold(ntr_scene *scene, float threshold);
+/* The refine mask of the last completed frame: one byte (1 = refined) per pixel of its window, row-major with a row of
+ * the window's width (for ntr_calculate_color: 1 x 1); len must cover the window or NTR_ERR_VALUE.  A sharded render
+ * (tile-row interleave) writes only its own rows.  *count_or_null receives the number of refined pixels.  A frame that
+ * was not adaptively supersampled has an all-zero mask.  NTR_ERR_RUNTIME before the first frame.  Either pointer may be
+ * NULL. */
+NTR_API int ntr_last_refine_mask(ntr_scene *scene, uint8_t *mask_or_null, size_t len, uint64_t *count_or_null);
 
 /* ---- the hot path ---------------------------------------------------------------------------- */
 /* Renders one frame into a HOST buffer: replaces worker_draw + process_pixel for all tiles
@@ -239,6 +259,10 @@ NTR_API int ntr_group_set_camera(ntr_group *group, const float *origin, const fl
 NTR_API int ntr_group_set_params(ntr_group *group, const ntr_scene_desc *desc);
 /* ntr_scene_set_supersampling for every device of the group. */
 NTR_API int ntr_group_set_supersampling(ntr_group *group, int factor);
+/* ntr_scene_set_supersampling_threshold for every device of the group. */
+NTR_API int ntr_group_set_supersampling_threshold(ntr_group *group, float threshold);
+/* ntr_last_refine_mask of the last group frame: every device writes its tile rows, the count is their sum. */
+NTR_API int ntr_group_last_refine_mask(ntr_group *group, uint8_t *mask_or_null, size_t len, uint64_t *count_or_null);
 /* ntr_render over the group: host destination, same contract (NTR_ERR_ABORTED after ntr_group_abort). */
 NTR_API int ntr_group_render(ntr_group *group, const ntr_image_format *fmt, void *dst, size_t dst_len);
 /* The same frame left in device memory: *dev_frame_out receives the frame buffer on the first device (pitch*height

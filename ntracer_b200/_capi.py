@@ -199,6 +199,8 @@ def load():
         'ntr_scene_set_camera': (C.c_int, [vp, vp, vp]),
         'ntr_scene_set_params': (C.c_int, [vp, C.POINTER(SceneDesc)]),
         'ntr_scene_set_supersampling': (C.c_int, [vp, i32]),
+        'ntr_scene_set_supersampling_threshold': (C.c_int, [vp, C.c_float]),
+        'ntr_last_refine_mask': (C.c_int, [vp, vp, C.c_size_t, C.POINTER(C.c_uint64)]),
         'ntr_render': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t]),
         'ntr_render_device': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t, vp, i32, i32, i32]),
         'ntr_render_begin': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t, C.POINTER(C.c_uint64)]),
@@ -228,6 +230,8 @@ def load():
         'ntr_group_set_camera': (C.c_int, [vp, vp, vp]),
         'ntr_group_set_params': (C.c_int, [vp, C.POINTER(SceneDesc)]),
         'ntr_group_set_supersampling': (C.c_int, [vp, i32]),
+        'ntr_group_set_supersampling_threshold': (C.c_int, [vp, C.c_float]),
+        'ntr_group_last_refine_mask': (C.c_int, [vp, vp, C.c_size_t, C.POINTER(C.c_uint64)]),
         'ntr_group_render': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t]),
         'ntr_group_render_device': (C.c_int, [vp, C.POINTER(ImageFormat), C.POINTER(vp)]),
         'ntr_group_abort': (C.c_int, [vp]),
@@ -257,7 +261,8 @@ EXPORTED_SYMBOLS = (
     'ntr_get_counters', 'ntr_set_instrumented', 'ntr_last_kernel_ms', 'ntr_launch_count',
     'ntr_measure_fp32_peak', 'ntr_simplex_from_points', 'ntr_build_kdtree', 'ntr_build_kdtree_culled', 'ntr_free', 'ntr_group_items',
     'ntr_group_create', 'ntr_group_destroy', 'ntr_group_size', 'ntr_group_set_camera', 'ntr_group_set_params',
-    'ntr_group_set_supersampling',
+    'ntr_group_set_supersampling', 'ntr_scene_set_supersampling_threshold', 'ntr_last_refine_mask',
+    'ntr_group_set_supersampling_threshold', 'ntr_group_last_refine_mask',
     'ntr_group_render', 'ntr_group_render_device', 'ntr_group_abort', 'ntr_group_get_counters',
     'ntr_group_last_kernel_ms', 'ntr_group_launch_count',
     'ntr_frame_alloc', 'ntr_frame_free', 'ntr_frame_export', 'ntr_frame_import', 'ntr_frame_release',

@@ -17,6 +17,13 @@ def _p(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
 
 
+def _refine_mask(fn, handle, w, h):
+    mask = np.zeros((h, w), dtype=np.uint8)
+    count = C.c_uint64(0)
+    _capi.check(fn(handle, _p(mask) if mask.size else None, mask.size, C.byref(count)))
+    return mask, int(count.value)
+
+
 class DeviceScene:
     def __init__(self, scene, device=-1):
         """scene: flat scene dict (DESIGN.md 'scene file'; ntracer_b200.scene_io.load_scene)."""
@@ -27,6 +34,8 @@ class DeviceScene:
         self._scene = scene
         self._open = {}
         self.supersampling = 1
+        self.supersampling_threshold = None
+        self._window = None                     # (width, height) of the last frame's window: the shape of refine_mask()
         desc, keep = _capi.make_desc(scene)
         _capi.check(self._lib.ntr_scene_create(C.byref(desc), device, C.byref(self._h)))
         if 'cam_origin' in scene and 'cam_axes' in scene:
@@ -69,6 +78,18 @@ class DeviceScene:
         _capi.check(self._lib.ntr_scene_set_supersampling(self._h, int(factor)))
         self.supersampling = int(factor)
 
+    def set_supersampling_threshold(self, threshold):
+        """Adaptive supersampling: with a factor above 1, only pixels whose corner colours differ by more than `threshold`
+        in some channel get the factor x factor samples (None = off: every pixel does)."""
+        _capi.check(self._lib.ntr_scene_set_supersampling_threshold(self._h, -1.0 if threshold is None else float(threshold)))
+        self.supersampling_threshold = None if threshold is None else float(threshold)
+
+    def refine_mask(self):
+        """-> (mask, count): the refine mask of the last frame as a (height, width) uint8 array over its window (1 =
+        refined; rows a sharded render does not own stay 0) and the number of refined pixels."""
+        w, h = self._window if self._window else (0, 0)
+        return _refine_mask(self._lib.ntr_last_refine_mask, self._h, w, h)
+
     # ---- the hot path ----
     def render(self, fmt, dest=None):
         """BlockingRenderer.render: packs the frame into `dest` (any writable buffer) or a new uint8 array."""
@@ -81,6 +102,7 @@ class DeviceScene:
             buf = np.frombuffer(dest, dtype=np.uint8)
             if buf.size < need:
                 raise ValueError('the buffer is too small for an image with the given dimensions')
+        self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_render(self._h, C.byref(fmt), _p(buf), buf.size))
         return out
 
@@ -91,6 +113,7 @@ class DeviceScene:
         if buf.size < fmt.pitch * fmt.height:
             raise ValueError('the buffer is too small for an image with the given dimensions')
         ticket = C.c_uint64(0)
+        self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_render_begin(self._h, C.byref(fmt), _p(buf), buf.size, C.byref(ticket)))
         self._open[ticket.value] = buf          # keeps the exported buffer alive while the copy engine writes it
         return ticket.value
@@ -104,16 +127,19 @@ class DeviceScene:
 
     def render_device(self, fmt, dev_ptr, nbytes, stream=0, tile_row_first=0, tile_row_step=1, compact=False):
         """Asynchronous render into device memory (a torch tensor's data_ptr()) on a CUDA stream handle."""
+        self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_render_device(self._h, C.byref(fmt), C.c_void_p(dev_ptr), nbytes,
                                                 C.c_void_p(stream), tile_row_first, tile_row_step, int(compact)))
 
     def render_float(self, width, height):
         out = np.zeros((height, width, 3), dtype=np.float32)
+        self._window = (width, height)
         _capi.check(self._lib.ntr_render_float(self._h, width, height, _p(out)))
         return out
 
     def calculate_color(self, x, y, width, height):
         out = (C.c_float * 3)()
+        self._window = (1, 1)
         _capi.check(self._lib.ntr_calculate_color(self._h, x, y, width, height, out))
         return np.array(list(out), dtype=np.float32)
 
@@ -196,6 +222,8 @@ class DeviceGroup:
         _capi.check(self._lib.ntr_group_create(C.byref(desc), len(devices) if devices is not None else int(n), devs, C.byref(self._h)))
         self.size = int(self._lib.ntr_group_size(self._h))
         self.supersampling = 1
+        self.supersampling_threshold = None
+        self._window = None
         if 'cam_origin' in scene and 'cam_axes' in scene:
             self.set_camera(scene['cam_origin'], scene['cam_axes'])
 
@@ -225,18 +253,29 @@ class DeviceGroup:
         _capi.check(self._lib.ntr_group_set_supersampling(self._h, int(factor)))
         self.supersampling = int(factor)
 
+    def set_supersampling_threshold(self, threshold):
+        _capi.check(self._lib.ntr_group_set_supersampling_threshold(self._h, -1.0 if threshold is None else float(threshold)))
+        self.supersampling_threshold = None if threshold is None else float(threshold)
+
+    def refine_mask(self):
+        """DeviceScene.refine_mask of the last group frame: every device's rows, their refined pixels summed."""
+        w, h = self._window if self._window else (0, 0)
+        return _refine_mask(self._lib.ntr_group_last_refine_mask, self._h, w, h)
+
     def render(self, fmt, dest=None):
         need = fmt.pitch * fmt.height
         out = np.zeros(need, dtype=np.uint8) if dest is None else dest
         buf = out if dest is None else np.frombuffer(dest, dtype=np.uint8)
         if buf.size < need:
             raise ValueError('the buffer is too small for an image with the given dimensions')
+        self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_group_render(self._h, C.byref(fmt), _p(buf), buf.size))
         return out
 
     def render_device(self, fmt):
         """-> address of the frame on the first device (valid until the next render)"""
         ptr = C.c_void_p()
+        self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_group_render_device(self._h, C.byref(fmt), C.byref(ptr)))
         return ptr.value
 

@@ -14,6 +14,8 @@
 #include <vector>
 
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_select.cuh>
+#include <thrust/iterator/counting_iterator.h>
 
 #include "arena_pack.h"
 #include "errors.h"
@@ -49,14 +51,18 @@ int fail(int code, const char *fmt, ...) {
 
 constexpr int kMaxPasses = 64;          // upper bound on max_reflect_depth handled by the control block
 
-// control block layout (uint32 words)
+// control block layout (uint32 words); an adaptively supersampled frame runs a second round of passes with queue
+// counters and cursors of its own (CTL_COUNT0B / CTL_CURSOR0B), the halo and refine passes' cursors and the number of
+// refined pixels (written by the device, read by the refine pass and the host)
 constexpr int kSlabMax = 4;
 enum { CTL_TILE_CURSOR = 0, CTL_OVERFLOW = 1, CTL_COUNT0 = 2, CTL_CURSOR0 = CTL_COUNT0 + kMaxPasses + 1,
-       CTL_WORDS = CTL_CURSOR0 + kMaxPasses + 1 };
+       CTL_COUNT0B = CTL_CURSOR0 + kMaxPasses + 1, CTL_CURSOR0B = CTL_COUNT0B + kMaxPasses + 1,
+       CTL_HALO_CURSOR = CTL_CURSOR0B + kMaxPasses + 1, CTL_LIST_CURSOR, CTL_REFINED, CTL_WORDS };
 
 size_t align_up(size_t v, size_t a) { return (v + a - 1) / a * a; }
 
 __global__ void pack_kernel(const __grid_constant__ FrameDev f);
+__global__ void classify_kernel(const __grid_constant__ FrameDev f, float threshold, unsigned char *mask);
 __global__ void ray_keys_kernel(const float4 *recs, uint32_t rec4, uint32_t n, const uint32_t *count, uint32_t capacity, int D,
                                 const __grid_constant__ SceneDev s, uint32_t *keys, uint32_t *idx, int heavy_first);
 __global__ void ring_bounds_kernel(const uint32_t *sorted_keys, uint32_t n, const uint32_t *count, uint32_t capacity, uint32_t *ring_start);
@@ -151,6 +157,19 @@ struct ntr_scene {
     bool pass_timing = false;
     ntr_counters counters{};
     int ss = 1;                         // supersampling factor (ntr_scene_set_supersampling), read when a frame is enqueued
+    float ss_threshold = -1.0f;         // adaptive supersampling threshold (ntr_scene_set_supersampling_threshold), < 0: off
+    // adaptive frames: refine mask of the launch's own pixels, the compacted list of refined slots, CUB scratch, and the
+    // pass sizes of the refine round in the previous frame (its sort sizes)
+    unsigned char *d_mask = nullptr; size_t mask_cap = 0;
+    uint32_t *d_list = nullptr; size_t list_cap = 0;
+    void *d_select_tmp = nullptr; size_t select_tmp_cap = 0;
+    uint32_t prev_pass_count2[kMaxPasses + 2] = {};
+    // what ntr_last_refine_mask reports: the geometry of the last frame, whether it was adaptive, its halo and refined pixels
+    struct {
+        bool valid = false, adaptive = false;
+        int win_w = 0, win_h = 0, out_rows = 0, trf = 0, trs = 1, compact = 0;
+        uint64_t halo = 0, refined = 0;
+    } last;
     // pageable destinations (what BlockingRenderer.render is handed: a bytearray): frames cross PCIe into this pinned
     // staging buffer in row chunks, and the host copies chunk k into the caller's buffer while chunk k+1 is in flight
     unsigned char *h_stage = nullptr; size_t h_stage_cap = 0;
@@ -158,7 +177,7 @@ struct ntr_scene {
     uint32_t *h_ctl = nullptr;              // pinned read-back of the control block and the counters (frame_readback)
     unsigned long long *h_cnt = nullptr;
     uint64_t launches = 0;
-    int grid_blocks[32] = {};          // per variant flags (NTR_F_SS included)
+    int grid_blocks[64] = {};          // per variant flags (NTR_F_SS and NTR_F_LIST included)
     // NTR_F_WIDE builds (96 registers, 5 CTAs per SM): for frames sharded over 4 or more GPUs, whose passes all end in a few
     // long rays (measured, config 4: 1/4 share 20.9 -> 19.9 ms, 1/8 share 15.2 -> 14.4 ms; 1/2 share and whole frames lose
     // 2..12 %).  Picking the build per pass from pass times measured on the second and third frame of a view gained another
@@ -360,11 +379,30 @@ struct RenderTarget {
 
 // Supersampling factor of a frame: the hit-id hook traces one ray per pixel whatever the scene's factor
 int frame_ss(const ntr_scene *sc, int out_mode) { return out_mode == NTR_OUT_IDS ? 1 : sc->ss; }
+// Adaptive supersampling: a factor above 1 and a threshold.  Such frames always take the accumulator route
+bool frame_adaptive(const ntr_scene *sc, int out_mode) { return frame_ss(sc, out_mode) > 1 && sc->ss_threshold >= 0.0f; }
+
+// Pixels of the halo of frame f that are traced (trace_core.cuh: halo_pixel): the column right of the window and, per owned
+// tile row, the row below it (every pixel but the one past the window is valid or not alike)
+uint64_t count_halo(const FrameDev &f) {
+    uint64_t n = 0;
+    int wx = 0, wy = 0;
+    for (int r = 0; r < f.out_rows; ++r) n += halo_pixel(f, (uint32_t)r, &wx, &wy);
+    for (int k = 0; k < owned_tile_rows(f); ++k) {
+        const uint32_t h = (uint32_t)f.out_rows + (uint32_t)k * (uint32_t)(f.win_w + 1);
+        n += (uint64_t)halo_pixel(f, h, &wx, &wy) * (uint64_t)f.win_w + halo_pixel(f, h + (uint32_t)f.win_w, &wx, &wy);
+    }
+    return n;
+}
 
 // Enqueues every kernel of one frame on `st`.  view = (width,height), window = (x0,y0,w,h).
 // A supersampled frame (factor ss > 1) traces the ss-times-larger view: FrameDev describes that view, while the window,
 // the tile grid and every output stay in output pixels (slabs, tile-row interleaving, compact strips and the 1x1 window of
 // ntr_calculate_color work unchanged).
+// An adaptively supersampled frame (frame_adaptive) runs in two rounds: the plain frame -- the base primary pass into the
+// accumulator, the halo pass (list-driven, factor 1) and the bounce passes -- then classify_kernel marks the pixels to
+// refine and compacts them into a list, the list-driven pass traces them at factor ss over their accumulator slots, the
+// second round of bounce passes follows, and pack_kernel packs the frame.
 int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0, int y0, int win_w, int win_h,
                   const ntr_image_format *fmt, const RenderTarget &tgt, int tile_row_first, int tile_row_step,
                   int compact, bool *used_passes) {
@@ -374,7 +412,8 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         CUDA_TRY(cudaStreamWaitEvent(st, sc->frame_done[sc->ctl_slot], 0));
     FrameDev f;
     memset(&f, 0, sizeof f);
-    const int ss = frame_ss(sc, tgt.out_mode);
+    const bool adaptive = frame_adaptive(sc, tgt.out_mode);
+    const int ss = adaptive ? 1 : frame_ss(sc, tgt.out_mode);          // the base of an adaptive frame is the plain frame
     f.ss = ss;
     f.width = width * ss; f.height = height * ss;
     // flat_origin_ray_source::set_params (tracer.hpp:65-69)
@@ -403,10 +442,11 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         f.out_rows = compact ? my_rows * NTR_TILE : win_h;
     }
     const size_t npix = (size_t)win_w * f.out_rows;
+    const size_t nhalo = adaptive ? halo_slots(f) : 0;          // accumulator slots behind the window's own pixels
     f.packed = tgt.packed; f.accum = tgt.accum; f.ids = tgt.ids; f.dists = tgt.dists;
     f.out_mode = tgt.out_mode;
-    if (passes && tgt.out_mode == NTR_OUT_PACKED) {
-        int rc = ensure((void **)&sc->d_accum, &sc->accum_cap, npix * 3 * sizeof(float));
+    if (adaptive || (passes && tgt.out_mode == NTR_OUT_PACKED)) {
+        int rc = ensure((void **)&sc->d_accum, &sc->accum_cap, (npix + nhalo) * 3 * sizeof(float));
         if (rc) return rc;
         f.accum = sc->d_accum;
         f.out_mode = NTR_OUT_ACCUM;
@@ -415,7 +455,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         // each pass can emit at most (1 + transparent layers) rays per input ray; start with 2 rays per traced sample
         // (ss*ss per pixel; capped at 2^26 records -- 4 GB per queue in 4 dimensions -- unless a plain frame needs more)
         // and let the overflow check regrow (ntr_counters.queue_overflows)
-        const uint64_t plain = (uint64_t)npix * 2;
+        const uint64_t plain = (uint64_t)(npix + nhalo) * 2;
         const uint64_t want = sc->queue_init ? sc->queue_init
                                              : std::max<uint64_t>(std::min<uint64_t>(plain * ss * ss, std::max<uint64_t>(plain, 1ull << 26)), 1u << 16);
         if (sc->queue_capacity < want) {
@@ -495,6 +535,13 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     q.out = sc->d_queue[0];
     q.out_count = d_ctl + CTL_COUNT0 + 1;
     q.in_count = q.in_cursor = nullptr;
+    if (tgt.out_mode != NTR_OUT_IDS) {            // the hit-id hook leaves the last frame's refine mask alone
+        sc->last = {};
+        sc->last.valid = true; sc->last.adaptive = adaptive;
+        sc->last.win_w = win_w; sc->last.win_h = win_h; sc->last.out_rows = f.out_rows;
+        sc->last.trf = tile_row_first; sc->last.trs = f.tile_row_step; sc->last.compact = compact;
+        sc->last.halo = adaptive ? count_halo(f) : 0;
+    }
     auto mark = [&]() {
         if (!(sc->pass_timing || passes) || sc->n_pass_ev >= kMaxPasses + 4) return;
         if (!sc->pass_ev[sc->n_pass_ev]) cudaEventCreate(&sc->pass_ev[sc->n_pass_ev]);
@@ -516,25 +563,45 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         sc->launches += 2;
         sc->sched_ready = true;
     }
-    if (passes) {
+    // the list-driven primary passes of an adaptive frame: per-lane, non-wide NTR_F_LIST builds; no more CTAs than the
+    // exact mailbox has columns
+    const int lflags = (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_LIST;
+    auto list_pass = [&](const FrameDev &fl, uint32_t *cursor, QueueDev ql) {
+        ControlDev cl = ctl;
+        cl.tile_cursor = cursor;
+        if (!passes) ql.out = nullptr;
+        int lgrid = grid_for(sc, lflags);
+        if (sc->dev.mb_table) lgrid = std::min(lgrid, (int)(sc->dev.mb_threads / kCtaThreads));
+        sc->kset(lflags)->render_pass(dim3(lgrid), dim3(kCtaThreads), st, sc->dev, sc->cam, fl, ql, cl);
+        ++sc->launches;
+    };
+    if (adaptive && sc->last.halo) {
+        // the corner pixels of the mask that this launch does not own, at factor 1; their bounces join the base frame's
+        FrameDev fh = f;
+        fh.list_n = (uint32_t)nhalo;
+        list_pass(fh, d_ctl + CTL_HALO_CURSOR, q);
+        mark();
+    }
+    // one round of bounce passes: queue counters at cnt0 + depth, cursors at cur0 + depth, sort sizes from prev[depth]
+    auto bounces = [&](int cnt0, int cur0, const uint32_t *prev) -> int {
         for (int depth = 1; depth <= sc->dev.max_depth; ++depth) {
             q.in = sc->d_queue[(depth - 1) & 1];
             q.out = sc->d_queue[depth & 1];
-            q.in_count = d_ctl + CTL_COUNT0 + depth;
-            q.out_count = d_ctl + CTL_COUNT0 + depth + 1;
-            q.in_cursor = d_ctl + CTL_CURSOR0 + depth;
+            q.in_count = d_ctl + cnt0 + depth;
+            q.out_count = d_ctl + cnt0 + depth + 1;
+            q.in_cursor = d_ctl + cur0 + depth;
             q.in_perm = nullptr;
             q.n_sorted = 0;
             q.ring_start = nullptr;
             // adaptive: the sort (one read-back + key kernel + radix sort per pass) only pays for expensive rays; cheap scenes
             // (config 3: 0.45 ns/ray) lose 20 % to it, star polytopes (6-16 ns/ray unsorted) gain 26-29 %
-            if (sc->sort_rays && sc->pass_ns_per_ray > 1.5f && sc->prev_pass_count[depth] >= (1u << 15)) {
+            if (sc->sort_rays && sc->pass_ns_per_ray > 1.5f && prev[depth] >= (1u << 15)) {
                 // Re-bin the bounces for coherence: reflection rays get more divergent with every depth (measured on
                 // config 4: 1.5 ns/ray for primaries, 6 -> 16 ns/ray for depths 1 -> 4).  Sorting them by a key made of
                 // direction signs + quantised direction + quantised origin hands every warp 32 rays that walk the same
                 // part of the tree.  The sort size is the count this pass had in the previous frame plus a margin (no
                 // read-back between the passes; see ray_keys_kernel).
-                const uint32_t n = (uint32_t)std::min<uint64_t>((uint64_t)sc->prev_pass_count[depth] + sc->prev_pass_count[depth] / 8 + 4096, sc->queue_capacity);
+                const uint32_t n = (uint32_t)std::min<uint64_t>((uint64_t)prev[depth] + prev[depth] / 8 + 4096, sc->queue_capacity);
                 if (sc->sort_cap < n) {
                     for (int k = 0; k < 2; ++k) { cudaFree(sc->d_keys[k]); cudaFree(sc->d_perm[k]); sc->d_keys[k] = sc->d_perm[k] = nullptr; }
                     cudaFree(sc->d_sort_tmp); sc->d_sort_tmp = nullptr; sc->sort_cap = 0;
@@ -574,13 +641,50 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
             dump_stats("bounce", depth);
 #endif
         }
-        if (tgt.out_mode == NTR_OUT_PACKED) {
-            f.out_mode = NTR_OUT_PACKED;
-            const long long groups = (long long)((win_w + 3) / 4) * f.out_rows;
-            const int blocks = (int)std::min<long long>((groups + 255) / 256, (long long)sc->sm_count * 8);
-            pack_kernel<<<blocks, 256, 0, st>>>(f);
-            ++sc->launches;
-        }
+        return NTR_OK;
+    };
+    if (passes) {
+        const int rc = bounces(CTL_COUNT0, CTL_CURSOR0, sc->prev_pass_count);
+        if (rc) return rc;
+    }
+    if (adaptive) {
+        // classify the plain frame: mask and row-major list of the pixels to refine; their count stays on the device
+        int rc = ensure((void **)&sc->d_mask, &sc->mask_cap, std::max<size_t>(npix, 1));
+        if (!rc) rc = ensure((void **)&sc->d_list, &sc->list_cap, std::max<size_t>(npix, 1) * sizeof(uint32_t));
+        if (rc) return rc;
+        size_t bytes = 0;
+        thrust::counting_iterator<uint32_t> slots(0);
+        CUDA_TRY(cub::DeviceSelect::Flagged(nullptr, bytes, slots, sc->d_mask, sc->d_list, d_ctl + CTL_REFINED, (int)npix, st));
+        if ((rc = ensure(&sc->d_select_tmp, &sc->select_tmp_cap, std::max<size_t>(bytes, 256)))) return rc;
+        const int blocks = (int)std::min<long long>(((long long)npix + 255) / 256, (long long)sc->sm_count * 8);
+        if (npix) classify_kernel<<<blocks, 256, 0, st>>>(f, sc->ss_threshold, sc->d_mask);
+        bytes = sc->select_tmp_cap;
+        CUDA_TRY(cub::DeviceSelect::Flagged(sc->d_select_tmp, bytes, slots, sc->d_mask, sc->d_list, d_ctl + CTL_REFINED, (int)npix, st));
+        sc->launches += 2;
+        // refine: the listed pixels at factor s over their slots, in a second round of passes of their own
+        FrameDev fr = f;
+        fr.ss = sc->ss;
+        fr.width = width * fr.ss; fr.height = height * fr.ss;
+        fr.half_w = (float)fr.width / 2.0f;
+        fr.half_h = (float)fr.height / 2.0f;
+        fr.fovI = tanf(sc->dev.fov / 2) / fr.half_w;
+        fr.list = sc->d_list;
+        fr.list_count = d_ctl + CTL_REFINED;
+        QueueDev qr;
+        memset(&qr, 0, sizeof qr);
+        qr.capacity = sc->queue_capacity; qr.rec4 = rec4;
+        qr.out = sc->d_queue[0];
+        qr.out_count = d_ctl + CTL_COUNT0B + 1;
+        list_pass(fr, d_ctl + CTL_LIST_CURSOR, qr);
+        mark();
+        if (passes && (rc = bounces(CTL_COUNT0B, CTL_CURSOR0B, sc->prev_pass_count2))) return rc;
+    }
+    if ((passes || adaptive) && tgt.out_mode == NTR_OUT_PACKED) {
+        f.out_mode = NTR_OUT_PACKED;
+        const long long groups = (long long)((win_w + 3) / 4) * f.out_rows;
+        const int blocks = (int)std::min<long long>((groups + 255) / 256, (long long)sc->sm_count * 8);
+        pack_kernel<<<blocks, 256, 0, st>>>(f);
+        ++sc->launches;
     }
     CUDA_TRY(cudaGetLastError());
     if (!sc->frame_done[sc->ctl_slot]) CUDA_TRY(cudaEventCreateWithFlags(&sc->frame_done[sc->ctl_slot], cudaEventDisableTiming));
@@ -629,15 +733,20 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
     CUDA_TRY(cudaStreamSynchronize(j.st));
     const uint32_t *h_ctl = sc->h_ctl;
     const unsigned long long *h_cnt = sc->h_cnt;
+    const bool adaptive = frame_adaptive(sc, j.tgt.out_mode);
     if (j.passes && sc->n_pass_ev > 2) {
         // cost of the wavefront passes per ray: feeds the decision to re-bin rays in the next frame
         float ms = 0;
         cudaEventElapsedTime(&ms, sc->pass_ev[1], sc->pass_ev[sc->n_pass_ev - 1]);
         uint64_t rays = 0;
         for (int d = 1; d <= sc->dev.max_depth && d <= kMaxPasses; ++d) rays += std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
+        if (adaptive)
+            for (int d = 1; d <= sc->dev.max_depth && d <= kMaxPasses; ++d) rays += std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
         if (rays > 0) sc->pass_ns_per_ray = ms * 1e6f / (float)rays;
     }
     if (j.passes) for (int d = 1; d <= kMaxPasses; ++d) sc->prev_pass_count[d] = std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
+    if (j.passes && adaptive)
+        for (int d = 1; d <= kMaxPasses; ++d) sc->prev_pass_count2[d] = std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
     if (sc->pass_timing && sc->n_pass_ev > 1) {
         fprintf(stderr, "ntr pass ms:");
         for (int i = 0; i + 1 < sc->n_pass_ev; ++i) {
@@ -651,13 +760,18 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
     }
     if (sc->h_abort[sc->abort_idx]) return fail(NTR_ERR_ABORTED, "render aborted");
     const uint64_t overflows = sc->counters.queue_overflows;
-    const uint64_t spp = (uint64_t)frame_ss(sc, j.tgt.out_mode) * frame_ss(sc, j.tgt.out_mode);
+    // an adaptive frame traces its own pixels and its halo once, and the refined pixels ss*ss times more
+    const uint64_t fss = adaptive ? 1 : (uint64_t)frame_ss(sc, j.tgt.out_mode), spp = fss * fss;
     sc->counters.primary_rays = (uint64_t)j.win_w * j.win_h * spp;
     if (j.trs > 1) {
         const int tiles_y = (j.win_h + NTR_TILE - 1) / NTR_TILE;
         uint64_t rows = 0;
         for (int ty = j.trf; ty < tiles_y; ty += j.trs) rows += std::min(NTR_TILE, j.win_h - ty * NTR_TILE);
         sc->counters.primary_rays = rows * (uint64_t)j.win_w * spp;
+    }
+    if (adaptive) {
+        sc->last.refined = h_ctl[CTL_REFINED];
+        sc->counters.primary_rays += sc->last.halo + sc->last.refined * (uint64_t)sc->ss * sc->ss;
     }
     sc->counters.reflection_rays = h_cnt[1]; sc->counters.shadow_rays = h_cnt[2]; sc->counters.node_steps = h_cnt[3];
     sc->counters.simplex_tests = h_cnt[4]; sc->counters.solid_tests = h_cnt[5]; sc->counters.shaded_hits = h_cnt[6];
@@ -666,7 +780,7 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
     if (!j.passes || !h_ctl[CTL_OVERFLOW]) return NTR_OK;
     // a wavefront queue was too small: the counters say how many records were wanted
     uint32_t need = 0;
-    for (int d = 1; d <= kMaxPasses; ++d) need = std::max(need, h_ctl[CTL_COUNT0 + d]);
+    for (int d = 1; d <= kMaxPasses; ++d) need = std::max(need, std::max(h_ctl[CTL_COUNT0 + d], h_ctl[CTL_COUNT0B + d]));
     sc->counters.queue_overflows = overflows + 1;
     int rc = ensure_queues(sc, (uint32_t)std::min<uint64_t>((uint64_t)need * 2 + 1024, 0x7FFFFFFFu));
     if (rc) return rc;
@@ -770,6 +884,7 @@ int run_frame_slabs(ntr_scene *sc, const ntr_image_format *fmt, unsigned char *d
     }
     for (int i = 1; i < S; ++i) cudaStreamWaitEvent(sc->stream, sc->slab_done[i], 0);
     if (rc) { cudaStreamSynchronize(sc->stream); return rc; }
+    sc->last.win_h = fmt->height; sc->last.out_rows = fmt->height;      // the refine mask covers the whole (plain) frame
     CUDA_TRY(cudaEventRecord(sc->ev1, sc->stream));
     sc->timing_valid = true;
     if (staged) {
@@ -838,6 +953,16 @@ __global__ void pack_kernel(const __grid_constant__ FrameDev f) {
         } else {
             for (int j = 0; j < nb; ++j) dst[j] = buf[j];
         }
+    }
+}
+
+// Refine mask of the pixels an adaptive frame owns (trace_core.cuh: refine_pixel), f: the plain frame in the accumulator
+__global__ void classify_kernel(const __grid_constant__ FrameDev f, float threshold, unsigned char *mask) {
+    const long long npix = (long long)f.win_w * f.out_rows;
+    for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < npix; i += (long long)gridDim.x * blockDim.x) {
+        const int wx = (int)(i % f.win_w), wy = window_row(f, (int)(i / f.win_w));
+        int r = 0;
+        mask[i] = owned_row(f, wy, &r) && refine_pixel(f, f.accum, wx, wy, threshold) ? 1 : 0;
     }
 }
 
@@ -1034,6 +1159,7 @@ NTR_API void ntr_scene_destroy(ntr_scene *sc) {
     cudaFree(sc->d_queue[0]); cudaFree(sc->d_queue[1]); cudaFree(sc->d_scratch);
     cudaFree(sc->d_tile_cost); cudaFree(sc->d_tile_order); cudaFree(sc->d_ring);
     cudaFree(sc->d_keys[0]); cudaFree(sc->d_keys[1]); cudaFree(sc->d_perm[0]); cudaFree(sc->d_perm[1]); cudaFree(sc->d_sort_tmp);
+    cudaFree(sc->d_mask); cudaFree(sc->d_list); cudaFree(sc->d_select_tmp);
     if (sc->copy_stream) { cudaStreamSynchronize(sc->copy_stream); cudaStreamDestroy(sc->copy_stream); }
     for (int i = 0; i < kSlabMax; ++i) {
         if (sc->slab_stream[i]) { cudaStreamSynchronize(sc->slab_stream[i]); cudaStreamDestroy(sc->slab_stream[i]); }
@@ -1077,6 +1203,42 @@ NTR_API int ntr_scene_set_supersampling(ntr_scene *sc, int factor) {
     return NTR_OK;
 }
 
+NTR_API int ntr_scene_set_supersampling_threshold(ntr_scene *sc, float threshold) {
+    if (!sc) return fail(NTR_ERR_VALUE, "scene is NULL");
+    if (isnan(threshold) || threshold == INFINITY) return fail(NTR_ERR_VALUE, "the supersampling threshold must be a finite number (negative: off)");
+    if (sc->busy) return fail(NTR_ERR_RUNTIME, "the scene is locked while rendering");
+    sc->ss_threshold = threshold < 0.0f ? -1.0f : threshold;
+    return NTR_OK;
+}
+
+NTR_API int ntr_last_refine_mask(ntr_scene *sc, uint8_t *mask, size_t len, uint64_t *count) {
+    if (!sc) return fail(NTR_ERR_VALUE, "scene is NULL");
+    if (!sc->last.valid) return fail(NTR_ERR_RUNTIME, "nothing has been rendered yet");
+    if (sc->busy) return fail(NTR_ERR_RUNTIME, "the renderer is running");
+    const auto &L = sc->last;
+    if (mask) {
+        if (len < (size_t)L.win_w * L.win_h) return fail(NTR_ERR_VALUE, "the mask of the last frame needs %d x %d bytes", L.win_w, L.win_h);
+        std::vector<unsigned char> h;
+        if (L.adaptive) {
+            h.resize((size_t)L.win_w * L.out_rows);
+            CUDA_TRY(cudaSetDevice(sc->device));
+            CUDA_TRY(cudaMemcpy(h.data(), sc->d_mask, h.size(), cudaMemcpyDeviceToHost));
+        }
+        FrameDev g;
+        memset(&g, 0, sizeof g);
+        g.win_w = L.win_w; g.win_h = L.win_h; g.tiles_y = (L.win_h + NTR_TILE - 1) / NTR_TILE;
+        g.tile_row_first = L.trf; g.tile_row_step = L.trs; g.compact = L.compact;
+        for (int wy = 0, r = 0; wy < L.win_h; ++wy) {
+            if (!owned_row(g, wy, &r)) continue;
+            unsigned char *row = mask + (size_t)wy * L.win_w;
+            if (L.adaptive) memcpy(row, h.data() + (size_t)r * L.win_w, (size_t)L.win_w);
+            else memset(row, 0, (size_t)L.win_w);
+        }
+    }
+    if (count) *count = L.adaptive ? L.refined : 0;
+    return NTR_OK;
+}
+
 NTR_API int ntr_scene_set_params(ntr_scene *sc, const ntr_scene_desc *desc) {
     if (!sc || !desc) return fail(NTR_ERR_VALUE, "NULL argument");
     if (sc->busy) return fail(NTR_ERR_RUNTIME, "the scene is locked while rendering");
@@ -1110,7 +1272,7 @@ NTR_API int ntr_render_device(ntr_scene *sc, const ntr_image_format *fmt, void *
     RenderTarget tgt;
     tgt.out_mode = NTR_OUT_PACKED;
     tgt.packed = static_cast<unsigned char *>(dev_dst);
-    if (!passes) {
+    if (!passes && !frame_adaptive(sc, NTR_OUT_PACKED)) {
         // single persistent kernel, fully asynchronous on the caller's stream
         bool p = false;
         CUDA_TRY(cudaEventRecord(sc->ev0, st));
@@ -1137,7 +1299,8 @@ NTR_API int ntr_render(ntr_scene *sc, const ntr_image_format *fmt, void *dst, si
     if (dst_len < bytes) return fail(NTR_ERR_VALUE, "the buffer is too small for an image with the given dimensions");
     RenderTarget tgt;
     tgt.out_mode = NTR_OUT_PACKED;
-    if (sc->zero_copy && !(sc->dev.kind == NTR_SCENE_COMPOSITE && sc->any_reflective && sc->dev.max_depth > 0)) {
+    const bool adaptive = frame_adaptive(sc, NTR_OUT_PACKED);
+    if (sc->zero_copy && !adaptive && !(sc->dev.kind == NTR_SCENE_COMPOSITE && sc->any_reflective && sc->dev.max_depth > 0)) {
         // Single-pass frame into a pinned (mapped) destination: the packing epilogue of the kernel stores the pixels
         // straight into host memory, so the PCIe transfer runs underneath the tracing instead of after it.
         // MEASURED (B200, PCIe Gen5): byte-identical frames, but SLOWER end to end -- config 1 0.114 -> 0.186 ms,
@@ -1161,7 +1324,7 @@ NTR_API int ntr_render(ntr_scene *sc, const ntr_image_format *fmt, void *dst, si
     const bool pinned = cudaPointerGetAttributes(&attr, dst) == cudaSuccess && attr.type == cudaMemoryTypeHost;
     cudaGetLastError();
     const bool staged = !pinned && getenv("NTR_NO_STAGING") == nullptr;
-    if (sc->slabs && (pinned || staged) && !(sc->dev.kind == NTR_SCENE_COMPOSITE && sc->any_reflective && sc->dev.max_depth > 0)) {
+    if (sc->slabs && (pinned || staged) && !adaptive && !(sc->dev.kind == NTR_SCENE_COMPOSITE && sc->any_reflective && sc->dev.max_depth > 0)) {
         rc = run_frame_slabs(sc, fmt, static_cast<unsigned char *>(dst), staged);
         if (rc <= 0) return rc;
     }
@@ -1214,7 +1377,7 @@ NTR_API int ntr_render_begin(ntr_scene *sc, const ntr_image_format *fmt, void *d
     tgt.packed = fs.d_buf;
     const bool composite = sc->dev.kind == NTR_SCENE_COMPOSITE;
     const bool passes = composite && sc->any_reflective && sc->dev.max_depth > 0;
-    if (!passes) {
+    if (!passes && !frame_adaptive(sc, NTR_OUT_PACKED)) {
         // one persistent kernel: fully asynchronous
         bool p = false;
         cudaEventRecord(sc->ev0, sc->stream);
@@ -1224,7 +1387,8 @@ NTR_API int ntr_render_begin(ntr_scene *sc, const ntr_image_format *fmt, void *d
         sc->counters = ntr_counters{};
         sc->counters.primary_rays = (uint64_t)fmt->width * fmt->height * sc->ss * sc->ss;
     } else {
-        // wavefront passes need their counters back between passes: traced synchronously, only the copy overlaps
+        // wavefront passes need their counters back between passes, an adaptive frame its refined count: traced
+        // synchronously, only the copy overlaps
         rc = run_frame_sync(sc, fmt->width, fmt->height, 0, 0, fmt->width, fmt->height, fmt, tgt, 0, 1, 0, sc->stream);
         if (rc == NTR_ERR_ABORTED) rc = NTR_OK;     // reported by ntr_render_end
     }
@@ -1642,6 +1806,25 @@ NTR_API int ntr_group_set_params(ntr_group *g, const ntr_scene_desc *desc) {
 NTR_API int ntr_group_set_supersampling(ntr_group *g, int factor) {
     if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
     for (ntr_scene *sc : g->sc) { const int rc = ntr_scene_set_supersampling(sc, factor); if (rc) return rc; }
+    return NTR_OK;
+}
+
+NTR_API int ntr_group_set_supersampling_threshold(ntr_group *g, float threshold) {
+    if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
+    for (ntr_scene *sc : g->sc) { const int rc = ntr_scene_set_supersampling_threshold(sc, threshold); if (rc) return rc; }
+    return NTR_OK;
+}
+
+NTR_API int ntr_group_last_refine_mask(ntr_group *g, uint8_t *mask, size_t len, uint64_t *count) {
+    if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
+    uint64_t total = 0;
+    for (ntr_scene *sc : g->sc) {
+        uint64_t n = 0;
+        const int rc = ntr_last_refine_mask(sc, mask, len, &n);
+        if (rc) return rc;
+        total += n;
+    }
+    if (count) *count = total;
     return NTR_OK;
 }
 

@@ -36,8 +36,10 @@ enum : int {
                             // with big leaves; otherwise every lane traces for itself (trace_core.cuh)
     NTR_F_WIDE = 8,         // render_pass_kernel only, general variant in 3..5 dimensions: 96 registers / 5 CTAs per SM instead of
                             // 64 / 8 -- no spills, fewer warps: the build for passes that end in a few long rays (kernels.cuh)
-    NTR_F_SS = 16           // render_pass_kernel only, per-lane form: the primary pass of a supersampled frame (FrameDev::ss > 1),
+    NTR_F_SS = 16,          // render_pass_kernel only, per-lane form: the primary pass of a supersampled frame (FrameDev::ss > 1),
                             // every lane traces the ss x ss samples of its pixel one after the other (trace_core.cuh: ss_pixel_color)
+    NTR_F_LIST = 32         // render_pass_kernel only, per-lane form: the list-driven primary pass of an adaptively supersampled
+                            // frame (FrameDev::list): every lane traces one listed pixel with ss_pixel_color at factor FrameDev::ss
 };
 
 struct SceneDev {
@@ -100,6 +102,11 @@ struct FrameDev {
     FormatDev fmt;
     int ss;                         // supersampling factor: width / height / half_w / half_h / fovI describe the ss-times-larger
                                     // view, the window and tile grid stay in output pixels (1: plain frame)
+    // adaptive supersampling (ntr_scene_set_supersampling_threshold): the NTR_F_LIST pass traces the accumulator slots
+    // list[0 .. *list_count) (list == nullptr: the halo slots npix .. npix + list_n, trace_core.cuh: halo_pixel)
+    const uint32_t *list;
+    const uint32_t *list_count;
+    uint32_t list_n;
 };
 
 // One deferred ray of the wavefront (a reflection bounce): 16-byte aligned record.

@@ -132,6 +132,54 @@ __device__ __forceinline__ void store_block_packed(const FrameDev &f, unsigned c
 #ifndef NTR_MIN_CTAS_WIDE
 #define NTR_MIN_CTAS_WIDE 5
 #endif
+// NTR_F_LIST: the list-driven primary pass of an adaptively supersampled frame.  Every fetch takes up to 32 list entries,
+// one accumulator slot per lane; the lane traces its pixel with ss_pixel_color at the factor f describes (1 for the halo,
+// s for the refinement), stores the colour over the slot and emits the bounces for the next pass.
+template <int DT, int FLAGS>
+__device__ __forceinline__ void list_pass(const SceneDev &s, const CameraDev &cam, const FrameDev &f, const QueueDev &q,
+                                          const ControlDev &ctl) {
+    const int lane = threadIdx.x & 31;
+    Counters cnt;
+    MailboxStore ms;
+    ms.attach((FLAGS & NTR_F_GENERAL) ? s.mb_table : nullptr, s.mb_words, s.mb_threads, blockIdx.x * blockDim.x + threadIdx.x, s.n_simplex, s.mb_shift);
+    const uint32_t npix = (uint32_t)f.win_w * (uint32_t)f.out_rows;
+    const uint32_t total = f.list_count ? *f.list_count : f.list_n;
+    for (;;) {
+        uint32_t b = 0;
+        if (lane == 0) b = atomicAdd(ctl.tile_cursor, 32u);
+        b = __shfl_sync(0xFFFFFFFFu, b, 0);
+        if (b >= total) break;
+        // the abort poll of the bounce passes: the fetch whose range crosses a multiple of 8192 entries looks
+        if ((b & 8191u) < 32u && *ctl.abort_flag) {
+            if (lane == 0) atomicAdd(ctl.tile_cursor, 0x40000000u);
+            break;
+        }
+        const uint32_t idx = b + lane;
+        uint32_t slot = 0;
+        int wx = 0, wy = 0;
+        bool inside = false;
+        if (idx < total) {
+            slot = f.list ? __ldg(f.list + idx) : npix + idx;
+            if (slot < npix) {
+                wx = (int)(slot % (uint32_t)f.win_w);
+                wy = window_row(f, (int)(slot / (uint32_t)f.win_w));
+                inside = true;
+            } else {
+                inside = halo_pixel(f, slot - npix, &wx, &wy);
+            }
+        }
+        if (inside) {
+            float acc[3];
+            QueueEmit<DT> emit{q, ctl, slot, q.out != nullptr};
+            ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT)>(s, cam, f, f.x0 + wx, f.y0 + wy, acc, emit, cnt, &ms);
+            f.accum[(size_t)slot * 3 + 0] = acc[0]; f.accum[(size_t)slot * 3 + 1] = acc[1]; f.accum[(size_t)slot * 3 + 2] = acc[2];
+        }
+    }
+    __syncwarp();
+    ms.detach();
+    flush_counters(ctl, cnt);
+}
+
 template <int DT, int FLAGS = 0> struct MinCtas {
     static constexpr int value = (FLAGS & NTR_F_WIDE) ? NTR_MIN_CTAS_WIDE : DT > 8 ? NTR_MIN_CTAS_HI : (DT >= 6 ? NTR_MIN_CTAS_MID : NTR_MIN_CTAS);
 };
@@ -140,6 +188,10 @@ __global__ void __launch_bounds__(kCtaThreads, MinCtas<DT, FLAGS>::value)
 render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ CameraDev cam,
                    const __grid_constant__ FrameDev f, const __grid_constant__ QueueDev q,
                    const __grid_constant__ ControlDev ctl) {
+    if constexpr ((FLAGS & NTR_F_LIST) != 0) {
+        list_pass<DT, FLAGS>(s, cam, f, q, ctl);
+        return;
+    }
     constexpr int CAP = DimCap<DT>::value;
     __shared__ __align__(16) unsigned char stage_all[(kCtaThreads / 32) * 512];
     __shared__ int done_all[kCtaThreads / 32];
@@ -437,9 +489,9 @@ template <int DT, int FLAGS> struct Launch {
     }
 };
 
-// defined in kern_d*.cu: variant index = FLAGS (0..31; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
-// everywhere else the index falls back to the build without it; NTR_F_SS builds exist in the per-lane, non-wide form only,
-// so NTR_F_SS overrides NTR_F_WARP and NTR_F_WIDE)
+// defined in kern_d*.cu: variant index = FLAGS (0..63; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
+// everywhere else the index falls back to the build without it; NTR_F_SS and NTR_F_LIST builds exist in the per-lane,
+// non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE)
 const KernelSet *kernel_set_d3(int flags);
 const KernelSet *kernel_set_d4(int flags);
 const KernelSet *kernel_set_d5(int flags);
@@ -453,7 +505,10 @@ const KernelSet *kernel_set_dn(int flags);
 #define NTR_SS_SETS(DT)                                                                                 \
         static const KernelSet ss[4] = {Launch<DT, NTR_F_SS>::get(), Launch<DT, 1 | NTR_F_SS>::get(),   \
                                         Launch<DT, 2 | NTR_F_SS>::get(), Launch<DT, 3 | NTR_F_SS>::get()}; \
-        if (flags & NTR_F_SS) return &ss[flags & 3];
+        if (flags & NTR_F_SS) return &ss[flags & 3];                                                     \
+        static const KernelSet list[4] = {Launch<DT, NTR_F_LIST>::get(), Launch<DT, 1 | NTR_F_LIST>::get(), \
+                                          Launch<DT, 2 | NTR_F_LIST>::get(), Launch<DT, 3 | NTR_F_LIST>::get()}; \
+        if (flags & NTR_F_LIST) return &list[flags & 3];
 #define NTR_INSTANTIATE_DIM(NAME, DT)                                                                   \
     const KernelSet *NAME(int flags) {                                                                  \
         NTR_SS_SETS(DT)                                                                                 \

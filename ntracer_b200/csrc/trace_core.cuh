@@ -1555,6 +1555,77 @@ NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameD
     }
 }
 
+// ---- adaptive supersampling (ntr_scene_set_supersampling_threshold) -------------------------------------------------
+// Pixel (x, y) is refined -- traced again with ss_pixel_color -- iff, in some channel, the plain 1-spp colours of its
+// corner set {(x, y), (x+1, y), (x, y+1), (x+1, y+1)} intersected with the view span more than the threshold.
+//
+// Accumulator slots of one launch: first the npix = win_w * out_rows pixels it owns, slot = out_row * win_w + x (out_row:
+// the window row, or the row of the compacted strip of a sharded render); then the halo, the corner pixels the mask
+// needs that the launch does not own, which it traces itself at factor 1 (no exchange between devices):
+//   npix + r                                 pixel (win_w, row of output row r): the column right of the window
+//   npix + out_rows + k * (win_w + 1) + x    pixel (x, row below the k-th owned tile row), when that row is not owned
+// Slots whose pixel lies outside the view, or whose row is not a real owned row, are never traced or read.
+NTR_HD int owned_tile_rows(const FrameDev &f) {
+    return f.tile_row_first < f.tiles_y ? (f.tiles_y - f.tile_row_first + f.tile_row_step - 1) / f.tile_row_step : 0;
+}
+NTR_HD uint32_t halo_slots(const FrameDev &f) {
+    return (uint32_t)f.out_rows + (uint32_t)owned_tile_rows(f) * (uint32_t)(f.win_w + 1);
+}
+// window row wy -> its output row, if this launch owns it
+NTR_HD bool owned_row(const FrameDev &f, int wy, int *out_row) {
+    if (wy < 0 || wy >= f.win_h) return false;
+    const int ty = wy / NTR_TILE;
+    if (ty < f.tile_row_first || (ty - f.tile_row_first) % f.tile_row_step != 0) return false;
+    *out_row = f.compact ? (ty - f.tile_row_first) / f.tile_row_step * NTR_TILE + wy % NTR_TILE : wy;
+    return true;
+}
+// output row -> window row (the inverse of owned_row; the row may lie past the window in the last tile of a strip)
+NTR_HD int window_row(const FrameDev &f, int out_row) {
+    return f.compact ? (f.tile_row_first + out_row / NTR_TILE * f.tile_row_step) * NTR_TILE + out_row % NTR_TILE : out_row;
+}
+// halo slot npix + h -> window pixel (wx, wy); false when the slot holds no pixel of this frame
+NTR_HD bool halo_pixel(const FrameDev &f, uint32_t h, int *wx, int *wy) {
+    const int vw = f.width / f.ss, vh = f.height / f.ss;
+    int r = 0;
+    if (h < (uint32_t)f.out_rows) {
+        *wx = f.win_w;
+        *wy = window_row(f, (int)h);
+        return f.x0 + f.win_w < vw && owned_row(f, *wy, &r);
+    }
+    h -= (uint32_t)f.out_rows;
+    const int k = (int)(h / (uint32_t)(f.win_w + 1));
+    *wx = (int)(h % (uint32_t)(f.win_w + 1));
+    const int ty = f.tile_row_first + k * f.tile_row_step;
+    *wy = (ty + 1) * NTR_TILE < f.win_h ? (ty + 1) * NTR_TILE : f.win_h;
+    return k < owned_tile_rows(f) && !owned_row(f, *wy, &r) && f.y0 + *wy < vh && f.x0 + *wx < vw;
+}
+// slot of corner pixel (wx, wy) of an owned pixel, or -1 when it lies outside the view
+NTR_HD long long corner_slot(const FrameDev &f, int wx, int wy) {
+    const int vw = f.width / f.ss, vh = f.height / f.ss;
+    if (f.x0 + wx >= vw || f.y0 + wy >= vh) return -1;
+    const long long npix = (long long)f.win_w * f.out_rows;
+    int r = 0;
+    if (owned_row(f, wy, &r)) return wx < f.win_w ? (long long)r * f.win_w + wx : npix + r;
+    // the row above is owned: wy is the halo row below the k-th owned tile row
+    const int k = ((wy - 1) / NTR_TILE - f.tile_row_first) / f.tile_row_step;
+    return npix + f.out_rows + (long long)k * (f.win_w + 1) + wx;
+}
+// The refine rule for owned pixel (wx, wy) over the plain colours in accum (3 floats per slot): f describes the plain
+// frame (factor 1), t >= 0 is the threshold.
+NTR_HD bool refine_pixel(const FrameDev &f, const float *accum, int wx, int wy, float t) {
+    float lo[3], hi[3];
+    for (int c = 0; c < 4; ++c) {
+        const long long slot = corner_slot(f, wx + (c & 1), wy + (c >> 1));
+        if (slot < 0) continue;                     // (wx, wy) itself is always in the view
+        for (int k = 0; k < 3; ++k) {
+            const float v = accum[slot * 3 + k];
+            lo[k] = c ? fminf(lo[k], v) : v;
+            hi[k] = c ? fmaxf(hi[k], v) : v;
+        }
+    }
+    return hi[0] - lo[0] > t || hi[1] - lo[1] > t || hi[2] - lo[2] > t;
+}
+
 // ---- pixel packing ------------------------------------------------------------------------------------
 // process_pixel::operator() (reference src/render.cpp:421-462): channel = clamp(f_r*r+f_g*g+f_b*b+f_c,0,1);
 // integer channels lround(v * double(2^bits-1)), float channels raw IEEE bits; bits appended MSB-first into

@@ -967,6 +967,7 @@ class _LightList(list):
 
 class _SceneBase(Scene):
     supersampling = 1           # class-level default: scenes pickled before the attribute existed load with it
+    supersampling_threshold = None      # likewise: off, and a scene that never sets it pickles as before
 
     def __init__(self, dimension):
         self.locked = 0
@@ -999,18 +1000,32 @@ class _SceneBase(Scene):
         self._check_unlocked()
         self.fov = float(fov)
 
-    def set_supersampling(self, factor):
+    def set_supersampling(self, factor, threshold=None):
         """Anti-aliasing (no counterpart in the reference, which traces one ray through the corner of every pixel): every
         pixel of a frame becomes the mean of factor x factor samples on an ordered grid over the pixel, i.e. the box-filtered
         factor-times-larger frame.  factor is an integer from 1 to 8; 1 (the default) is one ray per pixel.  Every renderer
         and calculate_color honour it.  A frame costs about factor ** 2 times the rays, and the device memory that holds the
-        reflection rays of a frame grows with factor ** 2 as well."""
+        reflection rays of a frame grows with factor ** 2 as well.
+
+        threshold (a real number >= 0, or None for off) makes it adaptive: the frame is traced at one ray per pixel, and
+        only the pixels whose four corner colours (the pixel and its right, lower and lower-right neighbours) differ by
+        more than threshold in some channel (colours in 0..1) get the factor x factor samples; the others keep their plain
+        colour.  4/255 is a good default (README, "Adaptive anti-aliasing")."""
         self._check_unlocked()
         if isinstance(factor, bool) or not isinstance(factor, numbers.Integral):
             raise TypeError('the supersampling factor must be an integer')
         if not 1 <= factor <= _capi.NTR_MAX_SUPERSAMPLING:
             raise ValueError('the supersampling factor must be between 1 and %d' % _capi.NTR_MAX_SUPERSAMPLING)
+        if threshold is not None:
+            if isinstance(threshold, bool) or not isinstance(threshold, numbers.Real):
+                raise TypeError('the supersampling threshold must be a real number or None')
+            if not (math.isfinite(threshold) and threshold >= 0):
+                raise ValueError('the supersampling threshold must be a finite number >= 0, or None for off')
         self.supersampling = int(factor)
+        if threshold is None:
+            self.__dict__.pop('supersampling_threshold', None)
+        else:
+            self.supersampling_threshold = float(threshold)
 
     # ---- backend ----
     def _device_scene(self):
@@ -1033,6 +1048,8 @@ class _SceneBase(Scene):
         dev.set_camera(self._cam._origin, self._cam._axes)
         if getattr(dev, 'supersampling', 1) != self.supersampling:
             dev.set_supersampling(self.supersampling)
+        if getattr(dev, 'supersampling_threshold', None) != self.supersampling_threshold:
+            dev.set_supersampling_threshold(self.supersampling_threshold)
         return dev
 
     def calculate_color(self, x, y, width, height):
