@@ -119,12 +119,14 @@ struct ntr_scene {
     float4 *d_queue[2] = {nullptr, nullptr};
     uint32_t queue_capacity = 0;
     void *d_scratch = nullptr; size_t scratch_cap = 0;
-    // cost-sorted tile schedule (valid for one window / interleave geometry at a time)
-    unsigned long long *d_tile_cost = nullptr;
-    uint32_t *d_tile_order = nullptr;
-    size_t tile_cap = 0;
-    long long sched_key = -1;           // geometry the stored order belongs to
-    bool sched_ready = false;           // an order has been computed for sched_key
+    // cost-sorted tile schedule, one per control slot (valid for one window / interleave geometry at a time).  The slabs of
+    // a frame run side by side on their own streams, so each needs its own: slot k's order is written by the
+    // order_tiles_kernel behind slot k's primary pass, and slot k is reused only on the same stream or after its frame_done.
+    unsigned long long *d_tile_cost[kSlabMax] = {};
+    uint32_t *d_tile_order[kSlabMax] = {};
+    size_t tile_cap[kSlabMax] = {};
+    long long sched_key[kSlabMax] = {-1, -1, -1, -1};      // geometry the stored order belongs to
+    bool sched_ready[kSlabMax] = {};                        // an order has been computed for sched_key
     // coherence sort of the wavefront queues (keys, permutation, CUB scratch)
     uint32_t *d_keys[2] = {nullptr, nullptr}, *d_perm[2] = {nullptr, nullptr};
     void *d_sort_tmp = nullptr; size_t sort_tmp_bytes = 0; uint32_t sort_cap = 0;
@@ -474,22 +476,23 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     // (config 4: primary pass 11.2-11.6 -> 10.4 ms, frame 43.3 -> 42.4 ms, calls 17 and 20)
     const bool use_sched = n_tiles >= 64 && composite && tgt.out_mode != NTR_OUT_IDS && !sc->no_tile_sched &&
                            (f.tile_row_step > 1 || sc->force_tile_sched || sc->max_leaf >= 256);
+    const int slot = sc->ctl_slot;
     if (use_sched) {
-        if (sc->tile_cap < n_tiles) {
-            cudaFree(sc->d_tile_cost); cudaFree(sc->d_tile_order);
-            sc->d_tile_cost = nullptr; sc->d_tile_order = nullptr; sc->tile_cap = 0;
-            CUDA_TRY(cudaMalloc(&sc->d_tile_cost, n_tiles * sizeof(unsigned long long)));
-            CUDA_TRY(cudaMalloc(&sc->d_tile_order, n_tiles * sizeof(uint32_t)));
-            sc->tile_cap = n_tiles;
-            sc->sched_key = -1;
+        if (sc->tile_cap[slot] < n_tiles) {
+            cudaFree(sc->d_tile_cost[slot]); cudaFree(sc->d_tile_order[slot]);
+            sc->d_tile_cost[slot] = nullptr; sc->d_tile_order[slot] = nullptr; sc->tile_cap[slot] = 0;
+            CUDA_TRY(cudaMalloc(&sc->d_tile_cost[slot], n_tiles * sizeof(unsigned long long)));
+            CUDA_TRY(cudaMalloc(&sc->d_tile_order[slot], n_tiles * sizeof(uint32_t)));
+            sc->tile_cap[slot] = n_tiles;
+            sc->sched_key[slot] = -1;
         }
-        if (sc->sched_key != key) {
-            CUDA_TRY(cudaMemsetAsync(sc->d_tile_cost, 0, n_tiles * sizeof(unsigned long long), st));
-            sc->sched_key = key;
-            sc->sched_ready = false;
+        if (sc->sched_key[slot] != key) {
+            CUDA_TRY(cudaMemsetAsync(sc->d_tile_cost[slot], 0, n_tiles * sizeof(unsigned long long), st));
+            sc->sched_key[slot] = key;
+            sc->sched_ready[slot] = false;
         }
-        f.tile_cost = sc->d_tile_cost;
-        f.tile_order = sc->sched_ready ? sc->d_tile_order : nullptr;
+        f.tile_cost = sc->d_tile_cost[slot];
+        f.tile_order = sc->sched_ready[slot] ? sc->d_tile_order[slot] : nullptr;
     }
 
     ControlDev ctl;
@@ -558,10 +561,10 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     if (use_sched) {
         // schedule for the next frame of this view, computed on the device right behind the primary pass
         const int tb = (int)((n_tiles + 127) / 128);
-        order_tiles_kernel<<<tb, 128, 0, st>>>(sc->d_tile_cost, sc->d_tile_order, (uint32_t)n_tiles);
-        decay_tile_cost_kernel<<<tb, 128, 0, st>>>(sc->d_tile_cost, (uint32_t)n_tiles);
+        order_tiles_kernel<<<tb, 128, 0, st>>>(sc->d_tile_cost[slot], sc->d_tile_order[slot], (uint32_t)n_tiles);
+        decay_tile_cost_kernel<<<tb, 128, 0, st>>>(sc->d_tile_cost[slot], (uint32_t)n_tiles);
         sc->launches += 2;
-        sc->sched_ready = true;
+        sc->sched_ready[slot] = true;
     }
     // the list-driven primary passes of an adaptive frame: per-lane, non-wide NTR_F_LIST builds; no more CTAs than the
     // exact mailbox has columns
@@ -1157,7 +1160,8 @@ NTR_API void ntr_scene_destroy(ntr_scene *sc) {
     cudaFree(sc->arena); cudaFree(sc->d_lights); cudaFree(sc->d_ctl); cudaFree(sc->d_counters); cudaFree(sc->dev.mb_table);
     cudaFree(sc->d_accum); cudaFree(sc->d_packed); cudaFree(sc->d_ids); cudaFree(sc->d_dists);
     cudaFree(sc->d_queue[0]); cudaFree(sc->d_queue[1]); cudaFree(sc->d_scratch);
-    cudaFree(sc->d_tile_cost); cudaFree(sc->d_tile_order); cudaFree(sc->d_ring);
+    for (int i = 0; i < kSlabMax; ++i) { cudaFree(sc->d_tile_cost[i]); cudaFree(sc->d_tile_order[i]); }
+    cudaFree(sc->d_ring);
     cudaFree(sc->d_keys[0]); cudaFree(sc->d_keys[1]); cudaFree(sc->d_perm[0]); cudaFree(sc->d_perm[1]); cudaFree(sc->d_sort_tmp);
     cudaFree(sc->d_mask); cudaFree(sc->d_list); cudaFree(sc->d_select_tmp);
     if (sc->copy_stream) { cudaStreamSynchronize(sc->copy_stream); cudaStreamDestroy(sc->copy_stream); }

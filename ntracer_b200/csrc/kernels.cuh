@@ -10,6 +10,8 @@
 //   trace_rays_kernel / occludes_rays_kernel   KDNode.intersects / KDNode.occludes parity hooks
 #pragma once
 #include <cuda_runtime.h>
+#include <stdio.h>
+#include <stdlib.h>
 
 #include "trace_warp.cuh"
 
@@ -466,6 +468,9 @@ struct KernelSet {
 template <int DT, int FLAGS> struct Launch {
     static void render_pass(dim3 g, dim3 b, cudaStream_t st, const SceneDev &s, const CameraDev &cam,
                             const FrameDev &f, const QueueDev &q, const ControlDev &ctl) {
+        // NTR_LAUNCH_LOG=1: one line per launch naming the build that runs (family: the dimension, 0 = run-time dimension)
+        const char *log = getenv("NTR_LAUNCH_LOG");
+        if (log && atoi(log) != 0) fprintf(stderr, "ntr launch family=%d flags=%d grid=%u\n", DT, FLAGS, g.x);
         render_pass_kernel<DT, FLAGS><<<g, b, 0, st>>>(s, cam, f, q, ctl);
     }
     static void trace_rays(dim3 g, dim3 b, cudaStream_t st, const SceneDev &s, uint32_t n, const float *o,

@@ -718,6 +718,16 @@ NTR_HD float prim_test_general(const SceneDev &s, uint2 it, const float *o, cons
     return dist;
 }
 
+// The count of the `goto hit` re-test of an item that gave the first opaque hit of a leaf (below): the test always misses
+// its own cutoff, so it is counted, not run.  The item-by-item scan and the chunked replay count it alike.
+template <int DT, int FLAGS>
+NTR_HD void count_retest(const SceneDev &s, uint32_t item, Counters &cnt) {
+    if (FLAGS & NTR_F_COUNT) {
+        if ((item >> 30) == NTR_REF_SOLID) cnt.solid_tests++;
+        else cnt.simplex_tests += (item >> 30) == NTR_REF_BATCH ? (uint32_t)(((DT > 0 ? 4 : s.batch) + 3) / 4 * 4) : 1u;
+    }
+}
+
 // kd_leaf<Store,true>::intersects (tracer.hpp:977-1086), every observable behaviour kept:
 //   phase 0 (before the first opaque hit of this leaf): tests write straight into o_hit.normal;
 //   the first opaque hit switches to phase 1 WITHOUT marking the item checked, so the same item is
@@ -757,10 +767,7 @@ NTR_HD bool leaf_general(const SceneDev &s, const uint4 node, const float *o, co
                     // same) and a miss in phase 1 writes nothing: what it leaves behind is the last-test result 0 (Q13)
                     // and its count.
                     dist = 0;
-                    if (FLAGS & NTR_F_COUNT) {
-                        if ((item >> 30) == NTR_REF_SOLID) cnt.solid_tests++;
-                        else cnt.simplex_tests += is_batch ? (uint32_t)(((DT > 0 ? 4 : s.batch) + 3) / 4 * 4) : 1u;
-                    }
+                    count_retest<DT, FLAGS>(s, item, cnt);
                 } else {
                     g.th.add(dist, item, lane);
                 }
@@ -881,6 +888,7 @@ NTR_HD void replay_item(const SceneDev &s, const uint2 it, const float *o, const
                 oh.dist = dist; oh.ref = item; oh.lane = e.lane;
                 phase1 = true;
                 dist = 0;       // the re-test of `goto hit` misses its own cutoff (and then the item is added)
+                count_retest<DT, FLAGS>(s, item, cnt);
             } else {
                 g.th.add(dist, item, e.lane);
             }

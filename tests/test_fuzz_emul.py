@@ -98,6 +98,8 @@ def test_chunked_leaf_scan_is_bit_identical_to_the_sequential_one(tmp_path):
                 assert np.array_equal(a, b)
                 for k in ('reflection_rays', 'shadow_rays', 'shaded_hits', 'node_steps'):
                     assert ca[k] == cb[k], k
+                # (a hypercube hit demoted by a stale cutoff is tested again: solid tests may be more)
+                assert ca['simplex_tests'] == cb['simplex_tests'], (ca['simplex_tests'], cb['simplex_tests'])
                 assert np.array_equal(el.render(sc, w, h, generic=True)[0], a)
         for var in variants:
             el._lib = var
@@ -114,8 +116,8 @@ def test_warp_synchronous_path_on_an_emulated_warp(tmp_path):
     __reduce_*_sync a rendezvous of the 32 (tests/host_emul/emul.cpp, -DNTR_EMULATE_WARP) -- once with cooperation
     forced onto almost every leaf (leaf minimum 4 items, no overhead term in the cost model) and once with the shipped
     thresholds, and must reproduce the per-ray form (trace_core.cuh, itself checked against the oracle) bit for bit:
-    images and ray counters.  A lane sequence that diverged between warp intrinsics would hang here (the test is under
-    a timeout) or change the image.  (The wider sweep -- 200 random scenes at 24x14, the 1,600-item leaves of
+    images, ray counters and node steps, and with the shipped thresholds the primitive tests too.  A lane sequence that
+    diverged between warp intrinsics would hang here (the test is under a timeout) or change the image.  (The wider sweep -- 200 random scenes at 24x14, the 1,600-item leaves of
     {5/2,3,3} at 48x27 -- was run once with the same result, DESIGN.md section 5.)"""
     import ctypes as C
     import os
@@ -147,6 +149,11 @@ def test_warp_synchronous_path_on_an_emulated_warp(tmp_path):
                 assert np.array_equal(a, b)
                 for k in ('reflection_rays', 'shadow_rays', 'shaded_hits', 'node_steps'):
                     assert ca[k] == cb[k], k
+                if lib is libs[1]:
+                    # with cooperation forced onto small leaves, lanes also test items the owner's mailbox would skip and
+                    # the rest of a chunk behind a shadow ray's blocker: more tests, the same answers
+                    for k in ('simplex_tests', 'solid_tests'):
+                        assert ca[k] == cb[k], (k, ca[k], cb[k])
             is_general = bool(np.any(sc['materials'][:, 6] < 1)) or len(sc['solids']) > 0
             general += is_general
             opaque += not is_general
