@@ -214,6 +214,25 @@ NTR_API int ntr_render_device(ntr_scene *scene, const ntr_image_format *fmt, voi
 NTR_API int ntr_render_begin(ntr_scene *scene, const ntr_image_format *fmt, void *dst, size_t dst_len,
                              uint64_t *ticket_out);
 NTR_API int ntr_render_end(ntr_scene *scene, uint64_t ticket);
+/* A batch of camera views in one call (no counterpart in the reference): origins is n x D and axes n x D x D, each view in
+ * the layout of ntr_scene_set_camera.  Frame k is written at byte offset k*pitch*height of dst (dst_len must be at least
+ * n*pitch*height); only pixel bytes are written, the pitch padding is left alone.  Frame k is what ntr_render produces after
+ * ntr_scene_set_camera(origins[k], axes[k]) with the scene's current parameters and supersampling factor: byte-identical
+ * for frames without reflection passes (BoxScenes and every factor, 1 included), within 1 LSB per channel with them
+ * (float atomics add in no fixed order).  The scene's own camera is unchanged afterwards.
+ * The views share launches: one persistent launch per pass covers up to V views (V*width*height*factor^2 <= 2^25; the
+ * environment variable NTR_VIEWS_PER_LAUNCH=V overrides), so each bounce depth of all views is one pass, and the frames of
+ * one launch cross PCIe while the next is traced.  Counters are the sums over the views (primary_rays =
+ * n*width*height*factor^2).  With a supersampling threshold set (adaptive supersampling) the views are rendered one after
+ * the other through the ntr_render route instead, and ntr_last_refine_mask describes the last view.
+ * NTR_ERR_VALUE: n < 1, a NULL pointer, a bad format or a short buffer.  NTR_ERR_RUNTIME while a frame of the scene is
+ * rendering or open (ntr_render_begin).  NTR_ERR_ABORTED after ntr_abort(); the frames' contents are then unspecified. */
+NTR_API int ntr_render_views(ntr_scene *scene, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                             void *dst, size_t dst_len);
+/* The same frames into DEVICE memory of the scene's device, on a caller-supplied CUDA stream (NULL = the scene's own):
+ * asynchronous when the frames need a single pass, synchronous on that stream with reflection passes, as ntr_render_device. */
+NTR_API int ntr_render_views_device(ntr_scene *scene, int n, const float *origins, const float *axes,
+                                    const ntr_image_format *fmt, void *dev_dst, size_t dst_len, void *stream);
 /* Float RGB of every pixel (3 floats per pixel, row-major) = scene::calculate_color for the whole
  * view (src/render.hpp:12-13) before channel packing; host destination. */
 NTR_API int ntr_render_float(ntr_scene *scene, int width, int height, float *dst_rgb);
@@ -268,6 +287,12 @@ NTR_API int ntr_group_render(ntr_group *group, const ntr_image_format *fmt, void
 /* The same frame left in device memory: *dev_frame_out receives the frame buffer on the first device (pitch*height
  * bytes, owned by the group, valid until the next render of the group). */
 NTR_API int ntr_group_render_device(ntr_group *group, const ntr_image_format *fmt, void **dev_frame_out);
+/* ntr_render_views over the group, whole views per device: entry i (a device listed twice is two entries) gets views
+ * [floor(i*n/G), floor((i+1)*n/G)), traces them with the batched kernels into its own memory and copies its frames straight
+ * to their place in dst; no frame is split and nothing crosses NVLink.  Counters are summed over the entries,
+ * ntr_group_last_kernel_ms is the slowest entry's.  With a supersampling threshold set, view after view via ntr_group_render. */
+NTR_API int ntr_group_render_views(ntr_group *group, int n, const float *origins, const float *axes,
+                                   const ntr_image_format *fmt, void *dst, size_t dst_len);
 NTR_API int ntr_group_abort(ntr_group *group);
 /* Counters of the last frame summed over the devices; device time of the last frame from the first kernel to the last
  * one of the slowest device (CUDA events on the first device's stream, which waits for the others). */

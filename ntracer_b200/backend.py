@@ -17,6 +17,47 @@ def _p(a):
     return a.ctypes.data_as(C.c_void_p) if a is not None else None
 
 
+def camera_arrays(cameras, dim):
+    """The cameras of a views call -> (origins [n, dim], axes [n, dim, dim]) float32, C-contiguous.  `cameras` is a sequence
+    of tracern.Camera objects or (origin, axes) pairs (what stream.rotation_cameras returns), or a mix of both.
+    TypeError: not such a sequence; ValueError: no camera, or one of another dimension."""
+    from .tracern import Camera
+    try:
+        items = list(cameras)
+    except TypeError:
+        raise TypeError('cameras must be a sequence of Camera objects or (origin, axes) pairs') from None
+    if not items:
+        raise ValueError('at least one camera is needed')
+    origins = np.empty((len(items), dim), np.float32)
+    axes = np.empty((len(items), dim, dim), np.float32)
+    for k, c in enumerate(items):
+        if isinstance(c, Camera):
+            o, a = c._origin, c._axes
+        elif isinstance(c, (tuple, list)) and len(c) == 2:
+            try:
+                o, a = np.asarray(c[0], np.float32), np.asarray(c[1], np.float32)
+            except (TypeError, ValueError):
+                raise TypeError('camera %d: origin and axes must be arrays of numbers' % k) from None
+        else:
+            raise TypeError('camera %d is neither a Camera nor an (origin, axes) pair' % k)
+        if o.shape != (dim,) or a.shape != (dim, dim):
+            raise ValueError('camera %d: the scene and camera must have the same dimension (%d)' % (k, dim))
+        origins[k], axes[k] = o, a
+    return origins, axes
+
+
+def _views_dest(dest, n, fmt):
+    """-> (what render_views returns, the uint8 view of it the library writes)"""
+    need = n * fmt.pitch * fmt.height
+    if dest is None:
+        out = np.zeros((n, fmt.pitch * fmt.height), dtype=np.uint8)
+        return out, out
+    buf = np.frombuffer(dest, dtype=np.uint8)
+    if buf.size < need:
+        raise ValueError('the buffer is too small for %d images with the given dimensions' % n)
+    return dest, buf
+
+
 def _refine_mask(fn, handle, w, h):
     mask = np.zeros((h, w), dtype=np.uint8)
     count = C.c_uint64(0)
@@ -105,6 +146,24 @@ class DeviceScene:
         self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_render(self._h, C.byref(fmt), _p(buf), buf.size))
         return out
+
+    def render_views(self, fmt, cameras, dest=None):
+        """One frame per camera in one call (ntr_render_views): frame k of `dest` (any writable buffer) at byte offset
+        k * pitch * height, or a new (n, pitch * height) uint8 array.  cameras: Camera objects or (origin, axes) pairs.
+        Frame k is what render() gives with camera k; the scene's own camera is left as it is."""
+        origins, axes = camera_arrays(cameras, self.dim)
+        out, buf = _views_dest(dest, len(origins), fmt)
+        self._window = (fmt.width, fmt.height)
+        _capi.check(self._lib.ntr_render_views(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt), _p(buf), buf.size))
+        return out
+
+    def render_views_device(self, fmt, cameras, dev_ptr, nbytes, stream=0):
+        """render_views into device memory (a (n, height, pitch) uint8 torch tensor's data_ptr()) on a CUDA stream handle:
+        asynchronous for frames without reflection passes, synchronous on the stream with them."""
+        origins, axes = camera_arrays(cameras, self.dim)
+        self._window = (fmt.width, fmt.height)
+        _capi.check(self._lib.ntr_render_views_device(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt),
+                                                      C.c_void_p(dev_ptr), int(nbytes), C.c_void_p(stream)))
 
     def render_begin(self, fmt, dest):
         """Enqueue one frame with the current camera and return a ticket (the interactive loop: frame k+1 is traced
@@ -270,6 +329,15 @@ class DeviceGroup:
             raise ValueError('the buffer is too small for an image with the given dimensions')
         self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_group_render(self._h, C.byref(fmt), _p(buf), buf.size))
+        return out
+
+    def render_views(self, fmt, cameras, dest=None):
+        """DeviceScene.render_views over the group: whole views dealt to the devices in contiguous runs
+        (ntr_group_render_views)."""
+        origins, axes = camera_arrays(cameras, self.dim)
+        out, buf = _views_dest(dest, len(origins), fmt)
+        self._window = (fmt.width, fmt.height)
+        _capi.check(self._lib.ntr_group_render_views(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt), _p(buf), buf.size))
         return out
 
     def render_device(self, fmt):

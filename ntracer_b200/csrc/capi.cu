@@ -55,6 +55,7 @@ constexpr int kMaxPasses = 64;          // upper bound on max_reflect_depth hand
 // counters and cursors of its own (CTL_COUNT0B / CTL_CURSOR0B), the halo and refine passes' cursors and the number of
 // refined pixels (written by the device, read by the refine pass and the host)
 constexpr int kSlabMax = 4;
+constexpr int kSchedViews = kSlabMax, kSchedSlots = kSlabMax + 1;     // tile schedules: one per control slot, one for views calls
 enum { CTL_TILE_CURSOR = 0, CTL_OVERFLOW = 1, CTL_COUNT0 = 2, CTL_CURSOR0 = CTL_COUNT0 + kMaxPasses + 1,
        CTL_COUNT0B = CTL_CURSOR0 + kMaxPasses + 1, CTL_CURSOR0B = CTL_COUNT0B + kMaxPasses + 1,
        CTL_HALO_CURSOR = CTL_CURSOR0B + kMaxPasses + 1, CTL_LIST_CURSOR, CTL_REFINED, CTL_WORDS };
@@ -122,11 +123,12 @@ struct ntr_scene {
     // cost-sorted tile schedule, one per control slot (valid for one window / interleave geometry at a time).  The slabs of
     // a frame run side by side on their own streams, so each needs its own: slot k's order is written by the
     // order_tiles_kernel behind slot k's primary pass, and slot k is reused only on the same stream or after its frame_done.
-    unsigned long long *d_tile_cost[kSlabMax] = {};
-    uint32_t *d_tile_order[kSlabMax] = {};
-    size_t tile_cap[kSlabMax] = {};
-    long long sched_key[kSlabMax] = {-1, -1, -1, -1};      // geometry the stored order belongs to
-    bool sched_ready[kSlabMax] = {};                        // an order has been computed for sched_key
+    // Views calls (ntr_render_views) keep one more schedule of their own, at kSchedViews.
+    unsigned long long *d_tile_cost[kSchedSlots] = {};
+    uint32_t *d_tile_order[kSchedSlots] = {};
+    size_t tile_cap[kSchedSlots] = {};
+    long long sched_key[kSchedSlots] = {-1, -1, -1, -1, -1};      // geometry the stored order belongs to
+    bool sched_ready[kSchedSlots] = {};                            // an order has been computed for sched_key
     // coherence sort of the wavefront queues (keys, permutation, CUB scratch)
     uint32_t *d_keys[2] = {nullptr, nullptr}, *d_perm[2] = {nullptr, nullptr};
     void *d_sort_tmp = nullptr; size_t sort_tmp_bytes = 0; uint32_t sort_cap = 0;
@@ -179,7 +181,7 @@ struct ntr_scene {
     uint32_t *h_ctl = nullptr;              // pinned read-back of the control block and the counters (frame_readback)
     unsigned long long *h_cnt = nullptr;
     uint64_t launches = 0;
-    int grid_blocks[64] = {};          // per variant flags (NTR_F_SS and NTR_F_LIST included)
+    int grid_blocks[128] = {};         // per variant flags (NTR_F_SS, NTR_F_LIST and NTR_F_VIEWS included)
     // NTR_F_WIDE builds (96 registers, 5 CTAs per SM): for frames sharded over 4 or more GPUs, whose passes all end in a few
     // long rays (measured, config 4: 1/4 share 20.9 -> 19.9 ms, 1/8 share 15.2 -> 14.4 ms; 1/2 share and whole frames lose
     // 2..12 %).  Picking the build per pass from pass times measured on the second and third frame of a view gained another
@@ -189,7 +191,15 @@ struct ntr_scene {
     int warp_path = 0;                  // 1: bounce passes use the warp-synchronous kernels (scenes with big leaves), 2: every pass; NTR_WARP overrides
     const KernelSet *(*kset)(int) = nullptr;
     std::atomic<bool> busy{false};
-    // begin/end frames (ntr_render_begin / ntr_render_end)
+    // batches of views (ntr_render_views): the cameras of the call on the device, and the wavefront statistics of views calls.
+    // They are kept apart from the single frames' (pass_ns_per_ray, prev_pass_count) -- as the tile schedule is (kSchedViews)
+    // -- so that a frame rendered after a views call makes the decisions it would have made without it, and vice versa.
+    CameraDev *d_views = nullptr; size_t views_cap = 0;
+    float views_pass_ns_per_ray = 0.0f;
+    uint32_t views_prev_pass_count[kMaxPasses + 2] = {};
+    uint32_t views_per_launch = 0;      // NTR_VIEWS_PER_LAUNCH: views per launch of a views call (0: from kViewsSampleCap)
+    // begin/end frames (ntr_render_begin / ntr_render_end); a views call uses their device buffers, staging buffers, events and
+    // copy stream for its double-buffered launches
     FrameSlot slots[NTR_FRAMES_IN_FLIGHT];
     cudaStream_t copy_stream = nullptr;
     uint64_t next_ticket = 0;
@@ -405,9 +415,12 @@ uint64_t count_halo(const FrameDev &f) {
 // accumulator, the halo pass (list-driven, factor 1) and the bounce passes -- then classify_kernel marks the pixels to
 // refine and compacts them into a list, the list-driven pass traces them at factor ss over their accumulator slots, the
 // second round of bounce passes follows, and pack_kernel packs the frame.
+// A batch of views (n_views > 0, whole frames at a factor >= 1, never adaptive) runs the NTR_F_VIEWS primary pass over the
+// cameras views[0 .. n_views): view v has accumulator slots v * npix .. and its packed frame at tgt.packed + v * pitch * win_h;
+// the bounce passes and pack_kernel are the single frame's, over all views at once.
 int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0, int y0, int win_w, int win_h,
                   const ntr_image_format *fmt, const RenderTarget &tgt, int tile_row_first, int tile_row_step,
-                  int compact, bool *used_passes) {
+                  int compact, bool *used_passes, const CameraDev *views = nullptr, uint32_t n_views = 0) {
     uint32_t *const d_ctl = sc->d_ctl + (size_t)sc->ctl_slot * CTL_WORDS;                 // one control block per slab
     unsigned long long *const d_counters = sc->d_counters + (size_t)sc->ctl_slot * 8;
     if (sc->frame_done[sc->ctl_slot] && sc->frame_stream[sc->ctl_slot] != st)
@@ -427,6 +440,10 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     f.tiles_y = (win_h + NTR_TILE - 1) / NTR_TILE;
     f.tile_row_first = tile_row_first; f.tile_row_step = tile_row_step < 1 ? 1 : tile_row_step; f.compact = compact;
     if (fmt) fill_format(f.fmt, fmt);
+    f.views = views; f.n_views = n_views;
+    const size_t nv = n_views ? n_views : 1;
+    // wavefront statistics of the previous frame (of the previous views call, for a batch of views)
+    float &pass_ns_per_ray = n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray;
 
     // Scenes with big leaves: the bounce passes run the warp-synchronous kernels (incoherent rays; lanes that run out of
     // work help the ones parked at big leaves), the primary pass every lane for itself (the 32 rays of an 8x4 pixel block
@@ -448,7 +465,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     f.packed = tgt.packed; f.accum = tgt.accum; f.ids = tgt.ids; f.dists = tgt.dists;
     f.out_mode = tgt.out_mode;
     if (adaptive || (passes && tgt.out_mode == NTR_OUT_PACKED)) {
-        int rc = ensure((void **)&sc->d_accum, &sc->accum_cap, (npix + nhalo) * 3 * sizeof(float));
+        int rc = ensure((void **)&sc->d_accum, &sc->accum_cap, (npix * nv + nhalo) * 3 * sizeof(float));
         if (rc) return rc;
         f.accum = sc->d_accum;
         f.out_mode = NTR_OUT_ACCUM;
@@ -457,7 +474,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         // each pass can emit at most (1 + transparent layers) rays per input ray; start with 2 rays per traced sample
         // (ss*ss per pixel; capped at 2^26 records -- 4 GB per queue in 4 dimensions -- unless a plain frame needs more)
         // and let the overflow check regrow (ntr_counters.queue_overflows)
-        const uint64_t plain = (uint64_t)(npix + nhalo) * 2;
+        const uint64_t plain = (uint64_t)(npix * nv + nhalo) * 2;
         const uint64_t want = sc->queue_init ? sc->queue_init
                                              : std::max<uint64_t>(std::min<uint64_t>(plain * ss * ss, std::max<uint64_t>(plain, 1ull << 26)), 1u << 16);
         if (sc->queue_capacity < want) {
@@ -476,7 +493,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     // (config 4: primary pass 11.2-11.6 -> 10.4 ms, frame 43.3 -> 42.4 ms, calls 17 and 20)
     const bool use_sched = n_tiles >= 64 && composite && tgt.out_mode != NTR_OUT_IDS && !sc->no_tile_sched &&
                            (f.tile_row_step > 1 || sc->force_tile_sched || sc->max_leaf >= 256);
-    const int slot = sc->ctl_slot;
+    const int slot = n_views ? kSchedViews : sc->ctl_slot;
     if (use_sched) {
         if (sc->tile_cap[slot] < n_tiles) {
             cudaFree(sc->d_tile_cost[slot]); cudaFree(sc->d_tile_order[slot]);
@@ -527,9 +544,13 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     const uint32_t wide_now = wide_ok && (sc->wide_mode == 1 || f.tile_row_step >= 4) ? 0xFFFFFFFFu : 0u;
     auto wide_for = [&](int pass) { return (wide_now >> pass) & 1u ? (int)NTR_F_WIDE : 0; };
     // a supersampled primary pass runs the per-lane, non-wide NTR_F_SS build whatever NTR_WARP / NTR_WIDE say (kernels.cuh)
-    const int pflags = ss > 1 ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_SS : primary_flags | wide_for(0);
+    // a batch of views runs the per-lane, non-wide NTR_F_VIEWS build at every factor, 1 included; no more CTAs than the exact
+    // mailbox has columns
+    const int pflags = n_views ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_VIEWS
+                       : ss > 1 ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_SS : primary_flags | wide_for(0);
     const KernelSet *ks = sc->kset(pflags);
-    const int grid = grid_for(sc, pflags);
+    int grid = grid_for(sc, pflags);
+    if (n_views && sc->dev.mb_table) grid = std::min(grid, (int)(sc->dev.mb_threads / kCtaThreads));
     const uint32_t rec4 = 2 + 2 * ((sc->dev.dim + 3) / 4);
     QueueDev q;
     memset(&q, 0, sizeof q);
@@ -598,7 +619,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
             q.ring_start = nullptr;
             // adaptive: the sort (one read-back + key kernel + radix sort per pass) only pays for expensive rays; cheap scenes
             // (config 3: 0.45 ns/ray) lose 20 % to it, star polytopes (6-16 ns/ray unsorted) gain 26-29 %
-            if (sc->sort_rays && sc->pass_ns_per_ray > 1.5f && prev[depth] >= (1u << 15)) {
+            if (sc->sort_rays && pass_ns_per_ray > 1.5f && prev[depth] >= (1u << 15)) {
                 // Re-bin the bounces for coherence: reflection rays get more divergent with every depth (measured on
                 // config 4: 1.5 ns/ray for primaries, 6 -> 16 ns/ray for depths 1 -> 4).  Sorting them by a key made of
                 // direction signs + quantised direction + quantised origin hands every warp 32 rays that walk the same
@@ -647,7 +668,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         return NTR_OK;
     };
     if (passes) {
-        const int rc = bounces(CTL_COUNT0, CTL_CURSOR0, sc->prev_pass_count);
+        const int rc = bounces(CTL_COUNT0, CTL_CURSOR0, n_views ? sc->views_prev_pass_count : sc->prev_pass_count);
         if (rc) return rc;
     }
     if (adaptive) {
@@ -684,7 +705,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     }
     if ((passes || adaptive) && tgt.out_mode == NTR_OUT_PACKED) {
         f.out_mode = NTR_OUT_PACKED;
-        const long long groups = (long long)((win_w + 3) / 4) * f.out_rows;
+        const long long groups = (long long)((win_w + 3) / 4) * f.out_rows * (long long)nv;
         const int blocks = (int)std::min<long long>((groups + 255) / 256, (long long)sc->sm_count * 8);
         pack_kernel<<<blocks, 256, 0, st>>>(f);
         ++sc->launches;
@@ -714,11 +735,15 @@ struct FrameJob {
     int trf, trs, compact;
     cudaStream_t st;
     bool passes = false;
+    const CameraDev *views = nullptr;   // a batch of views (device array) and its size; 0: one frame through the scene's camera
+    uint32_t n_views = 0;
+    bool restart_clock = true;          // false: ev0 keeps marking the start of an earlier launch of the same call
 };
 
 int frame_submit(ntr_scene *sc, FrameJob &j) {
-    CUDA_TRY(cudaEventRecord(sc->ev0, j.st));
-    int rc = enqueue_frame(sc, j.st, j.width, j.height, j.x0, j.y0, j.win_w, j.win_h, j.fmt, j.tgt, j.trf, j.trs, j.compact, &j.passes);
+    if (j.restart_clock) CUDA_TRY(cudaEventRecord(sc->ev0, j.st));
+    int rc = enqueue_frame(sc, j.st, j.width, j.height, j.x0, j.y0, j.win_w, j.win_h, j.fmt, j.tgt, j.trf, j.trs, j.compact, &j.passes,
+                           j.views, j.n_views);
     if (rc) return rc;
     CUDA_TRY(cudaEventRecord(sc->ev1, j.st));
     sc->timing_valid = true;
@@ -745,9 +770,10 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
         for (int d = 1; d <= sc->dev.max_depth && d <= kMaxPasses; ++d) rays += std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
         if (adaptive)
             for (int d = 1; d <= sc->dev.max_depth && d <= kMaxPasses; ++d) rays += std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
-        if (rays > 0) sc->pass_ns_per_ray = ms * 1e6f / (float)rays;
+        if (rays > 0) (j.n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray) = ms * 1e6f / (float)rays;
     }
-    if (j.passes) for (int d = 1; d <= kMaxPasses; ++d) sc->prev_pass_count[d] = std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
+    uint32_t *const prev = j.n_views ? sc->views_prev_pass_count : sc->prev_pass_count;
+    if (j.passes) for (int d = 1; d <= kMaxPasses; ++d) prev[d] = std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
     if (j.passes && adaptive)
         for (int d = 1; d <= kMaxPasses; ++d) sc->prev_pass_count2[d] = std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
     if (sc->pass_timing && sc->n_pass_ev > 1) {
@@ -765,7 +791,7 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
     const uint64_t overflows = sc->counters.queue_overflows;
     // an adaptive frame traces its own pixels and its halo once, and the refined pixels ss*ss times more
     const uint64_t fss = adaptive ? 1 : (uint64_t)frame_ss(sc, j.tgt.out_mode), spp = fss * fss;
-    sc->counters.primary_rays = (uint64_t)j.win_w * j.win_h * spp;
+    sc->counters.primary_rays = (uint64_t)j.win_w * j.win_h * spp * (j.n_views ? j.n_views : 1);
     if (j.trs > 1) {
         const int tiles_y = (j.win_h + NTR_TILE - 1) / NTR_TILE;
         uint64_t rows = 0;
@@ -926,11 +952,15 @@ struct BusyGuard {
 
 // accum (3 floats per window pixel) -> packed image.  One thread packs 4 consecutive pixels of a row so the
 // 4*bpp bytes it owns are a whole number of 32-bit words.
+// A batch of views packs all its frames: accumulator row v * out_rows + y is row y of frame v (at packed + v * pitch * win_h).
 __global__ void pack_kernel(const __grid_constant__ FrameDev f) {
     const int groups_x = (f.win_w + 3) / 4;
-    const long long total = (long long)groups_x * f.out_rows;
+    const long long total = (long long)groups_x * f.out_rows * (f.n_views ? f.n_views : 1);
     for (long long g = blockIdx.x * (long long)blockDim.x + threadIdx.x; g < total; g += (long long)gridDim.x * blockDim.x) {
-        const int y = (int)(g / groups_x), x0 = (int)(g % groups_x) * 4;
+        const long long ya = g / groups_x;          // accumulator row
+        const int x0 = (int)(g % groups_x) * 4;
+        const int y = (int)(ya % f.out_rows);
+        const long long view = ya / f.out_rows;
         if (!f.compact && f.tile_row_step > 1) {
             // interleaved render at frame positions: the rows of the other ranks' tile rows are not this rank's to write
             const int ty = y / NTR_TILE;
@@ -940,7 +970,7 @@ __global__ void pack_kernel(const __grid_constant__ FrameDev f) {
         const int bpp = f.fmt.bytes_per_pixel;
         __align__(16) unsigned char buf[64];
         for (int k = 0; k < n; ++k) {
-            const float *a = f.accum + ((size_t)y * f.win_w + x0 + k) * 3;
+            const float *a = f.accum + ((size_t)ya * f.win_w + x0 + k) * 3;
             const float rgb[3] = {a[0], a[1], a[2]};
             uint32_t w[4];
             pack_pixel(f.fmt, rgb, w);
@@ -949,7 +979,7 @@ __global__ void pack_kernel(const __grid_constant__ FrameDev f) {
                 buf[k * bpp + j] = (unsigned char)(w[sj >> 2] >> (8 * (3 - (sj & 3))));
             }
         }
-        unsigned char *dst = f.packed + (size_t)y * f.fmt.pitch + (size_t)x0 * bpp;
+        unsigned char *dst = f.packed + (size_t)view * f.fmt.pitch * f.win_h + (size_t)y * f.fmt.pitch + (size_t)x0 * bpp;
         const int nb = n * bpp;
         if (((size_t)dst & 3) == 0 && (nb & 3) == 0) {
             for (int j = 0; j < nb; j += 4) *(uint32_t *)(dst + j) = *(const uint32_t *)(buf + j);
@@ -1097,6 +1127,7 @@ NTR_API int ntr_scene_create(const ntr_scene_desc *desc, int device, ntr_scene *
         }
     }
     if (const char *qi = getenv("NTR_QUEUE_INIT")) sc->queue_init = (uint32_t)strtoul(qi, nullptr, 10);
+    if (const char *vl = getenv("NTR_VIEWS_PER_LAUNCH")) sc->views_per_launch = (uint32_t)strtoul(vl, nullptr, 10);
     sc->tree_depth = depth;
     sc->dev.dim = desc->dim;
     sc->dev.kind = desc->kind;
@@ -1160,7 +1191,8 @@ NTR_API void ntr_scene_destroy(ntr_scene *sc) {
     cudaFree(sc->arena); cudaFree(sc->d_lights); cudaFree(sc->d_ctl); cudaFree(sc->d_counters); cudaFree(sc->dev.mb_table);
     cudaFree(sc->d_accum); cudaFree(sc->d_packed); cudaFree(sc->d_ids); cudaFree(sc->d_dists);
     cudaFree(sc->d_queue[0]); cudaFree(sc->d_queue[1]); cudaFree(sc->d_scratch);
-    for (int i = 0; i < kSlabMax; ++i) { cudaFree(sc->d_tile_cost[i]); cudaFree(sc->d_tile_order[i]); }
+    for (int i = 0; i < kSchedSlots; ++i) { cudaFree(sc->d_tile_cost[i]); cudaFree(sc->d_tile_order[i]); }
+    cudaFree(sc->d_views);
     cudaFree(sc->d_ring);
     cudaFree(sc->d_keys[0]); cudaFree(sc->d_keys[1]); cudaFree(sc->d_perm[0]); cudaFree(sc->d_perm[1]); cudaFree(sc->d_sort_tmp);
     cudaFree(sc->d_mask); cudaFree(sc->d_list); cudaFree(sc->d_select_tmp);
@@ -1259,9 +1291,9 @@ NTR_API int ntr_scene_set_params(ntr_scene *sc, const ntr_scene_desc *desc) {
     return NTR_OK;
 }
 
-NTR_API int ntr_render_device(ntr_scene *sc, const ntr_image_format *fmt, void *dev_dst, size_t dst_len, void *stream,
-                              int tile_row_first, int tile_row_step, int compact) {
-    ENTER(sc);
+// ntr_render_device and ntr_render without the entry checks (the scene is locked by the caller)
+static int render_device_locked(ntr_scene *sc, const ntr_image_format *fmt, void *dev_dst, size_t dst_len, void *stream,
+                                int tile_row_first, int tile_row_step, int compact) {
     int rc = check_format(fmt);
     if (rc) return rc;
     if (!dev_dst) return fail(NTR_ERR_VALUE, "destination is NULL");
@@ -1294,8 +1326,13 @@ NTR_API int ntr_render_device(ntr_scene *sc, const ntr_image_format *fmt, void *
                           tile_row_step, compact, st);
 }
 
-NTR_API int ntr_render(ntr_scene *sc, const ntr_image_format *fmt, void *dst, size_t dst_len) {
+NTR_API int ntr_render_device(ntr_scene *sc, const ntr_image_format *fmt, void *dev_dst, size_t dst_len, void *stream,
+                              int tile_row_first, int tile_row_step, int compact) {
     ENTER(sc);
+    return render_device_locked(sc, fmt, dev_dst, dst_len, stream, tile_row_first, tile_row_step, compact);
+}
+
+static int render_locked(ntr_scene *sc, const ntr_image_format *fmt, void *dst, size_t dst_len) {
     int rc = check_format(fmt);
     if (rc) return rc;
     if (!dst) return fail(NTR_ERR_VALUE, "destination is NULL");
@@ -1341,6 +1378,11 @@ NTR_API int ntr_render(ntr_scene *sc, const ntr_image_format *fmt, void *dst, si
         CUDA_TRY(cudaStreamSynchronize(sc->stream));
     }
     return NTR_OK;
+}
+
+NTR_API int ntr_render(ntr_scene *sc, const ntr_image_format *fmt, void *dst, size_t dst_len) {
+    ENTER(sc);
+    return render_locked(sc, fmt, dst, dst_len);
 }
 
 NTR_API int ntr_render_begin(ntr_scene *sc, const ntr_image_format *fmt, void *dst, size_t dst_len, uint64_t *ticket_out) {
@@ -1426,6 +1468,250 @@ NTR_API int ntr_render_end(ntr_scene *sc, uint64_t ticket) {
         if (fs->row_bytes == fs->pitch) memcpy(fs->dst, fs->h_stage, fs->pitch * (size_t)fs->height);
         else for (int y = 0; y < fs->height; ++y) memcpy(fs->dst + (size_t)y * fs->pitch, fs->h_stage + (size_t)y * fs->pitch, fs->row_bytes);
     }
+    return NTR_OK;
+}
+
+// ---- batches of views (ntr_render_views) ------------------------------------------------------------------------------
+// A views call traces its views in launches of at most V views, each one pass per bounce depth over all its views.  V keeps
+// the samples of a launch, V * W * H * s^2, at or below kViewsSampleCap = 2^25: the wavefront queues want 2 records per
+// traced sample, 2^26 records at the cap, which is the size the queues of a single frame are capped at already
+// (enqueue_frame; 4 GB per queue in 4 dimensions); the accumulator then holds at most 2^25 pixels (384 MB) and the device
+// frames of a launch V * pitch * H bytes, twice over (one launch is traced while the previous one is copied).
+// At 1920x1080 that is 16 views per launch, at 640x480 109.  NTR_VIEWS_PER_LAUNCH=n overrides V (tests).
+static const uint64_t kViewsSampleCap = 1ull << 25;
+
+static int views_per_launch(const ntr_scene *sc, const ntr_image_format *fmt, int n) {
+    const uint64_t npix = (uint64_t)fmt->width * fmt->height, ss = (uint64_t)sc->ss;
+    uint64_t v = sc->views_per_launch ? sc->views_per_launch : kViewsSampleCap / (npix * ss * ss);
+    v = std::min<uint64_t>(v, 0x7FFFFFFFull / npix);        // pixel indices v * npix + pix stay below 2^31
+    return (int)std::max<uint64_t>(1, std::min<uint64_t>(v, (uint64_t)n));
+}
+
+// camera k of a views call, in the layout of ntr_scene_set_camera
+static void view_camera(CameraDev &c, const float *origins, const float *axes, int D, int k) {
+    memset(&c, 0, sizeof c);
+    const float *o = origins + (size_t)k * D, *a = axes + (size_t)k * D * D;
+    for (int i = 0; i < D; ++i) {
+        c.origin[i] = o[i];
+        c.right[i] = a[i]; c.up[i] = a[D + i]; c.fwd[i] = a[2 * D + i];
+    }
+}
+
+// the per-frame counters of c added to sum (queue_overflows, a running total of the scene, is the caller's business)
+static void add_counters(ntr_counters &sum, const ntr_counters &c) {
+    sum.primary_rays += c.primary_rays; sum.reflection_rays += c.reflection_rays; sum.shadow_rays += c.shadow_rays;
+    sum.node_steps += c.node_steps; sum.simplex_tests += c.simplex_tests; sum.solid_tests += c.solid_tests;
+    sum.shaded_hits += c.shaded_hits; sum.truncated_hit_lists += c.truncated_hit_lists;
+}
+
+static int check_views(const ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                       const void *dst, size_t dst_len) {
+    int rc = check_format(fmt);
+    if (rc) return rc;
+    if (n < 1) return fail(NTR_ERR_VALUE, "the number of views must be at least 1");
+    if (!origins || !axes || !dst) return fail(NTR_ERR_VALUE, "NULL argument");
+    if (dst_len / (size_t)n < (size_t)fmt->pitch * fmt->height)
+        return fail(NTR_ERR_VALUE, "the buffer is too small for %d images with the given dimensions", n);
+    for (const FrameSlot &fs : sc->slots)
+        if (fs.open) return fail(NTR_ERR_RUNTIME, "the renderer is already running: a frame of ntr_render_begin is open");
+    return NTR_OK;
+}
+
+// One scene's share of a views call: its cameras on the device and its launches.  Frames into host memory (`host`) are traced
+// into the device buffer of frame slot k % 2 and cross PCIe on the copy stream while launch k + 1 is traced; a pageable
+// destination gets them through the slot's pinned staging buffer, which the host empties while the next launch runs.
+// Frames into device memory are stored in place.
+struct ViewsRun {
+    ntr_scene *sc = nullptr;
+    const ntr_image_format *fmt = nullptr;
+    int n = 0, per = 1;                 // views of the run, views per launch
+    unsigned char *dst = nullptr;       // frame 0 of the run
+    cudaStream_t st = nullptr;
+    bool host = false, staged = false;
+    int done = 0, k = 0;                // views and launches finished
+    FrameJob j{};                       // the launch in flight
+    int unstage_slot = -1, unstage_first = 0, unstage_n = 0;     // a staged launch whose frames are still to reach dst
+    ntr_counters sum{};
+    size_t frame_bytes() const { return (size_t)fmt->pitch * fmt->height; }
+};
+
+static int views_begin(ViewsRun &r, const float *origins, const float *axes) {
+    ntr_scene *sc = r.sc;
+    if (r.n < 1) return NTR_OK;
+    r.per = views_per_launch(sc, r.fmt, r.n);
+    std::vector<CameraDev> cams(r.n);
+    for (int k = 0; k < r.n; ++k) view_camera(cams[k], origins, axes, sc->dev.dim, k);
+    // an asynchronous views call on another stream may still be reading the previous cameras
+    if (sc->frame_done[0] && sc->frame_stream[0] != r.st) CUDA_TRY(cudaStreamWaitEvent(r.st, sc->frame_done[0], 0));
+    int rc = ensure((void **)&sc->d_views, &sc->views_cap, cams.size() * sizeof(CameraDev));
+    if (rc) return rc;
+    CUDA_TRY(cudaMemcpyAsync(sc->d_views, cams.data(), cams.size() * sizeof(CameraDev), cudaMemcpyHostToDevice, r.st));
+    if (!r.host) return NTR_OK;
+    if (!sc->copy_stream) CUDA_TRY(cudaStreamCreateWithFlags(&sc->copy_stream, cudaStreamNonBlocking));
+    const size_t bytes = (size_t)r.per * r.frame_bytes();
+    for (FrameSlot &fs : sc->slots) {
+        if (!fs.rendered) CUDA_TRY(cudaEventCreateWithFlags(&fs.rendered, cudaEventDisableTiming));
+        if (!fs.copied) CUDA_TRY(cudaEventCreateWithFlags(&fs.copied, cudaEventDisableTiming));
+        if ((rc = ensure((void **)&fs.d_buf, &fs.d_cap, bytes))) return rc;
+        if (r.staged && fs.h_cap < bytes) {
+            if (fs.h_stage) { cudaFreeHost(fs.h_stage); fs.h_stage = nullptr; fs.h_cap = 0; }
+            CUDA_TRY(cudaHostAlloc((void **)&fs.h_stage, bytes + bytes / 8, cudaHostAllocDefault));
+            fs.h_cap = bytes + bytes / 8;
+        }
+    }
+    return NTR_OK;
+}
+
+// the frames of the staged launch that was copied last: staging buffer -> dst, pixel bytes only
+static int views_unstage(ViewsRun &r) {
+    if (r.unstage_slot < 0) return NTR_OK;
+    const FrameSlot &fs = r.sc->slots[r.unstage_slot];
+    r.unstage_slot = -1;
+    CUDA_TRY(cudaEventSynchronize(fs.copied));
+    const size_t pitch = (size_t)r.fmt->pitch, row_bytes = (size_t)r.fmt->width * r.fmt->bytes_per_pixel;
+    unsigned char *to = r.dst + (size_t)r.unstage_first * r.frame_bytes();
+    const size_t rows = (size_t)r.unstage_n * r.fmt->height;
+    if (row_bytes == pitch) memcpy(to, fs.h_stage, rows * pitch);
+    else for (size_t y = 0; y < rows; ++y) memcpy(to + y * pitch, fs.h_stage + y * pitch, row_bytes);
+    return NTR_OK;
+}
+
+// enqueues the next launch (again after an overflow); the host empties the staging buffer of the previous one meanwhile
+static int views_submit(ViewsRun &r) {
+    ntr_scene *sc = r.sc;
+    const int cnt = std::min(r.per, r.n - r.done);
+    RenderTarget tgt;
+    tgt.out_mode = NTR_OUT_PACKED;
+    if (r.host) {
+        FrameSlot &fs = sc->slots[r.k & 1];
+        CUDA_TRY(cudaStreamWaitEvent(r.st, fs.copied, 0));         // the launch before the last one has left the buffer
+        tgt.packed = fs.d_buf;
+    } else {
+        tgt.packed = r.dst + (size_t)r.done * r.frame_bytes();
+    }
+    r.j = FrameJob{r.fmt->width, r.fmt->height, 0, 0, r.fmt->width, r.fmt->height, r.fmt, tgt, 0, 1, 0, r.st};
+    r.j.views = sc->d_views + r.done;
+    r.j.n_views = (uint32_t)cnt;
+    r.j.restart_clock = r.done == 0;
+    int rc = frame_submit(sc, r.j);
+    if (!rc) rc = frame_readback(sc, r.j);
+    if (!rc) rc = views_unstage(r);
+    return rc;
+}
+
+// waits for the launch in flight; once it needs no retry, sums its counters and sends its frames on their way
+static int views_collect(ViewsRun &r, bool *again) {
+    ntr_scene *sc = r.sc;
+    int rc = frame_collect(sc, r.j, again);
+    if (rc || *again) return rc;
+    add_counters(r.sum, sc->counters);
+    r.sum.queue_overflows = sc->counters.queue_overflows;
+    const int cnt = (int)r.j.n_views;
+    if (r.host) {
+        const int slot = r.k & 1;
+        FrameSlot &fs = sc->slots[slot];
+        const size_t pitch = (size_t)r.fmt->pitch, row_bytes = (size_t)r.fmt->width * r.fmt->bytes_per_pixel;
+        CUDA_TRY(cudaEventRecord(fs.rendered, r.st));
+        CUDA_TRY(cudaStreamWaitEvent(sc->copy_stream, fs.rendered, 0));
+        unsigned char *to = r.staged ? fs.h_stage : r.dst + (size_t)r.done * r.frame_bytes();
+        // only the pixel bytes are written, like process_pixel: the pitch padding of `dst` is left alone
+        CUDA_TRY(cudaMemcpy2DAsync(to, pitch, fs.d_buf, pitch, row_bytes, (size_t)cnt * r.fmt->height, cudaMemcpyDeviceToHost, sc->copy_stream));
+        CUDA_TRY(cudaEventRecord(fs.copied, sc->copy_stream));
+        if (r.staged) { r.unstage_slot = slot; r.unstage_first = r.done; r.unstage_n = cnt; }
+    }
+    r.done += cnt;
+    ++r.k;
+    return NTR_OK;
+}
+
+// waits for the last copies (whatever `rc` says, so that nothing lands in dst after the call) and publishes the counters
+static int views_finish(ViewsRun &r, int rc) {
+    ntr_scene *sc = r.sc;
+    if (r.host && sc->copy_stream) {
+        const cudaError_t e = cudaStreamSynchronize(sc->copy_stream);
+        if (e != cudaSuccess && !rc) rc = fail(NTR_ERR_RUNTIME, "cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
+    }
+    if (!rc) rc = views_unstage(r);
+    r.unstage_slot = -1;
+    if (!rc && r.n > 0) sc->counters = r.sum;
+    return rc;
+}
+
+// the views of a call on one scene, launch after launch (a queue overflow regrows the queues and traces the launch again)
+static int views_run(ViewsRun &r, const float *origins, const float *axes) {
+    int rc = views_begin(r, origins, axes);
+    for (int attempt = 0; !rc && r.done < r.n;) {
+        if (++attempt > 8) { rc = fail(NTR_ERR_RUNTIME, "wavefront queue kept overflowing"); break; }
+        bool again = false;
+        if (!(rc = views_submit(r))) rc = views_collect(r, &again);
+        if (!again) attempt = 0;
+    }
+    return views_finish(r, rc);
+}
+
+// Adaptively supersampled views: one after the other through the single-view route (ntr_render / ntr_render_device), each
+// with its camera; the scene's own camera is put back afterwards and the counters are the sums over the views.
+static int views_one_by_one(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                            unsigned char *dst, bool device, cudaStream_t st) {
+    const CameraDev saved = sc->cam;
+    const size_t fb = (size_t)fmt->pitch * fmt->height;
+    ntr_counters sum{};
+    int rc = NTR_OK;
+    for (int k = 0; k < n && !rc; ++k) {
+        view_camera(sc->cam, origins, axes, sc->dev.dim, k);
+        rc = device ? render_device_locked(sc, fmt, dst + k * fb, fb, st, 0, 1, 0) : render_locked(sc, fmt, dst + k * fb, fb);
+        add_counters(sum, sc->counters);
+        sum.queue_overflows = sc->counters.queue_overflows;
+    }
+    sc->cam = saved;
+    if (!rc) sc->counters = sum;
+    return rc;
+}
+
+NTR_API int ntr_render_views(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                             void *dst, size_t dst_len) {
+    ENTER(sc);
+    int rc = check_views(sc, n, origins, axes, fmt, dst, dst_len);
+    if (rc) return rc;
+    if (frame_adaptive(sc, NTR_OUT_PACKED))
+        return views_one_by_one(sc, n, origins, axes, fmt, static_cast<unsigned char *>(dst), false, sc->stream);
+    cudaPointerAttributes attr;
+    const bool pinned = cudaPointerGetAttributes(&attr, dst) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+    cudaGetLastError();
+    ViewsRun r;
+    r.sc = sc; r.fmt = fmt; r.n = n; r.dst = static_cast<unsigned char *>(dst); r.st = sc->stream;
+    r.host = true; r.staged = !pinned;
+    return views_run(r, origins, axes);
+}
+
+NTR_API int ntr_render_views_device(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                                    void *dev_dst, size_t dst_len, void *stream) {
+    ENTER(sc);
+    int rc = check_views(sc, n, origins, axes, fmt, dev_dst, dst_len);
+    if (rc) return rc;
+    cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
+    if (frame_adaptive(sc, NTR_OUT_PACKED))
+        return views_one_by_one(sc, n, origins, axes, fmt, static_cast<unsigned char *>(dev_dst), true, st);
+    ViewsRun r;
+    r.sc = sc; r.fmt = fmt; r.n = n; r.dst = static_cast<unsigned char *>(dev_dst); r.st = st;
+    const bool passes = sc->dev.kind == NTR_SCENE_COMPOSITE && sc->any_reflective && sc->dev.max_depth > 0;
+    if (passes) return views_run(r, origins, axes);         // synchronous on `st`, as ntr_render_device with passes
+    // single-pass views: every launch fully asynchronous on the caller's stream
+    if ((rc = views_begin(r, origins, axes))) return rc;
+    CUDA_TRY(cudaEventRecord(sc->ev0, st));
+    for (int first = 0; first < n; first += r.per) {
+        const int cnt = std::min(r.per, n - first);
+        RenderTarget tgt;
+        tgt.out_mode = NTR_OUT_PACKED;
+        tgt.packed = r.dst + (size_t)first * r.frame_bytes();
+        bool p = false;
+        if ((rc = enqueue_frame(sc, st, fmt->width, fmt->height, 0, 0, fmt->width, fmt->height, fmt, tgt, 0, 1, 0, &p,
+                                sc->d_views + first, (uint32_t)cnt))) return rc;
+    }
+    CUDA_TRY(cudaEventRecord(sc->ev1, st));
+    sc->timing_valid = true;
+    sc->counters = ntr_counters{};
+    sc->counters.primary_rays = (uint64_t)n * fmt->width * fmt->height * sc->ss * sc->ss;
     return NTR_OK;
 }
 
@@ -1869,6 +2155,114 @@ NTR_API int ntr_group_render(ntr_group *g, const ntr_image_format *fmt, void *ds
     }
     g->busy.store(false);
     return rc;
+}
+
+// Views dealt to the entries in contiguous runs: entry i traces views [i * n / G, (i + 1) * n / G) with the batched kernels
+// into its own device memory and copies its frames straight to their place in dst.  Every round submits the next launch on
+// every entry before it collects any, so that all devices trace at once.
+NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                                   void *dst, size_t dst_len) {
+    if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
+    for (ntr_scene *sc : g->sc) { const int rc = check_views(sc, n, origins, axes, fmt, dst, dst_len); if (rc) return rc; }
+    if (g->busy.exchange(true)) return fail(NTR_ERR_RUNTIME, "the renderer is already running");
+    struct Unbusy { ntr_group *g; ~Unbusy() { g->busy.store(false); } } unbusy{g};
+    const int G = (int)g->sc.size();
+    const size_t fb = (size_t)fmt->pitch * fmt->height;
+    unsigned char *const out = static_cast<unsigned char *>(dst);
+    int rc = NTR_OK;
+    if (frame_adaptive(g->sc[0], NTR_OUT_PACKED)) {
+        // adaptive supersampling: view after view through the group's single-view route (ntr_group_render)
+        std::vector<CameraDev> saved(G);
+        for (int i = 0; i < G; ++i) saved[i] = g->sc[i]->cam;
+        ntr_counters sum{};
+        for (int k = 0; k < n && !rc; ++k) {
+            for (ntr_scene *sc : g->sc) view_camera(sc->cam, origins, axes, sc->dev.dim, k);
+            if ((rc = group_trace(g, fmt))) break;
+            cudaPointerAttributes attr;
+            const bool pinned = cudaPointerGetAttributes(&attr, out) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+            cudaGetLastError();
+            CUDA_TRY(cudaSetDevice(g->dev[0]));
+            if (!pinned) {
+                rc = download_staged(g->sc[0], out + k * fb, (size_t)fmt->pitch, (size_t)fmt->width * fmt->bytes_per_pixel,
+                                     fmt->height, g->d_frame, g->sc[0]->stream);
+            } else {
+                CUDA_TRY(cudaMemcpy2DAsync(out + k * fb, (size_t)fmt->pitch, g->d_frame, (size_t)fmt->pitch,
+                                           (size_t)fmt->width * fmt->bytes_per_pixel, fmt->height, cudaMemcpyDeviceToHost, g->sc[0]->stream));
+                CUDA_TRY(cudaStreamSynchronize(g->sc[0]->stream));
+            }
+            add_counters(sum, g->counters);
+            sum.queue_overflows += g->counters.queue_overflows;
+        }
+        for (int i = 0; i < G; ++i) g->sc[i]->cam = saved[i];
+        if (!rc) g->counters = sum;
+        return rc;
+    }
+    for (int i = 0; i < G; ++i) {
+        ntr_scene *sc = g->sc[i];
+        if (sc->busy.exchange(true)) {
+            for (int k = 0; k < i; ++k) g->sc[k]->busy.store(false);
+            return fail(NTR_ERR_RUNTIME, "the renderer is already running");
+        }
+        sc->h_abort[0] = 0;
+        sc->abort_idx = 0;
+    }
+    struct Release { ntr_group *g; ~Release() { for (ntr_scene *s : g->sc) s->busy.store(false); } } release{g};
+    cudaPointerAttributes attr;
+    const bool pinned = cudaPointerGetAttributes(&attr, dst) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+    cudaGetLastError();
+    std::vector<ViewsRun> runs(G);
+    std::vector<int> first(G), attempts(G, 0);
+    CUDA_TRY(cudaSetDevice(g->dev[0]));
+    CUDA_TRY(cudaEventRecord(g->ev0, g->sc[0]->stream));
+    for (int i = 0; i < G && !rc; ++i) {
+        ViewsRun &r = runs[i];
+        first[i] = (int)((long long)i * n / G);
+        r.sc = g->sc[i]; r.fmt = fmt; r.n = (int)((long long)(i + 1) * n / G) - first[i];
+        r.dst = out + (size_t)first[i] * fb; r.st = g->sc[i]->stream;
+        r.host = true; r.staged = !pinned;
+        CUDA_TRY(cudaSetDevice(g->dev[i]));
+        if (i) CUDA_TRY(cudaStreamWaitEvent(r.st, g->ev0, 0));      // the call's clock starts on dev[0]
+        rc = views_begin(r, origins + (size_t)first[i] * r.sc->dev.dim, axes + (size_t)first[i] * r.sc->dev.dim * r.sc->dev.dim);
+    }
+    for (bool any = true; any && !rc;) {
+        any = false;
+        std::vector<char> sent(G, 0);
+        for (int i = 0; i < G && !rc; ++i) {
+            if (runs[i].done >= runs[i].n) continue;
+            if (++attempts[i] > 8) { rc = fail(NTR_ERR_RUNTIME, "wavefront queue kept overflowing"); break; }
+            cudaSetDevice(g->dev[i]);
+            rc = views_submit(runs[i]);
+            sent[i] = 1;
+            any = true;
+        }
+        for (int i = 0; i < G; ++i) {
+            if (!sent[i]) continue;
+            cudaSetDevice(g->dev[i]);
+            bool again = false;
+            const int r = rc == NTR_OK ? views_collect(runs[i], &again) : (cudaStreamSynchronize(runs[i].st), NTR_OK);
+            if (r != NTR_OK && rc == NTR_OK) rc = r;
+            if (!again) attempts[i] = 0;
+        }
+    }
+    for (int i = 0; i < G; ++i) {
+        cudaSetDevice(g->dev[i]);
+        const int r = views_finish(runs[i], rc);
+        if (r != NTR_OK && rc == NTR_OK) rc = r;
+        if (i) cudaEventRecord(g->done[i], runs[i].st);
+    }
+    // dev[0]'s stream behind every entry: the call's clock stops when the slowest one is done
+    CUDA_TRY(cudaSetDevice(g->dev[0]));
+    for (int i = 1; i < G; ++i) CUDA_TRY(cudaStreamWaitEvent(g->sc[0]->stream, g->done[i], 0));
+    CUDA_TRY(cudaEventRecord(g->ev1, g->sc[0]->stream));
+    g->timing_valid = rc == NTR_OK;
+    if (rc) return rc;
+    g->counters = ntr_counters{};
+    for (const ViewsRun &r : runs) {
+        if (r.n < 1) continue;
+        add_counters(g->counters, r.sum);
+        g->counters.queue_overflows += r.sum.queue_overflows;
+    }
+    return NTR_OK;
 }
 
 NTR_API int ntr_group_abort(ntr_group *g) {

@@ -38,8 +38,11 @@ enum : int {
                             // 64 / 8 -- no spills, fewer warps: the build for passes that end in a few long rays (kernels.cuh)
     NTR_F_SS = 16,          // render_pass_kernel only, per-lane form: the primary pass of a supersampled frame (FrameDev::ss > 1),
                             // every lane traces the ss x ss samples of its pixel one after the other (trace_core.cuh: ss_pixel_color)
-    NTR_F_LIST = 32         // render_pass_kernel only, per-lane form: the list-driven primary pass of an adaptively supersampled
+    NTR_F_LIST = 32,        // render_pass_kernel only, per-lane form: the list-driven primary pass of an adaptively supersampled
                             // frame (FrameDev::list): every lane traces one listed pixel with ss_pixel_color at factor FrameDev::ss
+    NTR_F_VIEWS = 64        // render_pass_kernel only, per-lane form: the primary pass of a batch of views (ntr_render_views,
+                            // FrameDev::views): the blocks of all views in one launch, every lane traces its pixel with
+                            // ss_pixel_color at factor FrameDev::ss (1 included) through the camera of its view
 };
 
 struct SceneDev {
@@ -107,6 +110,10 @@ struct FrameDev {
     const uint32_t *list;
     const uint32_t *list_count;
     uint32_t list_n;
+    // a batch of views (NTR_F_VIEWS): view v traces through views[v]; its pixels take accumulator slots and bounce-record pixel
+    // words v * npix + pix (npix = win_w * out_rows), and its packed frame starts at packed + v * pitch * win_h
+    const CameraDev *views;
+    uint32_t n_views;
 };
 
 // One deferred ray of the wavefront (a reflection bounce): 16-byte aligned record.

@@ -80,7 +80,8 @@ __device__ __forceinline__ void flush_counters(const ControlDev &ctl, const Coun
 
 // Warp-cooperative store of an 8x4 pixel block: pixels are staged in shared memory in memory byte order,
 // then every lane moves one 16-byte chunk of one row segment with the widest aligned store.
-__device__ __forceinline__ void store_block_packed(const FrameDev &f, unsigned char *stage /*512 B per warp*/,
+// `packed`: the frame the block belongs to (f.packed, or frame v of a batch of views)
+__device__ __forceinline__ void store_block_packed(const FrameDev &f, unsigned char *packed, unsigned char *stage /*512 B per warp*/,
                                                    int px0, int py0, int ncols, int nrows, int out_row0,
                                                    const uint32_t w[4], bool inside) {
     const int lane = threadIdx.x & 31;
@@ -100,7 +101,7 @@ __device__ __forceinline__ void store_block_packed(const FrameDev &f, unsigned c
         int n = seg - off;
         if (n > 16) n = 16;
         if (n > 0) {
-            unsigned char *dst = f.packed + (size_t)(out_row0 + r) * f.fmt.pitch + (size_t)px0 * bpp + off;
+            unsigned char *dst = packed + (size_t)(out_row0 + r) * f.fmt.pitch + (size_t)px0 * bpp + off;
             const unsigned char *src = stage + r * 128 + off;
             while (n > 0) {
                 const size_t a = (size_t)dst | (size_t)src;      // both sides must be aligned for the unit
@@ -204,10 +205,12 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
 
     // One loop serves both kinds of pass so that the per-ray code (ray_color and everything it inlines) exists
     // exactly once in the kernel: only the work fetch and the epilogue differ.
-    const bool primary = (FLAGS & NTR_F_SS) != 0 || q.in == nullptr;       // NTR_F_SS builds only run primary passes
+    constexpr bool VIEWS = (FLAGS & NTR_F_VIEWS) != 0;
+    const bool primary = (FLAGS & (NTR_F_SS | NTR_F_VIEWS)) != 0 || q.in == nullptr;   // NTR_F_SS / NTR_F_VIEWS builds only run primary passes
     const int my_rows = f.tile_row_first < f.tiles_y
                             ? (f.tiles_y - f.tile_row_first + f.tile_row_step - 1) / f.tile_row_step : 0;
     uint32_t total = (uint32_t)my_rows * (uint32_t)f.tiles_x * NTR_BLOCKS_PER_TILE;
+    if constexpr (VIEWS) total *= f.n_views;
     const int D4 = (int)(q.rec4 - 2) / 2;
     if (!primary) {
         total = *q.in_count;
@@ -254,7 +257,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
         float acc[3] = {0.f, 0.f, 0.f};
         Skip skip = {NTR_NONE_REF, 0};
         int depth = 0;
-        uint32_t pix = 0;
+        uint32_t pix = 0, view = 0;
         bool active = false, inside = false;
         int bx = 0, by = 0, px = 0, out_row0 = 0;
         HitRec prim;
@@ -265,7 +268,12 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
             // Longest-processing-time-first scheduling: tiles are handed out in the order of their measured cost
             // in the previous frame of this view (order_tiles_kernel), so the kernel's tail consists of the cheapest
             // blocks (background) instead of whatever happens to be last in row-major order.
-            const uint32_t slot = b / NTR_BLOCKS_PER_TILE, sub = b % NTR_BLOCKS_PER_TILE;
+            uint32_t slot = b / NTR_BLOCKS_PER_TILE;
+            const uint32_t sub = b % NTR_BLOCKS_PER_TILE;
+            // a batch of views: block b is sub-block `sub` of tile slot `slot` in view `view`, tile-major with the views inner,
+            // so the 32 blocks of a tile in every view are handed out together, in the tile order of the schedule
+            // (view-major order, each view's tiles after the previous view's, measured 6.5 % slower on c4: DESIGN section 9)
+            if constexpr (VIEWS) { view = slot % f.n_views; slot /= f.n_views; }
             const uint32_t tile = f.tile_order ? __ldg(f.tile_order + slot) : slot;
             cost_tile = tile;
             if (f.tile_cost) t_start = clock64();
@@ -280,8 +288,15 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
             // output row of the block: frame position, or the compacted strip of this rank
             out_row0 = f.compact ? (tyi * NTR_TILE + (by - ty * NTR_TILE)) : by;
             pix = (uint32_t)(out_row0 + (lane >> 3)) * (uint32_t)f.win_w + (uint32_t)px;
+            if constexpr (VIEWS) pix += view * ((uint32_t)f.win_w * (uint32_t)f.out_rows);
             if (inside) {
-                if constexpr ((FLAGS & NTR_F_SS) != 0) {
+                if constexpr (VIEWS) {
+                    // the view's camera is read from global memory where it is used (by reference), not copied to registers;
+                    // at factor 1 the pixel gets the plain path's bits (ss_pixel_color, EXACT1)
+                    QueueEmit<DT> emit{q, ctl, pix, f.out_mode == NTR_OUT_ACCUM};
+                    ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true>(s, f.views[view], f, f.x0 + px, f.y0 + py,
+                                                                                                    acc, emit, cnt, &ms);
+                } else if constexpr ((FLAGS & NTR_F_SS) != 0) {
                     // supersampled frame: the lane traces the ss x ss samples of its pixel right here, one after the other
                     // (the loop count is the same for every lane); their bounces go to the next pass already weighted
                     QueueEmit<DT> emit{q, ctl, pix, f.out_mode == NTR_OUT_ACCUM};
@@ -323,7 +338,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
         // warp-synchronous form (trace_warp.cuh: all 32 lanes enter, `active` says who has a ray; rays park at big leaves
         // and the warp splits them over its lanes when enough lanes are idle) wins where single rays walk leaves of
         // hundreds of items (config 4: 58.4 -> 49.9 ms, its 1/8-frame share 26.3 -> 19.9 ms).
-        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE | NTR_F_SS);      // the per-ray code knows nothing of the switches
+        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE | NTR_F_SS | NTR_F_VIEWS);      // the per-ray code knows nothing of the switches
         if constexpr ((FLAGS & NTR_F_WARP) != 0) {
             if (s.kind != NTR_SCENE_BOX) {          // warp-uniform
                 if (!active) {
@@ -333,7 +348,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
                 QueueEmit<DT> emit{q, ctl, pix, !primary || f.out_mode == NTR_OUT_ACCUM};
                 ray_color_warp<DT, RF>(s, active, o, dir, depth, skip, w, acc, emit, cnt, &prim, done_ctr, &ms);
             }
-        } else if ((FLAGS & NTR_F_SS) == 0 && active) {
+        } else if ((FLAGS & (NTR_F_SS | NTR_F_VIEWS)) == 0 && active) {
             QueueEmit<DT> emit{q, ctl, pix, !primary || f.out_mode == NTR_OUT_ACCUM};
             ray_color<DT, RF>(s, active, o, dir, depth, skip, w, acc, emit, cnt, &prim, &ms);
         }
@@ -361,7 +376,9 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
             uint32_t pw[4] = {0, 0, 0, 0};
             if (inside) pack_pixel(f.fmt, acc, pw);
             const int ncols = min(NTR_BLK_W, f.win_w - bx), nrows = min(NTR_BLK_H, f.win_h - by);
-            store_block_packed(f, stage, bx, by, ncols, nrows, out_row0, pw, inside);
+            unsigned char *packed = f.packed;
+            if constexpr (VIEWS) packed += (size_t)view * (size_t)f.fmt.pitch * (size_t)f.win_h;
+            store_block_packed(f, packed, stage, bx, by, ncols, nrows, out_row0, pw, inside);
         } else if (inside) {
             if (f.out_mode == NTR_OUT_ACCUM) {
                 f.accum[(size_t)pix * 3 + 0] = acc[0]; f.accum[(size_t)pix * 3 + 1] = acc[1]; f.accum[(size_t)pix * 3 + 2] = acc[2];
@@ -494,9 +511,9 @@ template <int DT, int FLAGS> struct Launch {
     }
 };
 
-// defined in kern_d*.cu: variant index = FLAGS (0..63; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
-// everywhere else the index falls back to the build without it; NTR_F_SS and NTR_F_LIST builds exist in the per-lane,
-// non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE)
+// defined in kern_d*.cu: variant index = FLAGS (0..127; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
+// everywhere else the index falls back to the build without it; NTR_F_SS, NTR_F_LIST and NTR_F_VIEWS builds exist in the
+// per-lane, non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE)
 const KernelSet *kernel_set_d3(int flags);
 const KernelSet *kernel_set_d4(int flags);
 const KernelSet *kernel_set_d5(int flags);
@@ -513,8 +530,11 @@ const KernelSet *kernel_set_dn(int flags);
         if (flags & NTR_F_SS) return &ss[flags & 3];                                                     \
         static const KernelSet list[4] = {Launch<DT, NTR_F_LIST>::get(), Launch<DT, 1 | NTR_F_LIST>::get(), \
                                           Launch<DT, 2 | NTR_F_LIST>::get(), Launch<DT, 3 | NTR_F_LIST>::get()}; \
-        if (flags & NTR_F_LIST) return &list[flags & 3];
-#define NTR_INSTANTIATE_DIM(NAME, DT)                                                                   \
+        if (flags & NTR_F_LIST) return &list[flags & 3];                                                 \
+        static const KernelSet views[4] = {Launch<DT, NTR_F_VIEWS>::get(), Launch<DT, 1 | NTR_F_VIEWS>::get(), \
+                                           Launch<DT, 2 | NTR_F_VIEWS>::get(), Launch<DT, 3 | NTR_F_VIEWS>::get()}; \
+        if (flags & NTR_F_VIEWS) return &views[flags & 3];
+#define NTR_INSTANTIATE_DIM(NAME, DT)                                                                  \
     const KernelSet *NAME(int flags) {                                                                  \
         NTR_SS_SETS(DT)                                                                                 \
         static const KernelSet sets[8] = {Launch<DT, 0>::get(), Launch<DT, 1>::get(), Launch<DT, 2>::get(), \

@@ -1538,8 +1538,11 @@ NTR_HD float mul_rn(float a, float b) {
 #endif
 }
 
-// colour of output pixel (x, y) of a supersampled frame into sum[3]; samples go to the (per-lane) ray_color
-template <int DT, int FLAGS, typename EMIT>
+// colour of output pixel (x, y) of a supersampled frame into sum[3]; samples go to the (per-lane) ray_color.
+// EXACT1 (the primary pass of a batch of views, NTR_F_VIEWS, which runs factor 1 through here as well): at factor 1 the one
+// sample's colour is stored as it is, so that the pixel has the bits of the plain primary path -- 0.0f + c would turn a
+// negative zero into +0 (box_color stores -0 where the direction's gradient axis is +0; tests/test_views.py)
+template <int DT, int FLAGS, typename EMIT, bool EXACT1 = false>
 NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, float *sum,
                            EMIT &emit, Counters &cnt, MailboxStore *ms) {
     constexpr int CAP = DimCap<DT>::value;
@@ -1559,7 +1562,8 @@ NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameD
         } else {
             ray_color<DT, FLAGS>(s, true, o, dir, 0, none, w, c, emit, cnt, nullptr, ms);
         }
-        sum[0] = add_rn(sum[0], c[0]); sum[1] = add_rn(sum[1], c[1]); sum[2] = add_rn(sum[2], c[2]);
+        if (EXACT1 && ss == 1) { sum[0] = c[0]; sum[1] = c[1]; sum[2] = c[2]; }
+        else { sum[0] = add_rn(sum[0], c[0]); sum[1] = add_rn(sum[1], c[1]); sum[2] = add_rn(sum[2], c[2]); }
     }
 }
 

@@ -299,6 +299,43 @@ class BlockingRenderer:
         finally:
             self._lock.release()
 
+    def render_views(self, dest, format, scene, cameras):
+        """Extension without a reference counterpart: one frame per camera in one call, frame k at byte offset
+        k * pitch * height of `dest` (ntr_render_views).  Frame k is what render() gives after scene.set_camera(cameras[k]);
+        the scene's camera is left as it is.  cameras: Camera objects of the scene's dimension or (origin, axes) pairs
+        (stream.rotation_cameras).  With threads > 1 (or NTR_GPUS) whole views are dealt to the GPUs.
+        -> True, or False if signal_abort() was called while rendering."""
+        from .backend import camera_arrays
+        if not isinstance(format, ImageFormat):
+            raise TypeError('object is not an instance of ImageFormat')
+        if not isinstance(scene, Scene):
+            raise TypeError('object is not an instance of Scene')
+        origins, axes = camera_arrays(cameras, scene.dimension)
+        n = len(origins)
+        buf = _writable_buffer(dest)
+        fmt = format._native()
+        if buf.size < n * fmt.pitch * fmt.height:
+            raise ValueError('the buffer is too small for %d images with the given dimensions' % n)
+        if not self._lock.acquire(blocking=False):
+            raise RuntimeError('the renderer is already running')
+        try:
+            scene.locked += 1
+            try:
+                dev = scene._prepare(self._gpus) if self._gpus > 1 else scene._prepare()
+                self._dev = dev
+                fn = dev._lib.ntr_group_render_views if hasattr(dev, 'size') else dev._lib.ntr_render_views
+                rc = fn(dev._h, n, origins.ctypes.data_as(C.c_void_p), axes.ctypes.data_as(C.c_void_p), C.byref(fmt),
+                        buf.ctypes.data_as(C.c_void_p), buf.size)
+                if rc == _capi.NTR_ERR_ABORTED:
+                    return False
+                _capi.check(rc)
+                return True
+            finally:
+                self._dev = None
+                scene.locked -= 1
+        finally:
+            self._lock.release()
+
     def signal_abort(self):
         dev = self._dev
         if dev is not None:
