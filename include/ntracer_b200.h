@@ -233,6 +233,32 @@ NTR_API int ntr_render_views(ntr_scene *scene, int n, const float *origins, cons
  * asynchronous when the frames need a single pass, synchronous on that stream with reflection passes, as ntr_render_device. */
 NTR_API int ntr_render_views_device(ntr_scene *scene, int n, const float *origins, const float *axes,
                                     const ntr_image_format *fmt, void *dev_dst, size_t dst_len, void *stream);
+/* Per-pixel auxiliary outputs (AOVs) of a views call (no counterpart in the reference).  For view k and output pixel (x, y),
+ * at index (k*height + y)*width + x, they describe the pixel's plain primary ray -- the factor-1 ray ntr_primary_hit_ids
+ * traces after ntr_scene_set_camera(origins[k], axes[k]) -- whatever the supersampling factor or threshold:
+ *   ids      the flat id of its opaque hit as ntr_primary_hit_ids defines it (-1: a miss; transparent layers are not hits),
+ *   depth    its distance along the ray (0 on a miss), both bit-identical to ntr_primary_hit_ids,
+ *   normals  dim floats per pixel: the normal that shades the hit (RayIntersection.normal of the reference: a simplex's unit
+ *            face normal facing the ray, a solid's back-transformed normal as it is, a BoxScene face's axis vector), zeros
+ *            on a miss.
+ * A NULL pointer means "not wanted"; each *_len counts elements (n*width*height, times dim for the normals). */
+typedef struct ntr_aov_buffers {
+    int32_t *ids;
+    float *depth;
+    float *normals;
+    size_t ids_len, depth_len, normals_len;
+} ntr_aov_buffers;
+/* ntr_render_views plus the AOVs in the same launches, into host memory; the frames and counters are those of ntr_render_views
+ * (the rays traced for the AOVs are not counted).  aovs == NULL or all three NULL is ntr_render_views.  A launch then covers
+ * at most as many views as keep its AOVs within about 1 GB (NTR_VIEWS_PER_LAUNCH still overrides).  NTR_ERR_VALUE also for
+ * a short AOV buffer, checked before any work; after NTR_ERR_ABORTED the AOVs' contents are unspecified. */
+NTR_API int ntr_render_views_aovs(ntr_scene *scene, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                                  void *dst, size_t dst_len, const ntr_aov_buffers *aovs);
+/* The same with the frames and the AOVs in DEVICE memory of the scene's device, on a caller-supplied stream, as
+ * ntr_render_views_device. */
+NTR_API int ntr_render_views_aovs_device(ntr_scene *scene, int n, const float *origins, const float *axes,
+                                         const ntr_image_format *fmt, void *dev_dst, size_t dst_len,
+                                         const ntr_aov_buffers *dev_aovs, void *stream);
 /* Float RGB of every pixel (3 floats per pixel, row-major) = scene::calculate_color for the whole
  * view (src/render.hpp:12-13) before channel packing; host destination. */
 NTR_API int ntr_render_float(ntr_scene *scene, int width, int height, float *dst_rgb);
@@ -293,6 +319,9 @@ NTR_API int ntr_group_render_device(ntr_group *group, const ntr_image_format *fm
  * ntr_group_last_kernel_ms is the slowest entry's.  With a supersampling threshold set, view after view via ntr_group_render. */
 NTR_API int ntr_group_render_views(ntr_group *group, int n, const float *origins, const float *axes,
                                    const ntr_image_format *fmt, void *dst, size_t dst_len);
+/* ntr_render_views_aovs over the group: every entry writes the frames and AOVs of its own views straight to their place. */
+NTR_API int ntr_group_render_views_aovs(ntr_group *group, int n, const float *origins, const float *axes,
+                                        const ntr_image_format *fmt, void *dst, size_t dst_len, const ntr_aov_buffers *aovs);
 NTR_API int ntr_group_abort(ntr_group *group);
 /* Counters of the last frame summed over the devices; device time of the last frame from the first kernel to the last
  * one of the slowest device (CUDA events on the first device's stream, which waits for the others). */

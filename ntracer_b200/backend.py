@@ -58,6 +58,38 @@ def _views_dest(dest, n, fmt):
     return dest, buf
 
 
+AOV_NAMES = ('ids', 'depth', 'normals')
+AOV_DTYPES = {'ids': np.int32, 'depth': np.float32, 'normals': np.float32}
+
+
+def aov_shape(name, n, fmt, dim):
+    """shape of AOV `name` of n views: (n, height, width), and (n, height, width, dim) for the normals"""
+    return (n, fmt.height, fmt.width) + ((dim,) if name == 'normals' else ())
+
+
+def _aov_names(aovs):
+    names = tuple(aovs)
+    for name in names:
+        if name not in AOV_NAMES:
+            raise ValueError('unknown AOV %r (known: %s)' % (name, ', '.join(AOV_NAMES)))
+    return names
+
+
+def aov_struct(ptrs):
+    """{name: (address, length in elements)} -> _capi.AovBuffers (the AOVs not named are not wanted)"""
+    a = _capi.AovBuffers()
+    for name, (ptr, length) in ptrs.items():
+        setattr(a, name, ptr)
+        setattr(a, name + '_len', int(length))
+    return a
+
+
+def _new_aovs(aovs, n, fmt, dim):
+    """-> ({name: new array}, AovBuffers over them)"""
+    arrays = {name: np.zeros(aov_shape(name, n, fmt, dim), AOV_DTYPES[name]) for name in _aov_names(aovs)}
+    return arrays, aov_struct({k: (v.ctypes.data, v.size) for k, v in arrays.items()})
+
+
 def _refine_mask(fn, handle, w, h):
     mask = np.zeros((h, w), dtype=np.uint8)
     count = C.c_uint64(0)
@@ -164,6 +196,34 @@ class DeviceScene:
         self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_render_views_device(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt),
                                                       C.c_void_p(dev_ptr), int(nbytes), C.c_void_p(stream)))
+
+    def render_views_aovs(self, fmt, cameras, aovs=AOV_NAMES, dest=None):
+        """render_views plus per-pixel AOVs of every view in the same launches (ntr_render_views_aovs) -> (frames, {name:
+        array}) for the names in `aovs`: 'ids' int32 (n, height, width), the flat id of the plain primary ray's opaque hit
+        (-1: a miss) as primary_hit_ids gives it; 'depth' float32 (n, height, width), its distance (0 on a miss); 'normals'
+        float32 (n, height, width, dim), the normal that shades the hit (zeros on a miss).  Frames and counters are those of
+        render_views."""
+        origins, axes = camera_arrays(cameras, self.dim)
+        out, buf = _views_dest(dest, len(origins), fmt)
+        arrays, a = _new_aovs(aovs, len(origins), fmt, self.dim)
+        self._window = (fmt.width, fmt.height)
+        _capi.check(self._lib.ntr_render_views_aovs(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt), _p(buf), buf.size,
+                                                    C.byref(a)))
+        return out, arrays
+
+    def render_views_aovs_device(self, fmt, cameras, dev_ptr, nbytes, aovs, stream=0):
+        """render_views_aovs into device memory on a CUDA stream handle: the frames as render_views_device, `aovs` maps AOV
+        names to torch tensors on the scene's device (int32 ids, float32 depth and normals, in render_views_aovs's shapes) or
+        to (device address, length in elements) pairs."""
+        origins, axes = camera_arrays(cameras, self.dim)
+        ptrs = {}
+        for name in _aov_names(aovs):
+            t = aovs[name]
+            ptrs[name] = (t.data_ptr(), t.numel()) if hasattr(t, 'data_ptr') else (int(t[0]), int(t[1]))
+        a = aov_struct(ptrs)
+        self._window = (fmt.width, fmt.height)
+        _capi.check(self._lib.ntr_render_views_aovs_device(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt),
+                                                           C.c_void_p(dev_ptr), int(nbytes), C.byref(a), C.c_void_p(stream)))
 
     def render_begin(self, fmt, dest):
         """Enqueue one frame with the current camera and return a ticket (the interactive loop: frame k+1 is traced
@@ -339,6 +399,17 @@ class DeviceGroup:
         self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_group_render_views(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt), _p(buf), buf.size))
         return out
+
+    def render_views_aovs(self, fmt, cameras, aovs=AOV_NAMES, dest=None):
+        """DeviceScene.render_views_aovs over the group: every device writes the frames and AOVs of its own views
+        (ntr_group_render_views_aovs)."""
+        origins, axes = camera_arrays(cameras, self.dim)
+        out, buf = _views_dest(dest, len(origins), fmt)
+        arrays, a = _new_aovs(aovs, len(origins), fmt, self.dim)
+        self._window = (fmt.width, fmt.height)
+        _capi.check(self._lib.ntr_group_render_views_aovs(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt), _p(buf),
+                                                          buf.size, C.byref(a)))
+        return out, arrays
 
     def render_device(self, fmt):
         """-> address of the frame on the first device (valid until the next render)"""

@@ -75,6 +75,8 @@ __global__ void ring_bounds_kernel(const uint32_t *sorted_keys, uint32_t n, cons
 struct FrameSlot {
     unsigned char *d_buf = nullptr; size_t d_cap = 0;
     unsigned char *h_stage = nullptr; size_t h_cap = 0;
+    unsigned char *d_aov = nullptr; size_t d_aov_cap = 0;          // AOVs of a views launch (device) and their pinned staging
+    unsigned char *h_aov = nullptr; size_t h_aov_cap = 0;
     cudaEvent_t rendered = nullptr, copied = nullptr;
     unsigned char *dst = nullptr;
     size_t pitch = 0, row_bytes = 0;
@@ -181,7 +183,7 @@ struct ntr_scene {
     uint32_t *h_ctl = nullptr;              // pinned read-back of the control block and the counters (frame_readback)
     unsigned long long *h_cnt = nullptr;
     uint64_t launches = 0;
-    int grid_blocks[128] = {};         // per variant flags (NTR_F_SS, NTR_F_LIST and NTR_F_VIEWS included)
+    int grid_blocks[256] = {};         // per variant flags (NTR_F_SS, NTR_F_LIST, NTR_F_VIEWS and NTR_F_AOV included)
     // NTR_F_WIDE builds (96 registers, 5 CTAs per SM): for frames sharded over 4 or more GPUs, whose passes all end in a few
     // long rays (measured, config 4: 1/4 share 20.9 -> 19.9 ms, 1/8 share 15.2 -> 14.4 ms; 1/2 share and whole frames lose
     // 2..12 %).  Picking the build per pass from pass times measured on the second and third frame of a view gained another
@@ -381,12 +383,39 @@ int check_format(const ntr_image_format *f) {
     return NTR_OK;
 }
 
+// The AOVs of a batch of views (ntr_aov_buffers): p[k] is where kind k of view 0 goes (nullptr: not wanted), kind k taking
+// aov_bytes(k, dim) bytes per pixel -- 0 ids (int32), 1 depth (float), 2 normals (dim floats)
+struct AovTarget {
+    void *p[3] = {nullptr, nullptr, nullptr};
+    bool any() const { return p[0] || p[1] || p[2]; }
+};
+static size_t aov_bytes(int k, int dim) { return k == 2 ? 4 * (size_t)dim : 4; }
+// bytes per pixel of the AOVs wanted
+static size_t aov_pixel_bytes(const AovTarget &a, int dim) {
+    size_t b = 0;
+    for (int k = 0; k < 3; ++k) if (a.p[k]) b += aov_bytes(k, dim);
+    return b;
+}
+// a's arrays from pixel `pix` on
+static AovTarget aov_offset(const AovTarget &a, size_t pix, int dim) {
+    AovTarget o;
+    for (int k = 0; k < 3; ++k) if (a.p[k]) o.p[k] = static_cast<unsigned char *>(a.p[k]) + pix * aov_bytes(k, dim);
+    return o;
+}
+// the arrays of `want` for npix pixels laid out one after the other in buf
+static AovTarget aov_packed(unsigned char *buf, const AovTarget &want, size_t npix, int dim) {
+    AovTarget o;
+    for (int k = 0; k < 3; ++k) if (want.p[k]) { o.p[k] = buf; buf += npix * aov_bytes(k, dim); }
+    return o;
+}
+
 struct RenderTarget {
     int out_mode;               // what the caller wants
     unsigned char *packed = nullptr;
     float *accum = nullptr;
     int32_t *ids = nullptr;
     float *dists = nullptr;
+    AovTarget aov;              // a batch of views only: its AOVs (device memory), traced by the NTR_F_AOV build
 };
 
 // Supersampling factor of a frame: the hit-id hook traces one ray per pixel whatever the scene's factor
@@ -441,6 +470,16 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     f.tile_row_first = tile_row_first; f.tile_row_step = tile_row_step < 1 ? 1 : tile_row_step; f.compact = compact;
     if (fmt) fill_format(f.fmt, fmt);
     f.views = views; f.n_views = n_views;
+    const bool aov = n_views && tgt.aov.any();
+    if (aov) {
+        f.aov_ids = static_cast<int32_t *>(tgt.aov.p[0]);
+        f.aov_depth = static_cast<float *>(tgt.aov.p[1]);
+        f.aov_normals = static_cast<float *>(tgt.aov.p[2]);
+        // the plain frame's ray parameters, as ntr_primary_hit_ids sets them (factor 1)
+        f.aov_half_w = (float)width / 2.0f;
+        f.aov_half_h = (float)height / 2.0f;
+        f.aov_fovI = tanf(sc->dev.fov / 2) / f.aov_half_w;
+    }
     const size_t nv = n_views ? n_views : 1;
     // wavefront statistics of the previous frame (of the previous views call, for a batch of views)
     float &pass_ns_per_ray = n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray;
@@ -546,7 +585,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     // a supersampled primary pass runs the per-lane, non-wide NTR_F_SS build whatever NTR_WARP / NTR_WIDE say (kernels.cuh)
     // a batch of views runs the per-lane, non-wide NTR_F_VIEWS build at every factor, 1 included; no more CTAs than the exact
     // mailbox has columns
-    const int pflags = n_views ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_VIEWS
+    const int pflags = n_views ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_VIEWS | (aov ? NTR_F_AOV : 0)
                        : ss > 1 ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_SS : primary_flags | wide_for(0);
     const KernelSet *ks = sc->kset(pflags);
     int grid = grid_for(sc, pflags);
@@ -1205,6 +1244,8 @@ NTR_API void ntr_scene_destroy(ntr_scene *sc) {
     for (FrameSlot &fs : sc->slots) {
         cudaFree(fs.d_buf);
         if (fs.h_stage) cudaFreeHost(fs.h_stage);
+        cudaFree(fs.d_aov);
+        if (fs.h_aov) cudaFreeHost(fs.h_aov);
         if (fs.rendered) cudaEventDestroy(fs.rendered);
         if (fs.copied) cudaEventDestroy(fs.copied);
     }
@@ -1477,12 +1518,16 @@ NTR_API int ntr_render_end(ntr_scene *sc, uint64_t ticket) {
 // traced sample, 2^26 records at the cap, which is the size the queues of a single frame are capped at already
 // (enqueue_frame; 4 GB per queue in 4 dimensions); the accumulator then holds at most 2^25 pixels (384 MB) and the device
 // frames of a launch V * pitch * H bytes, twice over (one launch is traced while the previous one is copied).
-// At 1920x1080 that is 16 views per launch, at 640x480 109.  NTR_VIEWS_PER_LAUNCH=n overrides V (tests).
+// At 1920x1080 that is 16 views per launch, at 640x480 109.  With AOVs, V also keeps a launch's AOVs, V * W * H * (bytes per
+// pixel: 8 + 4 * dim for all three), at or below kViewsAovCap = 1 GB (they are held twice, as the frames are).
+// NTR_VIEWS_PER_LAUNCH=n overrides V (tests).
 static const uint64_t kViewsSampleCap = 1ull << 25;
+static const uint64_t kViewsAovCap = 1ull << 30;
 
-static int views_per_launch(const ntr_scene *sc, const ntr_image_format *fmt, int n) {
+static int views_per_launch(const ntr_scene *sc, const ntr_image_format *fmt, int n, size_t aov_px) {
     const uint64_t npix = (uint64_t)fmt->width * fmt->height, ss = (uint64_t)sc->ss;
     uint64_t v = sc->views_per_launch ? sc->views_per_launch : kViewsSampleCap / (npix * ss * ss);
+    if (aov_px && !sc->views_per_launch) v = std::min<uint64_t>(v, kViewsAovCap / (npix * aov_px));
     v = std::min<uint64_t>(v, 0x7FFFFFFFull / npix);        // pixel indices v * npix + pix stay below 2^31
     return (int)std::max<uint64_t>(1, std::min<uint64_t>(v, (uint64_t)n));
 }
@@ -1517,28 +1562,60 @@ static int check_views(const ntr_scene *sc, int n, const float *origins, const f
     return NTR_OK;
 }
 
+// the AOV buffers of a views call -> *out (all nullptr for a NULL `aovs`); NTR_ERR_VALUE for a short one
+static int check_aovs(int n, const ntr_image_format *fmt, int dim, const ntr_aov_buffers *aovs, AovTarget *out) {
+    *out = AovTarget{};
+    if (!aovs) return NTR_OK;
+    const size_t npix = (size_t)n * fmt->width * fmt->height;
+    const void *p[3] = {aovs->ids, aovs->depth, aovs->normals};
+    const size_t len[3] = {aovs->ids_len, aovs->depth_len, aovs->normals_len}, per[3] = {1, 1, (size_t)dim};
+    static const char *const name[3] = {"ids", "depth", "normals"};
+    for (int k = 0; k < 3; ++k) {
+        if (!p[k]) continue;
+        if (len[k] / per[k] < npix) return fail(NTR_ERR_VALUE, "the %s buffer is too small for %d views", name[k], n);
+        out->p[k] = const_cast<void *>(p[k]);
+    }
+    return NTR_OK;
+}
+
+// true when every AOV destination wanted is pinned (or registered) host memory
+static bool aovs_pinned(const AovTarget &a) {
+    for (int k = 0; k < 3; ++k) {
+        if (!a.p[k]) continue;
+        cudaPointerAttributes attr;
+        const bool pinned = cudaPointerGetAttributes(&attr, a.p[k]) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+        cudaGetLastError();
+        if (!pinned) return false;
+    }
+    return true;
+}
+
 // One scene's share of a views call: its cameras on the device and its launches.  Frames into host memory (`host`) are traced
 // into the device buffer of frame slot k % 2 and cross PCIe on the copy stream while launch k + 1 is traced; a pageable
 // destination gets them through the slot's pinned staging buffer, which the host empties while the next launch runs.
-// Frames into device memory are stored in place.
+// Frames into device memory are stored in place.  The AOVs take the same way as the frames: into the slot's device buffer, then
+// across PCIe behind the frames (through the slot's pinned staging buffer when a destination is pageable), or in place.
 struct ViewsRun {
     ntr_scene *sc = nullptr;
     const ntr_image_format *fmt = nullptr;
     int n = 0, per = 1;                 // views of the run, views per launch
     unsigned char *dst = nullptr;       // frame 0 of the run
+    AovTarget aov;                      // the AOVs of view 0 of the run (none wanted: all nullptr)
     cudaStream_t st = nullptr;
-    bool host = false, staged = false;
+    bool host = false, staged = false, aov_staged = false;
     int done = 0, k = 0;                // views and launches finished
     FrameJob j{};                       // the launch in flight
     int unstage_slot = -1, unstage_first = 0, unstage_n = 0;     // a staged launch whose frames are still to reach dst
     ntr_counters sum{};
     size_t frame_bytes() const { return (size_t)fmt->pitch * fmt->height; }
+    size_t frame_pixels() const { return (size_t)fmt->width * fmt->height; }
 };
 
 static int views_begin(ViewsRun &r, const float *origins, const float *axes) {
     ntr_scene *sc = r.sc;
     if (r.n < 1) return NTR_OK;
-    r.per = views_per_launch(sc, r.fmt, r.n);
+    const size_t aov_px = aov_pixel_bytes(r.aov, sc->dev.dim);
+    r.per = views_per_launch(sc, r.fmt, r.n, aov_px);
     std::vector<CameraDev> cams(r.n);
     for (int k = 0; k < r.n; ++k) view_camera(cams[k], origins, axes, sc->dev.dim, k);
     // an asynchronous views call on another stream may still be reading the previous cameras
@@ -1558,6 +1635,13 @@ static int views_begin(ViewsRun &r, const float *origins, const float *axes) {
             CUDA_TRY(cudaHostAlloc((void **)&fs.h_stage, bytes + bytes / 8, cudaHostAllocDefault));
             fs.h_cap = bytes + bytes / 8;
         }
+        const size_t abytes = (size_t)r.per * r.frame_pixels() * aov_px;
+        if (abytes && (rc = ensure((void **)&fs.d_aov, &fs.d_aov_cap, abytes))) return rc;
+        if (abytes && r.aov_staged && fs.h_aov_cap < abytes) {
+            if (fs.h_aov) { cudaFreeHost(fs.h_aov); fs.h_aov = nullptr; fs.h_aov_cap = 0; }
+            CUDA_TRY(cudaHostAlloc((void **)&fs.h_aov, abytes, cudaHostAllocDefault));
+            fs.h_aov_cap = abytes;
+        }
     }
     return NTR_OK;
 }
@@ -1571,8 +1655,16 @@ static int views_unstage(ViewsRun &r) {
     const size_t pitch = (size_t)r.fmt->pitch, row_bytes = (size_t)r.fmt->width * r.fmt->bytes_per_pixel;
     unsigned char *to = r.dst + (size_t)r.unstage_first * r.frame_bytes();
     const size_t rows = (size_t)r.unstage_n * r.fmt->height;
-    if (row_bytes == pitch) memcpy(to, fs.h_stage, rows * pitch);
-    else for (size_t y = 0; y < rows; ++y) memcpy(to + y * pitch, fs.h_stage + y * pitch, row_bytes);
+    if (r.staged) {
+        if (row_bytes == pitch) memcpy(to, fs.h_stage, rows * pitch);
+        else for (size_t y = 0; y < rows; ++y) memcpy(to + y * pitch, fs.h_stage + y * pitch, row_bytes);
+    }
+    if (r.aov_staged) {
+        const int D = r.sc->dev.dim;
+        const size_t npix = (size_t)r.unstage_n * r.frame_pixels();
+        const AovTarget from = aov_packed(fs.h_aov, r.aov, npix, D), into = aov_offset(r.aov, (size_t)r.unstage_first * r.frame_pixels(), D);
+        for (int k = 0; k < 3; ++k) if (into.p[k]) memcpy(into.p[k], from.p[k], npix * aov_bytes(k, D));
+    }
     return NTR_OK;
 }
 
@@ -1586,8 +1678,10 @@ static int views_submit(ViewsRun &r) {
         FrameSlot &fs = sc->slots[r.k & 1];
         CUDA_TRY(cudaStreamWaitEvent(r.st, fs.copied, 0));         // the launch before the last one has left the buffer
         tgt.packed = fs.d_buf;
+        tgt.aov = aov_packed(fs.d_aov, r.aov, (size_t)cnt * r.frame_pixels(), sc->dev.dim);
     } else {
         tgt.packed = r.dst + (size_t)r.done * r.frame_bytes();
+        tgt.aov = aov_offset(r.aov, (size_t)r.done * r.frame_pixels(), sc->dev.dim);
     }
     r.j = FrameJob{r.fmt->width, r.fmt->height, 0, 0, r.fmt->width, r.fmt->height, r.fmt, tgt, 0, 1, 0, r.st};
     r.j.views = sc->d_views + r.done;
@@ -1616,8 +1710,14 @@ static int views_collect(ViewsRun &r, bool *again) {
         unsigned char *to = r.staged ? fs.h_stage : r.dst + (size_t)r.done * r.frame_bytes();
         // only the pixel bytes are written, like process_pixel: the pitch padding of `dst` is left alone
         CUDA_TRY(cudaMemcpy2DAsync(to, pitch, fs.d_buf, pitch, row_bytes, (size_t)cnt * r.fmt->height, cudaMemcpyDeviceToHost, sc->copy_stream));
+        const int D = sc->dev.dim;
+        const size_t npix = (size_t)cnt * r.frame_pixels();
+        const AovTarget from = aov_packed(fs.d_aov, r.aov, npix, D);
+        const AovTarget into = r.aov_staged ? aov_packed(fs.h_aov, r.aov, npix, D) : aov_offset(r.aov, (size_t)r.done * r.frame_pixels(), D);
+        for (int k = 0; k < 3; ++k)
+            if (into.p[k]) CUDA_TRY(cudaMemcpyAsync(into.p[k], from.p[k], npix * aov_bytes(k, D), cudaMemcpyDeviceToHost, sc->copy_stream));
         CUDA_TRY(cudaEventRecord(fs.copied, sc->copy_stream));
-        if (r.staged) { r.unstage_slot = slot; r.unstage_first = r.done; r.unstage_n = cnt; }
+        if (r.staged || r.aov_staged) { r.unstage_slot = slot; r.unstage_first = r.done; r.unstage_n = cnt; }
     }
     r.done += cnt;
     ++r.k;
@@ -1649,10 +1749,50 @@ static int views_run(ViewsRun &r, const float *origins, const float *axes) {
     return views_finish(r, rc);
 }
 
+// The AOVs of view k of an adaptively supersampled views call into `into` (device memory of the scene's device): a one-view
+// NTR_F_AOV launch at factor 1 whose frame is thrown away.  The scene's factor, threshold, counters and refine-mask record are
+// put back afterwards, so the call's frames, masks and counters are those of the call without AOVs.
+static int views_aov_pass(ntr_scene *sc, const float *origins, const float *axes, int k, const ntr_image_format *fmt,
+                          const AovTarget &into, cudaStream_t st) {
+    const int D = sc->dev.dim;
+    int rc = ensure((void **)&sc->d_packed, &sc->packed_cap, (size_t)fmt->pitch * fmt->height);
+    if (rc) return rc;
+    const int ss = sc->ss;
+    const float threshold = sc->ss_threshold;
+    const ntr_counters counters = sc->counters;
+    const auto last = sc->last;
+    sc->ss = 1; sc->ss_threshold = -1.0f;
+    ViewsRun r;
+    r.sc = sc; r.fmt = fmt; r.n = 1; r.dst = sc->d_packed; r.aov = into; r.st = st;
+    rc = views_run(r, origins + (size_t)k * D, axes + (size_t)k * D * D);
+    sc->ss = ss; sc->ss_threshold = threshold; sc->counters = counters; sc->last = last;
+    return rc;
+}
+
+// views_aov_pass for view k into host or device destinations (view 0 of them at `dst`); host ones go through the AOV buffer of
+// frame slot 0
+static int views_aovs_of(ntr_scene *sc, const float *origins, const float *axes, int k, const ntr_image_format *fmt,
+                         const AovTarget &dst, bool device, cudaStream_t st) {
+    const int D = sc->dev.dim;
+    const size_t npix = (size_t)fmt->width * fmt->height;
+    const AovTarget into = aov_offset(dst, (size_t)k * npix, D);
+    if (device) return views_aov_pass(sc, origins, axes, k, fmt, into, st);
+    FrameSlot &fs = sc->slots[0];
+    int rc = ensure((void **)&fs.d_aov, &fs.d_aov_cap, npix * aov_pixel_bytes(dst, D));
+    if (rc) return rc;
+    const AovTarget scratch = aov_packed(fs.d_aov, dst, npix, D);
+    if ((rc = views_aov_pass(sc, origins, axes, k, fmt, scratch, st))) return rc;
+    for (int c = 0; c < 3; ++c)
+        if (into.p[c]) CUDA_TRY(cudaMemcpyAsync(into.p[c], scratch.p[c], npix * aov_bytes(c, D), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return NTR_OK;
+}
+
 // Adaptively supersampled views: one after the other through the single-view route (ntr_render / ntr_render_device), each
-// with its camera; the scene's own camera is put back afterwards and the counters are the sums over the views.
+// with its camera; the scene's own camera is put back afterwards and the counters are the sums over the views.  AOVs come from
+// views_aov_pass, view by view.
 static int views_one_by_one(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
-                            unsigned char *dst, bool device, cudaStream_t st) {
+                            unsigned char *dst, bool device, cudaStream_t st, const AovTarget &aov) {
     const CameraDev saved = sc->cam;
     const size_t fb = (size_t)fmt->pitch * fmt->height;
     ntr_counters sum{};
@@ -1662,38 +1802,54 @@ static int views_one_by_one(ntr_scene *sc, int n, const float *origins, const fl
         rc = device ? render_device_locked(sc, fmt, dst + k * fb, fb, st, 0, 1, 0) : render_locked(sc, fmt, dst + k * fb, fb);
         add_counters(sum, sc->counters);
         sum.queue_overflows = sc->counters.queue_overflows;
+        if (!rc && aov.any()) rc = views_aovs_of(sc, origins, axes, k, fmt, aov, device, st);
     }
     sc->cam = saved;
     if (!rc) sc->counters = sum;
     return rc;
 }
 
-NTR_API int ntr_render_views(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
-                             void *dst, size_t dst_len) {
-    ENTER(sc);
+static int render_views_host(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                             void *dst, size_t dst_len, const ntr_aov_buffers *aovs) {
     int rc = check_views(sc, n, origins, axes, fmt, dst, dst_len);
+    AovTarget aov;
+    if (!rc) rc = check_aovs(n, fmt, sc->dev.dim, aovs, &aov);
     if (rc) return rc;
     if (frame_adaptive(sc, NTR_OUT_PACKED))
-        return views_one_by_one(sc, n, origins, axes, fmt, static_cast<unsigned char *>(dst), false, sc->stream);
+        return views_one_by_one(sc, n, origins, axes, fmt, static_cast<unsigned char *>(dst), false, sc->stream, aov);
     cudaPointerAttributes attr;
     const bool pinned = cudaPointerGetAttributes(&attr, dst) == cudaSuccess && attr.type == cudaMemoryTypeHost;
     cudaGetLastError();
     ViewsRun r;
     r.sc = sc; r.fmt = fmt; r.n = n; r.dst = static_cast<unsigned char *>(dst); r.st = sc->stream;
     r.host = true; r.staged = !pinned;
+    r.aov = aov; r.aov_staged = aov.any() && !aovs_pinned(aov);
     return views_run(r, origins, axes);
 }
 
-NTR_API int ntr_render_views_device(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
-                                    void *dev_dst, size_t dst_len, void *stream) {
+NTR_API int ntr_render_views(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                             void *dst, size_t dst_len) {
     ENTER(sc);
+    return render_views_host(sc, n, origins, axes, fmt, dst, dst_len, nullptr);
+}
+
+NTR_API int ntr_render_views_aovs(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                                  void *dst, size_t dst_len, const ntr_aov_buffers *aovs) {
+    ENTER(sc);
+    return render_views_host(sc, n, origins, axes, fmt, dst, dst_len, aovs);
+}
+
+static int render_views_device(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                               void *dev_dst, size_t dst_len, const ntr_aov_buffers *aovs, void *stream) {
     int rc = check_views(sc, n, origins, axes, fmt, dev_dst, dst_len);
+    AovTarget aov;
+    if (!rc) rc = check_aovs(n, fmt, sc->dev.dim, aovs, &aov);
     if (rc) return rc;
     cudaStream_t st = stream ? (cudaStream_t)stream : sc->stream;
     if (frame_adaptive(sc, NTR_OUT_PACKED))
-        return views_one_by_one(sc, n, origins, axes, fmt, static_cast<unsigned char *>(dev_dst), true, st);
+        return views_one_by_one(sc, n, origins, axes, fmt, static_cast<unsigned char *>(dev_dst), true, st, aov);
     ViewsRun r;
-    r.sc = sc; r.fmt = fmt; r.n = n; r.dst = static_cast<unsigned char *>(dev_dst); r.st = st;
+    r.sc = sc; r.fmt = fmt; r.n = n; r.dst = static_cast<unsigned char *>(dev_dst); r.st = st; r.aov = aov;
     const bool passes = sc->dev.kind == NTR_SCENE_COMPOSITE && sc->any_reflective && sc->dev.max_depth > 0;
     if (passes) return views_run(r, origins, axes);         // synchronous on `st`, as ntr_render_device with passes
     // single-pass views: every launch fully asynchronous on the caller's stream
@@ -1704,6 +1860,7 @@ NTR_API int ntr_render_views_device(ntr_scene *sc, int n, const float *origins, 
         RenderTarget tgt;
         tgt.out_mode = NTR_OUT_PACKED;
         tgt.packed = r.dst + (size_t)first * r.frame_bytes();
+        tgt.aov = aov_offset(aov, (size_t)first * r.frame_pixels(), sc->dev.dim);
         bool p = false;
         if ((rc = enqueue_frame(sc, st, fmt->width, fmt->height, 0, 0, fmt->width, fmt->height, fmt, tgt, 0, 1, 0, &p,
                                 sc->d_views + first, (uint32_t)cnt))) return rc;
@@ -1713,6 +1870,19 @@ NTR_API int ntr_render_views_device(ntr_scene *sc, int n, const float *origins, 
     sc->counters = ntr_counters{};
     sc->counters.primary_rays = (uint64_t)n * fmt->width * fmt->height * sc->ss * sc->ss;
     return NTR_OK;
+}
+
+NTR_API int ntr_render_views_device(ntr_scene *sc, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                                    void *dev_dst, size_t dst_len, void *stream) {
+    ENTER(sc);
+    return render_views_device(sc, n, origins, axes, fmt, dev_dst, dst_len, nullptr, stream);
+}
+
+NTR_API int ntr_render_views_aovs_device(ntr_scene *sc, int n, const float *origins, const float *axes,
+                                         const ntr_image_format *fmt, void *dev_dst, size_t dst_len,
+                                         const ntr_aov_buffers *dev_aovs, void *stream) {
+    ENTER(sc);
+    return render_views_device(sc, n, origins, axes, fmt, dev_dst, dst_len, dev_aovs, stream);
 }
 
 NTR_API int ntr_render_float(ntr_scene *sc, int width, int height, float *dst_rgb) {
@@ -2160,10 +2330,12 @@ NTR_API int ntr_group_render(ntr_group *g, const ntr_image_format *fmt, void *ds
 // Views dealt to the entries in contiguous runs: entry i traces views [i * n / G, (i + 1) * n / G) with the batched kernels
 // into its own device memory and copies its frames straight to their place in dst.  Every round submits the next launch on
 // every entry before it collects any, so that all devices trace at once.
-NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
-                                   void *dst, size_t dst_len) {
+static int group_render_views(ntr_group *g, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                              void *dst, size_t dst_len, const ntr_aov_buffers *aovs) {
     if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
     for (ntr_scene *sc : g->sc) { const int rc = check_views(sc, n, origins, axes, fmt, dst, dst_len); if (rc) return rc; }
+    AovTarget aov;
+    if (const int rc = check_aovs(n, fmt, g->sc[0]->dev.dim, aovs, &aov)) return rc;
     if (g->busy.exchange(true)) return fail(NTR_ERR_RUNTIME, "the renderer is already running");
     struct Unbusy { ntr_group *g; ~Unbusy() { g->busy.store(false); } } unbusy{g};
     const int G = (int)g->sc.size();
@@ -2192,6 +2364,8 @@ NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, co
             }
             add_counters(sum, g->counters);
             sum.queue_overflows += g->counters.queue_overflows;
+            // the AOVs of the view on the first device (views_aov_pass leaves the frame's refine mask and counters alone)
+            if (!rc && aov.any()) rc = views_aovs_of(g->sc[0], origins, axes, k, fmt, aov, false, g->sc[0]->stream);
         }
         for (int i = 0; i < G; ++i) g->sc[i]->cam = saved[i];
         if (!rc) g->counters = sum;
@@ -2210,6 +2384,7 @@ NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, co
     cudaPointerAttributes attr;
     const bool pinned = cudaPointerGetAttributes(&attr, dst) == cudaSuccess && attr.type == cudaMemoryTypeHost;
     cudaGetLastError();
+    const bool aov_staged = aov.any() && !aovs_pinned(aov);
     std::vector<ViewsRun> runs(G);
     std::vector<int> first(G), attempts(G, 0);
     CUDA_TRY(cudaSetDevice(g->dev[0]));
@@ -2220,6 +2395,7 @@ NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, co
         r.sc = g->sc[i]; r.fmt = fmt; r.n = (int)((long long)(i + 1) * n / G) - first[i];
         r.dst = out + (size_t)first[i] * fb; r.st = g->sc[i]->stream;
         r.host = true; r.staged = !pinned;
+        r.aov = aov_offset(aov, (size_t)first[i] * fmt->width * fmt->height, r.sc->dev.dim); r.aov_staged = aov_staged;
         CUDA_TRY(cudaSetDevice(g->dev[i]));
         if (i) CUDA_TRY(cudaStreamWaitEvent(r.st, g->ev0, 0));      // the call's clock starts on dev[0]
         rc = views_begin(r, origins + (size_t)first[i] * r.sc->dev.dim, axes + (size_t)first[i] * r.sc->dev.dim * r.sc->dev.dim);
@@ -2263,6 +2439,16 @@ NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, co
         g->counters.queue_overflows += r.sum.queue_overflows;
     }
     return NTR_OK;
+}
+
+NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                                   void *dst, size_t dst_len) {
+    return group_render_views(g, n, origins, axes, fmt, dst, dst_len, nullptr);
+}
+
+NTR_API int ntr_group_render_views_aovs(ntr_group *g, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
+                                        void *dst, size_t dst_len, const ntr_aov_buffers *aovs) {
+    return group_render_views(g, n, origins, axes, fmt, dst, dst_len, aovs);
 }
 
 NTR_API int ntr_group_abort(ntr_group *g) {

@@ -40,9 +40,11 @@ enum : int {
                             // every lane traces the ss x ss samples of its pixel one after the other (trace_core.cuh: ss_pixel_color)
     NTR_F_LIST = 32,        // render_pass_kernel only, per-lane form: the list-driven primary pass of an adaptively supersampled
                             // frame (FrameDev::list): every lane traces one listed pixel with ss_pixel_color at factor FrameDev::ss
-    NTR_F_VIEWS = 64        // render_pass_kernel only, per-lane form: the primary pass of a batch of views (ntr_render_views,
+    NTR_F_VIEWS = 64,       // render_pass_kernel only, per-lane form: the primary pass of a batch of views (ntr_render_views,
                             // FrameDev::views): the blocks of all views in one launch, every lane traces its pixel with
                             // ss_pixel_color at factor FrameDev::ss (1 included) through the camera of its view
+    NTR_F_AOV = 128         // with NTR_F_VIEWS only: the lane also stores the hit id, depth and normal of its pixel's plain
+                            // (factor-1) primary ray into FrameDev::aov_* (ntr_render_views_aovs)
 };
 
 struct SceneDev {
@@ -114,6 +116,13 @@ struct FrameDev {
     // words v * npix + pix (npix = win_w * out_rows), and its packed frame starts at packed + v * pitch * win_h
     const CameraDev *views;
     uint32_t n_views;
+    // AOVs of a batch of views (NTR_F_AOV), per pixel slot v * npix + pix, nullptr where not wanted: the flat id of the plain
+    // primary ray's opaque hit (-1: miss), its distance, and dim floats of the hit's normal.  aov_half_w / aov_half_h /
+    // aov_fovI describe the plain (factor-1) view, whose ray a factor that is not a power of two traces separately.
+    int32_t *aov_ids;
+    float *aov_depth;
+    float *aov_normals;
+    float aov_half_w, aov_half_h, aov_fovI;
 };
 
 // One deferred ray of the wavefront (a reflection bounce): 16-byte aligned record.

@@ -183,6 +183,21 @@ __device__ __forceinline__ void list_pass(const SceneDev &s, const CameraDev &ca
     flush_counters(ctl, cnt);
 }
 
+// The AOVs of pixel slot pix of a batch of views (NTR_F_AOV): what ntr_primary_hit_ids stores, and the hit's normal
+template <int DT>
+__device__ __forceinline__ void store_aov(const SceneDev &s, const FrameDev &f, uint32_t pix, const PrimaryAov<DT> &a) {
+    const bool hit = a.hit.ref != NTR_NONE_REF;
+    if (f.aov_ids) f.aov_ids[pix] = !hit ? -1 : (s.kind == NTR_SCENE_BOX ? 0 : flat_prim_id(s, a.hit.ref, a.hit.lane));
+    if (f.aov_depth) f.aov_depth[pix] = a.hit.dist;
+    if (f.aov_normals) {
+        const int D = NTR_D(DT, s);
+        float *n = f.aov_normals + (size_t)pix * D;
+#pragma unroll
+        for (int k = 0; k < DimCap<DT>::value; ++k)
+            if (k < D) n[k] = a.n[k];
+    }
+}
+
 template <int DT, int FLAGS = 0> struct MinCtas {
     static constexpr int value = (FLAGS & NTR_F_WIDE) ? NTR_MIN_CTAS_WIDE : DT > 8 ? NTR_MIN_CTAS_HI : (DT >= 6 ? NTR_MIN_CTAS_MID : NTR_MIN_CTAS);
 };
@@ -294,8 +309,15 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
                     // the view's camera is read from global memory where it is used (by reference), not copied to registers;
                     // at factor 1 the pixel gets the plain path's bits (ss_pixel_color, EXACT1)
                     QueueEmit<DT> emit{q, ctl, pix, f.out_mode == NTR_OUT_ACCUM};
-                    ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true>(s, f.views[view], f, f.x0 + px, f.y0 + py,
-                                                                                                    acc, emit, cnt, &ms);
+                    if constexpr ((FLAGS & NTR_F_AOV) != 0) {
+                        PrimaryAov<DT> aov;
+                        ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true>(s, f.views[view], f, f.x0 + px, f.y0 + py,
+                                                                                                        acc, emit, cnt, &ms, &aov);
+                        store_aov<DT>(s, f, pix, aov);
+                    } else {
+                        ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true>(s, f.views[view], f, f.x0 + px, f.y0 + py,
+                                                                                                        acc, emit, cnt, &ms);
+                    }
                 } else if constexpr ((FLAGS & NTR_F_SS) != 0) {
                     // supersampled frame: the lane traces the ss x ss samples of its pixel right here, one after the other
                     // (the loop count is the same for every lane); their bounces go to the next pass already weighted
@@ -338,7 +360,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
         // warp-synchronous form (trace_warp.cuh: all 32 lanes enter, `active` says who has a ray; rays park at big leaves
         // and the warp splits them over its lanes when enough lanes are idle) wins where single rays walk leaves of
         // hundreds of items (config 4: 58.4 -> 49.9 ms, its 1/8-frame share 26.3 -> 19.9 ms).
-        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE | NTR_F_SS | NTR_F_VIEWS);      // the per-ray code knows nothing of the switches
+        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE | NTR_F_SS | NTR_F_VIEWS | NTR_F_AOV);      // the per-ray code knows nothing of the switches
         if constexpr ((FLAGS & NTR_F_WARP) != 0) {
             if (s.kind != NTR_SCENE_BOX) {          // warp-uniform
                 if (!active) {
@@ -511,9 +533,9 @@ template <int DT, int FLAGS> struct Launch {
     }
 };
 
-// defined in kern_d*.cu: variant index = FLAGS (0..127; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
+// defined in kern_d*.cu: variant index = FLAGS (0..255; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
 // everywhere else the index falls back to the build without it; NTR_F_SS, NTR_F_LIST and NTR_F_VIEWS builds exist in the
-// per-lane, non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE)
+// per-lane, non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE; NTR_F_AOV builds exist with NTR_F_VIEWS only)
 const KernelSet *kernel_set_d3(int flags);
 const KernelSet *kernel_set_d4(int flags);
 const KernelSet *kernel_set_d5(int flags);
@@ -533,7 +555,9 @@ const KernelSet *kernel_set_dn(int flags);
         if (flags & NTR_F_LIST) return &list[flags & 3];                                                 \
         static const KernelSet views[4] = {Launch<DT, NTR_F_VIEWS>::get(), Launch<DT, 1 | NTR_F_VIEWS>::get(), \
                                            Launch<DT, 2 | NTR_F_VIEWS>::get(), Launch<DT, 3 | NTR_F_VIEWS>::get()}; \
-        if (flags & NTR_F_VIEWS) return &views[flags & 3];
+        static const KernelSet aovs[4] = {Launch<DT, NTR_F_VIEWS | NTR_F_AOV>::get(), Launch<DT, 1 | NTR_F_VIEWS | NTR_F_AOV>::get(), \
+                                          Launch<DT, 2 | NTR_F_VIEWS | NTR_F_AOV>::get(), Launch<DT, 3 | NTR_F_VIEWS | NTR_F_AOV>::get()}; \
+        if (flags & NTR_F_VIEWS) return (flags & NTR_F_AOV) ? &aovs[flags & 3] : &views[flags & 3];
 #define NTR_INSTANTIATE_DIM(NAME, DT)                                                                  \
     const KernelSet *NAME(int flags) {                                                                  \
         NTR_SS_SETS(DT)                                                                                 \

@@ -1401,11 +1401,12 @@ NTR_HD void hit_geometry(const SceneDev &s, uint32_t ref, int lane, float dist, 
 
 // composite_scene::ray_color (tracer.hpp:1856-1883), linearised: the transparent layers (sorted near to
 // far) and the opaque hit / background each contribute base_color * op_i * prod_{j<i}(1 - op_j).
-// EMIT(const Bounce<DT>&) receives the deferred reflection rays.
+// EMIT(const Bounce<DT>&) receives the deferred reflection rays.  normal_out (D floats, left alone on a miss) receives
+// the normal that shades the opaque hit.
 template <int DT, int FLAGS, typename EMIT>
 NTR_HD void ray_color(const SceneDev &s, bool enabled, const float *o, const float *dir, int depth, Skip source,
                       const float *weight, float *acc, EMIT &emit, Counters &cnt, HitRec *primary_out,
-                      MailboxStore *ms = nullptr) {
+                      MailboxStore *ms = nullptr, float *normal_out = nullptr) {
     const int D = NTR_D(DT, s);
     GenState<DT> g;
     g.mb.big = (ms && ms->col) ? ms : nullptr;
@@ -1454,6 +1455,10 @@ NTR_HD void ray_color(const SceneDev &s, bool enabled, const float *o, const flo
             } else {
                 hit_geometry<DT, FLAGS>(s, ref, lane, oh.dist, o, dir, P, N);
             }
+            if (normal_out) {
+    NTR_UNROLL
+                for (int k = 0; k < D; ++k) normal_out[k] = N[k];
+            }
         }
         if (shade_hit<DT, FLAGS>(s, dir, P, N, ref, lane, depth, wl, acc, b, cnt)) emit(b);
     }
@@ -1469,9 +1474,10 @@ NTR_HD void ray_color(const SceneDev &s, bool enabled, const float *o, const flo
 
 // flat_origin_ray_source::operator() (tracer.hpp:71-75): integer pixel coordinates, no half-pixel offset
 template <int DT>
-NTR_HD void primary_ray(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, float *o, float *dir) {
+NTR_HD void primary_ray_of(const SceneDev &s, const CameraDev &cam, float fovI, float half_w, float half_h, int x, int y,
+                           float *o, float *dir) {
     const int D = NTR_D(DT, s);
-    const float fx = f.fovI * ((float)x - f.half_w), fy = f.fovI * ((float)y - f.half_h);
+    const float fx = fovI * ((float)x - half_w), fy = fovI * ((float)y - half_h);
     float sq = 0;
     NTR_UNROLL
     for (int i = 0; i < D; ++i) {
@@ -1483,11 +1489,17 @@ NTR_HD void primary_ray(const SceneDev &s, const CameraDev &cam, const FrameDev 
     NTR_UNROLL
     for (int i = 0; i < D; ++i) dir[i] /= len;
 }
+template <int DT>
+NTR_HD void primary_ray(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, float *o, float *dir) {
+    primary_ray_of<DT>(s, cam, f.fovI, f.half_w, f.half_h, x, y, o, dir);
+}
 
 // box_scene::calculate_color (tracer.hpp:101-114) with hypercube_intersects (:126-152) inlined:
 // the unit hypercube at the origin, fixed shading, gradient background.
+// normal_out (D floats, left alone on a miss): the axis vector of the face that was hit
 template <int DT>
-NTR_HD void box_color(const SceneDev &s, const float *o, const float *dir, float *rgb, HitRec *primary_out) {
+NTR_HD void box_color(const SceneDev &s, const float *o, const float *dir, float *rgb, HitRec *primary_out,
+                      float *normal_out = nullptr) {
     const int D = NTR_D(DT, s);
     for (int i = 0; i < D; ++i) {
         const float di = vsel<DT>(dir, i);
@@ -1505,6 +1517,7 @@ NTR_HD void box_color(const SceneDev &s, const float *o, const float *dir, float
                     const float k = sine <= 0 ? -sine : 0.0f;
                     rgb[0] = k * 1.0f; rgb[1] = k * 0.5f; rgb[2] = k * 0.5f;
                     if (primary_out) { primary_out->dist = dist; primary_out->ref = 0; primary_out->lane = -1; }
+                    if (normal_out) for (int j = 0; j < D; ++j) normal_out[j] = j == i ? face : 0.0f;
                     return;
                 }
             }
@@ -1542,11 +1555,28 @@ NTR_HD float mul_rn(float a, float b) {
 // EXACT1 (the primary pass of a batch of views, NTR_F_VIEWS, which runs factor 1 through here as well): at factor 1 the one
 // sample's colour is stored as it is, so that the pixel has the bits of the plain primary path -- 0.0f + c would turn a
 // negative zero into +0 (box_color stores -0 where the direction's gradient axis is +0; tests/test_views.py)
+//
+// aov (NTR_F_AOV): receives the hit of the pixel's plain (factor-1) primary ray.  For ss in {1, 2, 4, 8} that ray is sample
+// (0, 0) bit for bit -- fovI / ss and ss * x - ss * half_w scale exactly by a power of two (tests/test_aovs.py) -- so its hit
+// is taken from that sample's ray_color.  Any other factor traces the plain ray once more (plain_primary_hit).
+template <int DT> struct PrimaryAov {
+    HitRec hit;
+    float n[DimCap<DT>::value];     // the normal that shades the hit; zeros on a miss
+};
+template <int DT, int FLAGS>
+NTR_HD void plain_primary_hit(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, PrimaryAov<DT> &a,
+                              MailboxStore *ms);
+
 template <int DT, int FLAGS, typename EMIT, bool EXACT1 = false>
 NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, float *sum,
-                           EMIT &emit, Counters &cnt, MailboxStore *ms) {
+                           EMIT &emit, Counters &cnt, MailboxStore *ms, PrimaryAov<DT> *aov = nullptr) {
     constexpr int CAP = DimCap<DT>::value;
     const int ss = f.ss;
+    const bool pow2 = (ss & (ss - 1)) == 0;
+    if (aov) {
+        aov->hit.dist = 0; aov->hit.ref = NTR_NONE_REF; aov->hit.lane = -1;
+        for (int i = 0; i < CAP; ++i) aov->n[i] = 0.0f;
+    }
     const float wt = 1.0f / (float)(ss * ss);
     const float w[3] = {wt, wt, wt};
     const Skip none = {NTR_NONE_REF, 0};
@@ -1556,14 +1586,55 @@ NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameD
         float o[CAP], dir[CAP];
         float c[3] = {0.0f, 0.0f, 0.0f};
         primary_ray<DT>(s, cam, f, ss * x + i, ss * y + j, o, dir);
+        const bool capture = aov && pow2 && k == 0;
         if (s.kind == NTR_SCENE_BOX) {
-            box_color<DT>(s, o, dir, c, nullptr);                  // assigns the colour: weight it here
+            box_color<DT>(s, o, dir, c, capture ? &aov->hit : nullptr, capture ? aov->n : nullptr);   // assigns the colour: weight it here
             c[0] = mul_rn(c[0], wt); c[1] = mul_rn(c[1], wt); c[2] = mul_rn(c[2], wt);
         } else {
-            ray_color<DT, FLAGS>(s, true, o, dir, 0, none, w, c, emit, cnt, nullptr, ms);
+            ray_color<DT, FLAGS>(s, true, o, dir, 0, none, w, c, emit, cnt, capture ? &aov->hit : nullptr, ms,
+                                 capture ? aov->n : nullptr);
         }
         if (EXACT1 && ss == 1) { sum[0] = c[0]; sum[1] = c[1]; sum[2] = c[2]; }
         else { sum[0] = add_rn(sum[0], c[0]); sum[1] = add_rn(sum[1], c[1]); sum[2] = add_rn(sum[2], c[2]); }
+    }
+    if (aov && !pow2) plain_primary_hit<DT, FLAGS>(s, cam, f, x, y, *aov, ms);
+}
+
+// The hit of output pixel (x, y)'s plain primary ray, with the nearest-hit traversal of ray_color only: no shading, no
+// bounces, no counters.  a must hold ray_color's miss state (ss_pixel_color clears it).
+template <int DT, int FLAGS>
+NTR_HD void plain_primary_hit(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, PrimaryAov<DT> &a,
+                              MailboxStore *ms) {
+    constexpr int CAP = DimCap<DT>::value;
+    constexpr int TF = FLAGS & ~NTR_F_COUNT;
+    const int D = NTR_D(DT, s);
+    float o[CAP], dir[CAP];
+    primary_ray_of<DT>(s, cam, f.aov_fovI, f.aov_half_w, f.aov_half_h, x, y, o, dir);
+    if (s.kind == NTR_SCENE_BOX) {
+        float c[3];
+        box_color<DT>(s, o, dir, c, &a.hit, a.n);
+        return;
+    }
+    GenState<DT> g;
+    g.mb.big = (ms && ms->col) ? ms : nullptr;
+    HitRec oh;
+    oh.dist = FLT_MAX; oh.ref = NTR_NONE_REF; oh.lane = -1;
+    if (TF & NTR_F_GENERAL) {
+        g.th.clear();
+    NTR_UNROLL
+        for (int i = 0; i < D; ++i) { g.hitP[i] = 0; g.hitN[i] = 0; }
+    }
+    Counters none;
+    const Skip source = {NTR_NONE_REF, 0};
+    const float t0 = aabb_distance<DT>(s, o, dir);
+    if (!(t0 >= 0 && trace_nearest<DT, TF>(s, o, dir, source, t0, FLT_MAX, oh, &g, none))) return;
+    a.hit = oh;
+    if (TF & NTR_F_GENERAL) {
+    NTR_UNROLL
+        for (int k = 0; k < D; ++k) a.n[k] = g.hitN[k];
+    } else {
+        float P[CAP];
+        hit_geometry<DT, TF>(s, oh.ref, oh.lane, oh.dist, o, dir, P, a.n);
     }
 }
 

@@ -299,13 +299,17 @@ class BlockingRenderer:
         finally:
             self._lock.release()
 
-    def render_views(self, dest, format, scene, cameras):
+    def render_views(self, dest, format, scene, cameras, *, ids=None, depth=None, normals=None):
         """Extension without a reference counterpart: one frame per camera in one call, frame k at byte offset
         k * pitch * height of `dest` (ntr_render_views).  Frame k is what render() gives after scene.set_camera(cameras[k]);
         the scene's camera is left as it is.  cameras: Camera objects of the scene's dimension or (origin, axes) pairs
         (stream.rotation_cameras).  With threads > 1 (or NTR_GPUS) whole views are dealt to the GPUs.
+        ids / depth / normals: writable buffers that also receive the per-pixel AOVs of every view, in the same launches
+        (ntr_render_views_aovs): int32 hit ids (n x height x width, -1 on a miss), float32 hit distances (n x height x width)
+        and float32 normals (n x height x width x dimension) of each pixel's plain primary ray.  A numpy array must have
+        that dtype.
         -> True, or False if signal_abort() was called while rendering."""
-        from .backend import camera_arrays
+        from .backend import AOV_DTYPES, aov_shape, aov_struct, camera_arrays
         if not isinstance(format, ImageFormat):
             raise TypeError('object is not an instance of ImageFormat')
         if not isinstance(scene, Scene):
@@ -316,6 +320,16 @@ class BlockingRenderer:
         fmt = format._native()
         if buf.size < n * fmt.pitch * fmt.height:
             raise ValueError('the buffer is too small for %d images with the given dimensions' % n)
+        aovs = {}
+        for name, b in (('ids', ids), ('depth', depth), ('normals', normals)):
+            if b is None:
+                continue
+            if isinstance(b, np.ndarray) and b.dtype != AOV_DTYPES[name]:
+                raise TypeError('the %s buffer must hold %s' % (name, np.dtype(AOV_DTYPES[name]).name))
+            v = _writable_buffer(b)
+            if v.size < 4 * int(np.prod(aov_shape(name, n, fmt, scene.dimension))):
+                raise ValueError('the %s buffer is too small for %d images with the given dimensions' % (name, n))
+            aovs[name] = (v.ctypes.data, v.size // 4)
         if not self._lock.acquire(blocking=False):
             raise RuntimeError('the renderer is already running')
         try:
@@ -323,9 +337,14 @@ class BlockingRenderer:
             try:
                 dev = scene._prepare(self._gpus) if self._gpus > 1 else scene._prepare()
                 self._dev = dev
-                fn = dev._lib.ntr_group_render_views if hasattr(dev, 'size') else dev._lib.ntr_render_views
-                rc = fn(dev._h, n, origins.ctypes.data_as(C.c_void_p), axes.ctypes.data_as(C.c_void_p), C.byref(fmt),
+                args = (dev._h, n, origins.ctypes.data_as(C.c_void_p), axes.ctypes.data_as(C.c_void_p), C.byref(fmt),
                         buf.ctypes.data_as(C.c_void_p), buf.size)
+                if aovs:
+                    fn = dev._lib.ntr_group_render_views_aovs if hasattr(dev, 'size') else dev._lib.ntr_render_views_aovs
+                    rc = fn(*args, C.byref(aov_struct(aovs)))
+                else:
+                    fn = dev._lib.ntr_group_render_views if hasattr(dev, 'size') else dev._lib.ntr_render_views
+                    rc = fn(*args)
                 if rc == _capi.NTR_ERR_ABORTED:
                     return False
                 _capi.check(rc)
