@@ -288,6 +288,31 @@ NTR_API int ntr_occludes_rays(ntr_scene *scene, uint32_t n, const float *origins
                               const float *distance, const uint32_t *skip_ref, const int32_t *skip_lane,
                               int32_t *occluded_out, int32_t *n_transparent_out);
 
+/* Shading of caller-given primary rays (no counterpart in the reference, whose only primary rays are the camera's,
+ * flat_origin_ray_source, src/tracer.hpp:60-76).  origins / dirs are n x D row-major (as ntr_trace_rays); rgb_out is n x 3
+ * floats: for ray i the float colour the reference computes for (origins[i], dirs[i]) as a primary ray --
+ * composite_scene::ray_color(ray, depth 0, no source) with aabb_distance and the bounces up to max_reflect_depth
+ * (src/tracer.hpp:1856-1883), or box_scene::calculate_color's colour of that ray (:101-114) -- which is what
+ * ntr_render_float gives for a pixel whose primary ray is that ray.  Directions are used as given and are not normalised
+ * (neither does ray_color): the camera light and the specular term assume unit directions, as the camera's rays are.
+ * Like every per-ray hook the call ignores the scene's camera, fov, supersampling factor and threshold, and leaves the
+ * refine-mask record alone.  Counters: primary_rays = n, the others summed over everything traced.  A launch covers at most
+ * 2^25 rays (the environment variable NTR_RAYS_PER_LAUNCH=n overrides); longer batches run as consecutive launches.
+ * aovs (optional, may be NULL; a NULL pointer in it means "not wanted"): per ray, ids / depth one element and normals D
+ * floats (the *_len count elements), with the definitions of the views AOVs: the flat id of the ray's opaque hit (-1: a miss;
+ * a BoxScene's cube is 0), its distance (0 on a miss) and the normal that shades it (zeros on a miss).  For a composite scene
+ * the ids and distances equal, bit for bit, those of ntr_trace_rays(scene, 1, origins[i], dirs[i], t0, FLT_MAX, NULL, NULL,
+ * ...) with t0 = composite_scene::aabb_distance of the ray (src/tracer.hpp:1892-1918), and -1 / 0 where t0 < 0 (the ray
+ * misses the scene's box).  n = 0 does nothing.  NTR_ERR_VALUE: a NULL array or a short AOV buffer, checked before any
+ * work.  NTR_ERR_RUNTIME while a frame of the scene is rendering or open.  NTR_ERR_ABORTED after ntr_abort(); the outputs
+ * are then unspecified. */
+NTR_API int ntr_render_rays(ntr_scene *scene, uint32_t n, const float *origins, const float *dirs, float *rgb_out,
+                            const ntr_aov_buffers *aovs_or_null);
+/* The same with every pointer in DEVICE memory of the scene's device, on a caller-supplied CUDA stream (NULL = the scene's
+ * own): asynchronous when the scene needs no bounce passes, synchronous on that stream otherwise, as ntr_render_device. */
+NTR_API int ntr_render_rays_device(ntr_scene *scene, uint32_t n, const float *origins, const float *dirs, float *rgb_out,
+                                   const ntr_aov_buffers *aovs_or_null, void *stream);
+
 /* ---- several GPUs of one box (SURVEY.md section 8e; no counterpart in the reference, whose parallelism is worker
  * threads pulling 32x32 tiles, src/render.cpp:468-493,829-838) ---------------------------------------------------
  * A group replicates the scene on n devices.  A frame is split by interleaved 32-pixel tile rows (tile row ty belongs
@@ -322,6 +347,10 @@ NTR_API int ntr_group_render_views(ntr_group *group, int n, const float *origins
 /* ntr_render_views_aovs over the group: every entry writes the frames and AOVs of its own views straight to their place. */
 NTR_API int ntr_group_render_views_aovs(ntr_group *group, int n, const float *origins, const float *axes,
                                         const ntr_image_format *fmt, void *dst, size_t dst_len, const ntr_aov_buffers *aovs);
+/* ntr_render_rays over the group (host arrays): entry i gets rays [floor(i*n/G), floor((i+1)*n/G)), traces them in its own
+ * memory and copies its results straight to their place; nothing crosses NVLink.  Counters are summed over the entries. */
+NTR_API int ntr_group_render_rays(ntr_group *group, uint32_t n, const float *origins, const float *dirs, float *rgb_out,
+                                  const ntr_aov_buffers *aovs_or_null);
 NTR_API int ntr_group_abort(ntr_group *group);
 /* Counters of the last frame summed over the devices; device time of the last frame from the first kernel to the last
  * one of the slowest device (CUDA events on the first device's stream, which waits for the others). */

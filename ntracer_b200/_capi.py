@@ -216,6 +216,8 @@ def load():
         'ntr_render_views_aovs': (C.c_int, [vp, i32, vp, vp, C.POINTER(ImageFormat), vp, C.c_size_t, C.POINTER(AovBuffers)]),
         'ntr_render_views_aovs_device': (C.c_int, [vp, i32, vp, vp, C.POINTER(ImageFormat), vp, C.c_size_t,
                                                    C.POINTER(AovBuffers), vp]),
+        'ntr_render_rays': (C.c_int, [vp, u32, vp, vp, vp, C.POINTER(AovBuffers)]),
+        'ntr_render_rays_device': (C.c_int, [vp, u32, vp, vp, vp, C.POINTER(AovBuffers), vp]),
         'ntr_render_float': (C.c_int, [vp, i32, i32, vp]),
         'ntr_calculate_color': (C.c_int, [vp, i32, i32, i32, i32, f32p]),
         'ntr_primary_hit_ids': (C.c_int, [vp, i32, i32, vp, vp]),
@@ -247,6 +249,7 @@ def load():
         'ntr_group_render_device': (C.c_int, [vp, C.POINTER(ImageFormat), C.POINTER(vp)]),
         'ntr_group_render_views': (C.c_int, [vp, i32, vp, vp, C.POINTER(ImageFormat), vp, C.c_size_t]),
         'ntr_group_render_views_aovs': (C.c_int, [vp, i32, vp, vp, C.POINTER(ImageFormat), vp, C.c_size_t, C.POINTER(AovBuffers)]),
+        'ntr_group_render_rays': (C.c_int, [vp, u32, vp, vp, vp, C.POINTER(AovBuffers)]),
         'ntr_group_abort': (C.c_int, [vp]),
         'ntr_group_get_counters': (C.c_int, [vp, C.POINTER(Counters)]),
         'ntr_group_last_kernel_ms': (C.c_int, [vp, f32p]),
@@ -270,14 +273,15 @@ EXPORTED_SYMBOLS = (
     'ntr_abi_version', 'ntr_last_error', 'ntr_device_count', 'ntr_scene_create', 'ntr_scene_destroy',
     'ntr_scene_set_camera', 'ntr_scene_set_params', 'ntr_scene_set_supersampling', 'ntr_render', 'ntr_render_device', 'ntr_render_begin',
     'ntr_render_end', 'ntr_render_views', 'ntr_render_views_device', 'ntr_render_views_aovs', 'ntr_render_views_aovs_device',
-    'ntr_render_float',
+    'ntr_render_rays', 'ntr_render_rays_device', 'ntr_render_float',
     'ntr_calculate_color', 'ntr_primary_hit_ids', 'ntr_trace_rays', 'ntr_trace_rays_hits', 'ntr_occludes_rays', 'ntr_abort',
     'ntr_get_counters', 'ntr_set_instrumented', 'ntr_last_kernel_ms', 'ntr_launch_count',
     'ntr_measure_fp32_peak', 'ntr_simplex_from_points', 'ntr_build_kdtree', 'ntr_build_kdtree_culled', 'ntr_free', 'ntr_group_items',
     'ntr_group_create', 'ntr_group_destroy', 'ntr_group_size', 'ntr_group_set_camera', 'ntr_group_set_params',
     'ntr_group_set_supersampling', 'ntr_scene_set_supersampling_threshold', 'ntr_last_refine_mask',
     'ntr_group_set_supersampling_threshold', 'ntr_group_last_refine_mask',
-    'ntr_group_render', 'ntr_group_render_device', 'ntr_group_render_views', 'ntr_group_render_views_aovs', 'ntr_group_abort', 'ntr_group_get_counters',
+    'ntr_group_render', 'ntr_group_render_device', 'ntr_group_render_views', 'ntr_group_render_views_aovs', 'ntr_group_render_rays',
+    'ntr_group_abort', 'ntr_group_get_counters',
     'ntr_group_last_kernel_ms', 'ntr_group_launch_count',
     'ntr_frame_alloc', 'ntr_frame_free', 'ntr_frame_export', 'ntr_frame_import', 'ntr_frame_release',
     'ntr_frame_fill', 'ntr_frame_download')

@@ -97,11 +97,47 @@ def _refine_mask(fn, handle, w, h):
     return mask, int(count.value)
 
 
+def ray_arrays(origins, dirs, dim):
+    """The rays of a rays call -> (origins, dirs) as C-contiguous float32 (n, dim) arrays.  ValueError: not n x dim, or a
+    different number of origins and directions."""
+    o = np.ascontiguousarray(origins, dtype=np.float32)
+    d = np.ascontiguousarray(dirs, dtype=np.float32)
+    if o.ndim != 2 or d.ndim != 2 or o.shape[1] != dim or d.shape[1] != dim:
+        raise ValueError('origins and dirs must be (n, %d) arrays: the rays and the scene must have the same dimension' % dim)
+    if o.shape[0] != d.shape[0]:
+        raise ValueError('%d origins but %d directions' % (o.shape[0], d.shape[0]))
+    return o, d
+
+
+def _new_ray_aovs(aovs, n, dim):
+    """-> ({name: new array}, AovBuffers over them): ids / depth (n,), normals (n, dim)"""
+    arrays = {name: np.zeros((n,) + ((dim,) if name == 'normals' else ()), AOV_DTYPES[name]) for name in _aov_names(aovs)}
+    return arrays, aov_struct({k: (v.ctypes.data, v.size) for k, v in arrays.items()})
+
+
+def _tensor(t, what, dtype, shape, device):
+    """a torch tensor argument of a device rays call: TypeError for a wrong type, dtype or device (device < 0: any CUDA
+    device), ValueError for a wrong shape or a layout that is not contiguous"""
+    import torch
+    if not isinstance(t, torch.Tensor):
+        raise TypeError('%s must be a torch tensor' % what)
+    if t.dtype != dtype:
+        raise TypeError('%s must be %s, not %s' % (what, dtype, t.dtype))
+    if t.device.type != 'cuda' or (device >= 0 and t.device.index != device):
+        raise TypeError("%s must be on the scene's device, not %s" % (what, t.device))
+    if tuple(t.shape) != tuple(shape):
+        raise ValueError('%s must have shape %s, not %s' % (what, tuple(shape), tuple(t.shape)))
+    if not t.is_contiguous():
+        raise ValueError('%s must be contiguous' % what)
+    return t
+
+
 class DeviceScene:
     def __init__(self, scene, device=-1):
         """scene: flat scene dict (DESIGN.md 'scene file'; ntracer_b200.scene_io.load_scene)."""
         self._lib = _capi.load()
         self._h = C.c_void_p()
+        self.device = int(device)
         self.dim = int(scene['dim'])
         self.kind = int(scene['kind'])
         self._scene = scene
@@ -249,6 +285,42 @@ class DeviceScene:
         self._window = (fmt.width, fmt.height)
         _capi.check(self._lib.ntr_render_device(self._h, C.byref(fmt), C.c_void_p(dev_ptr), nbytes,
                                                 C.c_void_p(stream), tile_row_first, tile_row_step, int(compact)))
+
+    def render_rays(self, origins, dirs, aovs=()):
+        """The colour of caller-given primary rays (ntr_render_rays): origins and dirs are (n, dim); ray i gets the float RGB
+        the reference computes for it as a primary ray (what render_float gives a pixel whose primary ray it is).  Directions
+        are used as given: the camera light and the specular term assume unit directions.  -> (n, 3) float32, or (rgb,
+        {name: array}) when AOV names are asked for: 'ids' int32 (n,), 'depth' float32 (n,), 'normals' float32 (n, dim), with
+        the definitions of render_views_aovs.  The camera, fov and supersampling settings are not used."""
+        o, d = ray_arrays(origins, dirs, self.dim)
+        n = o.shape[0]
+        rgb = np.zeros((n, 3), np.float32)
+        arrays, a = _new_ray_aovs(aovs, n, self.dim)
+        _capi.check(self._lib.ntr_render_rays(self._h, n, _p(o), _p(d), _p(rgb), C.byref(a) if arrays else None))
+        return (rgb, arrays) if arrays else rgb
+
+    def render_rays_device(self, origins, dirs, rgb, aovs=None, stream=0):
+        """render_rays on torch tensors of the scene's device, on a CUDA stream handle (0: the scene's own stream): origins
+        and dirs float32 (n, dim), rgb float32 (n, 3), and `aovs` mapping AOV names to int32 (n,) ids, float32 (n,) depth or
+        float32 (n, dim) normals tensors, all contiguous.  Asynchronous when the scene needs no reflection passes, synchronous
+        on the stream otherwise.  TypeError: a wrong dtype or device; ValueError: a wrong shape or dimension."""
+        import torch
+        if not isinstance(origins, torch.Tensor):
+            raise TypeError('origins must be a torch tensor')
+        n = origins.shape[0] if origins.dim() else 0
+        o = _tensor(origins, 'origins', torch.float32, (n, self.dim), self.device)
+        dev = o.device.index
+        d = _tensor(dirs, 'dirs', torch.float32, (n, self.dim), dev)
+        c = _tensor(rgb, 'rgb', torch.float32, (n, 3), dev)
+        ptrs = {}
+        for name in _aov_names(aovs or {}):
+            t = _tensor(aovs[name], name, torch.int32 if name == 'ids' else torch.float32,
+                        (n, self.dim) if name == 'normals' else (n,), dev)
+            ptrs[name] = (t.data_ptr(), t.numel())
+        a = aov_struct(ptrs)
+        _capi.check(self._lib.ntr_render_rays_device(self._h, n, C.c_void_p(o.data_ptr()), C.c_void_p(d.data_ptr()),
+                                                     C.c_void_p(c.data_ptr()), C.byref(a) if ptrs else None,
+                                                     C.c_void_p(stream)))
 
     def render_float(self, width, height):
         out = np.zeros((height, width, 3), dtype=np.float32)
@@ -410,6 +482,16 @@ class DeviceGroup:
         _capi.check(self._lib.ntr_group_render_views_aovs(self._h, len(origins), _p(origins), _p(axes), C.byref(fmt), _p(buf),
                                                           buf.size, C.byref(a)))
         return out, arrays
+
+    def render_rays(self, origins, dirs, aovs=()):
+        """DeviceScene.render_rays over the group: every device traces a contiguous range of the rays and writes its
+        results straight to their place (ntr_group_render_rays)."""
+        o, d = ray_arrays(origins, dirs, self.dim)
+        n = o.shape[0]
+        rgb = np.zeros((n, 3), np.float32)
+        arrays, a = _new_ray_aovs(aovs, n, self.dim)
+        _capi.check(self._lib.ntr_group_render_rays(self._h, n, _p(o), _p(d), _p(rgb), C.byref(a) if arrays else None))
+        return (rgb, arrays) if arrays else rgb
 
     def render_device(self, fmt):
         """-> address of the frame on the first device (valid until the next render)"""

@@ -200,6 +200,12 @@ struct ntr_scene {
     float views_pass_ns_per_ray = 0.0f;
     uint32_t views_prev_pass_count[kMaxPasses + 2] = {};
     uint32_t views_per_launch = 0;      // NTR_VIEWS_PER_LAUNCH: views per launch of a views call (0: from kViewsSampleCap)
+    // batches of caller-given rays (ntr_render_rays): wavefront statistics of their own, kept apart like the views calls'; the
+    // grid of the ray-fed primary pass per build (FLAGS & 3); NTR_RAYS_PER_LAUNCH: rays per launch (0: kRaysPerLaunch)
+    float rays_pass_ns_per_ray = 0.0f;
+    uint32_t rays_prev_pass_count[kMaxPasses + 2] = {};
+    int rays_grid[4] = {};
+    uint32_t rays_per_launch = 0;
     // begin/end frames (ntr_render_begin / ntr_render_end); a views call uses their device buffers, staging buffers, events and
     // copy stream for its double-buffered launches
     FrameSlot slots[NTR_FRAMES_IN_FLIGHT];
@@ -415,11 +421,12 @@ struct RenderTarget {
     float *accum = nullptr;
     int32_t *ids = nullptr;
     float *dists = nullptr;
-    AovTarget aov;              // a batch of views only: its AOVs (device memory), traced by the NTR_F_AOV build
+    AovTarget aov;              // a batch of views or rays only: its AOVs (device memory)
+    const float *ray_o = nullptr, *ray_d = nullptr;     // NTR_OUT_RAYS: the rays (device memory, n x D), n = the window width
 };
 
-// Supersampling factor of a frame: the hit-id hook traces one ray per pixel whatever the scene's factor
-int frame_ss(const ntr_scene *sc, int out_mode) { return out_mode == NTR_OUT_IDS ? 1 : sc->ss; }
+// Supersampling factor of a frame: the hit-id hook and a batch of rays trace one ray per pixel whatever the scene's factor
+int frame_ss(const ntr_scene *sc, int out_mode) { return out_mode == NTR_OUT_IDS || out_mode == NTR_OUT_RAYS ? 1 : sc->ss; }
 // Adaptive supersampling: a factor above 1 and a threshold.  Such frames always take the accumulator route
 bool frame_adaptive(const ntr_scene *sc, int out_mode) { return frame_ss(sc, out_mode) > 1 && sc->ss_threshold >= 0.0f; }
 
@@ -447,6 +454,9 @@ uint64_t count_halo(const FrameDev &f) {
 // A batch of views (n_views > 0, whole frames at a factor >= 1, never adaptive) runs the NTR_F_VIEWS primary pass over the
 // cameras views[0 .. n_views): view v has accumulator slots v * npix .. and its packed frame at tgt.packed + v * pitch * win_h;
 // the bounce passes and pack_kernel are the single frame's, over all views at once.
+// A batch of caller-given rays (tgt.out_mode NTR_OUT_RAYS, factor 1) is a win_w x 1 window: render_rays_kernel traces ray i into
+// accumulator slot i, the bounce passes are the single frame's, nothing is packed, no tile schedule is kept and the refine-mask
+// record is left alone.
 int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0, int y0, int win_w, int win_h,
                   const ntr_image_format *fmt, const RenderTarget &tgt, int tile_row_first, int tile_row_step,
                   int compact, bool *used_passes, const CameraDev *views = nullptr, uint32_t n_views = 0) {
@@ -470,7 +480,8 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     f.tile_row_first = tile_row_first; f.tile_row_step = tile_row_step < 1 ? 1 : tile_row_step; f.compact = compact;
     if (fmt) fill_format(f.fmt, fmt);
     f.views = views; f.n_views = n_views;
-    const bool aov = n_views && tgt.aov.any();
+    const bool rays = tgt.out_mode == NTR_OUT_RAYS;
+    const bool aov = (n_views || rays) && tgt.aov.any();
     if (aov) {
         f.aov_ids = static_cast<int32_t *>(tgt.aov.p[0]);
         f.aov_depth = static_cast<float *>(tgt.aov.p[1]);
@@ -482,7 +493,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     }
     const size_t nv = n_views ? n_views : 1;
     // wavefront statistics of the previous frame (of the previous views call, for a batch of views)
-    float &pass_ns_per_ray = n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray;
+    float &pass_ns_per_ray = rays ? sc->rays_pass_ns_per_ray : n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray;
 
     // Scenes with big leaves: the bounce passes run the warp-synchronous kernels (incoherent rays; lanes that run out of
     // work help the ones parked at big leaves), the primary pass every lane for itself (the 32 rays of an 8x4 pixel block
@@ -530,7 +541,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     // whole frame on one GPU (loss of row-major locality + the cost bookkeeping), so it is used for sharded renders --
     // and for whole frames of scenes with giant leaves, whose few blocks through the centre cost 10-90x the mean
     // (config 4: primary pass 11.2-11.6 -> 10.4 ms, frame 43.3 -> 42.4 ms, calls 17 and 20)
-    const bool use_sched = n_tiles >= 64 && composite && tgt.out_mode != NTR_OUT_IDS && !sc->no_tile_sched &&
+    const bool use_sched = n_tiles >= 64 && composite && tgt.out_mode != NTR_OUT_IDS && !rays && !sc->no_tile_sched &&
                            (f.tile_row_step > 1 || sc->force_tile_sched || sc->max_leaf >= 256);
     const int slot = n_views ? kSchedViews : sc->ctl_slot;
     if (use_sched) {
@@ -598,7 +609,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     q.out = sc->d_queue[0];
     q.out_count = d_ctl + CTL_COUNT0 + 1;
     q.in_count = q.in_cursor = nullptr;
-    if (tgt.out_mode != NTR_OUT_IDS) {            // the hit-id hook leaves the last frame's refine mask alone
+    if (tgt.out_mode != NTR_OUT_IDS && !rays) {   // the hit-id hook and a batch of rays leave the last frame's refine mask alone
         sc->last = {};
         sc->last.valid = true; sc->last.adaptive = adaptive;
         sc->last.win_w = win_w; sc->last.win_h = win_h; sc->last.out_rows = f.out_rows;
@@ -612,7 +623,18 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     };
     sc->n_pass_ev = 0;
     mark();
-    ks->render_pass(dim3(grid), dim3(kCtaThreads), st, sc->dev, sc->cam, f, q, ctl);
+    if (rays) {
+        // the ray-fed primary pass: per lane, non-wide, one build per FLAGS & 3; no more CTAs than the exact mailbox has columns
+        const int rf = flags & (NTR_F_GENERAL | NTR_F_COUNT);
+        if (!sc->rays_grid[rf]) sc->rays_grid[rf] = std::max(1, sc->kset(rf)->rays_blocks_per_sm()) * sc->sm_count;
+        int rgrid = sc->rays_grid[rf];
+        if (sc->dev.mb_table) rgrid = std::min(rgrid, (int)(sc->dev.mb_threads / kCtaThreads));
+        QueueDev qr = q;
+        if (!passes) qr.out = nullptr;
+        sc->kset(rf)->render_rays(dim3(rgrid), dim3(kCtaThreads), st, sc->dev, f, qr, ctl, tgt.ray_o, tgt.ray_d, (uint32_t)win_w);
+    } else {
+        ks->render_pass(dim3(grid), dim3(kCtaThreads), st, sc->dev, sc->cam, f, q, ctl);
+    }
     ++sc->launches;
     mark();
 #if NTR_FETCH_STATS
@@ -707,7 +729,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         return NTR_OK;
     };
     if (passes) {
-        const int rc = bounces(CTL_COUNT0, CTL_CURSOR0, n_views ? sc->views_prev_pass_count : sc->prev_pass_count);
+        const int rc = bounces(CTL_COUNT0, CTL_CURSOR0, rays ? sc->rays_prev_pass_count : n_views ? sc->views_prev_pass_count : sc->prev_pass_count);
         if (rc) return rc;
     }
     if (adaptive) {
@@ -809,9 +831,12 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
         for (int d = 1; d <= sc->dev.max_depth && d <= kMaxPasses; ++d) rays += std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
         if (adaptive)
             for (int d = 1; d <= sc->dev.max_depth && d <= kMaxPasses; ++d) rays += std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
-        if (rays > 0) (j.n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray) = ms * 1e6f / (float)rays;
+        if (rays > 0)
+            (j.tgt.out_mode == NTR_OUT_RAYS ? sc->rays_pass_ns_per_ray : j.n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray) =
+                ms * 1e6f / (float)rays;
     }
-    uint32_t *const prev = j.n_views ? sc->views_prev_pass_count : sc->prev_pass_count;
+    uint32_t *const prev = j.tgt.out_mode == NTR_OUT_RAYS ? sc->rays_prev_pass_count
+                           : j.n_views ? sc->views_prev_pass_count : sc->prev_pass_count;
     if (j.passes) for (int d = 1; d <= kMaxPasses; ++d) prev[d] = std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
     if (j.passes && adaptive)
         for (int d = 1; d <= kMaxPasses; ++d) sc->prev_pass_count2[d] = std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
@@ -1167,6 +1192,7 @@ NTR_API int ntr_scene_create(const ntr_scene_desc *desc, int device, ntr_scene *
     }
     if (const char *qi = getenv("NTR_QUEUE_INIT")) sc->queue_init = (uint32_t)strtoul(qi, nullptr, 10);
     if (const char *vl = getenv("NTR_VIEWS_PER_LAUNCH")) sc->views_per_launch = (uint32_t)strtoul(vl, nullptr, 10);
+    if (const char *rl = getenv("NTR_RAYS_PER_LAUNCH")) sc->rays_per_launch = (uint32_t)strtoul(rl, nullptr, 10);
     sc->tree_depth = depth;
     sc->dev.dim = desc->dim;
     sc->dev.kind = desc->kind;
@@ -2026,6 +2052,171 @@ NTR_API int ntr_occludes_rays(ntr_scene *sc, uint32_t n, const float *origins, c
     return NTR_OK;
 }
 
+
+// ---- batches of caller-given rays (ntr_render_rays) ----------------------------------------------------------------------
+// A launch covers at most kRaysPerLaunch rays: with two bounce records per ray the wavefront queues then stay at the 2^26
+// records a single frame is capped at.  Longer batches run as consecutive launches, each with the regrow-and-retry of a frame.
+static const uint32_t kRaysPerLaunch = 1u << 25;
+
+// the AOV buffers of a rays call -> *out (all nullptr for a NULL `aovs`); NTR_ERR_VALUE for a short one
+static int check_ray_aovs(uint32_t n, int dim, const ntr_aov_buffers *aovs, AovTarget *out) {
+    *out = AovTarget{};
+    if (!aovs) return NTR_OK;
+    const void *p[3] = {aovs->ids, aovs->depth, aovs->normals};
+    const size_t len[3] = {aovs->ids_len, aovs->depth_len, aovs->normals_len}, per[3] = {1, 1, (size_t)dim};
+    static const char *const name[3] = {"ids", "depth", "normals"};
+    for (int k = 0; k < 3; ++k) {
+        if (!p[k]) continue;
+        if (len[k] / per[k] < n) return fail(NTR_ERR_VALUE, "the %s buffer is too small for %u rays", name[k], n);
+        out->p[k] = const_cast<void *>(p[k]);
+    }
+    return NTR_OK;
+}
+
+static int check_rays(const ntr_scene *sc, uint32_t n, const float *origins, const float *dirs, const float *rgb,
+                      const ntr_aov_buffers *aovs, AovTarget *aov) {
+    if (n && (!origins || !dirs || !rgb)) return fail(NTR_ERR_VALUE, "NULL argument");
+    int rc = check_ray_aovs(n, sc->dev.dim, aovs, aov);
+    if (rc) return rc;
+    for (const FrameSlot &fs : sc->slots)
+        if (fs.open) return fail(NTR_ERR_RUNTIME, "the renderer is already running: a frame of ntr_render_begin is open");
+    return NTR_OK;
+}
+
+// One scene's share of a rays call, launch after launch.  Host arrays (`host`) go through the scene's scratch memory: the
+// rays of a launch are copied in, traced into the scratch accumulator and AOVs, and copied out once the launch needs no
+// retry.  Device arrays are read and written in place.
+struct RaysRun {
+    ntr_scene *sc = nullptr;
+    uint32_t n = 0, per = 1, done = 0;
+    const float *o = nullptr, *d = nullptr;     // ray 0 of the run
+    float *rgb = nullptr;
+    AovTarget aov;
+    cudaStream_t st = nullptr;
+    bool host = false;
+    size_t offs[4] = {};                        // scratch: origins, dirs, rgb, AOVs
+    FrameJob j{};
+    ntr_counters sum{};
+};
+
+static int rays_begin(RaysRun &r) {
+    ntr_scene *sc = r.sc;
+    r.per = std::max<uint32_t>(1, std::min<uint32_t>(sc->rays_per_launch ? sc->rays_per_launch : kRaysPerLaunch, std::max<uint32_t>(r.n, 1)));
+    if (!r.host || !r.n) return NTR_OK;
+    const size_t vb = (size_t)r.per * sc->dev.dim * sizeof(float);
+    const size_t sizes[4] = {vb, vb, (size_t)r.per * 3 * sizeof(float), (size_t)r.per * aov_pixel_bytes(r.aov, sc->dev.dim)};
+    return ray_batch_scratch(sc, r.per, r.offs, sizes, 4);
+}
+
+static int rays_submit(RaysRun &r) {
+    ntr_scene *sc = r.sc;
+    const int D = sc->dev.dim;
+    const uint32_t cnt = std::min(r.per, r.n - r.done);
+    RenderTarget tgt;
+    tgt.out_mode = NTR_OUT_RAYS;
+    if (r.host) {
+        unsigned char *b = static_cast<unsigned char *>(sc->d_scratch);
+        const size_t vb = (size_t)cnt * D * sizeof(float);
+        CUDA_TRY(cudaMemcpyAsync(b + r.offs[0], r.o + (size_t)r.done * D, vb, cudaMemcpyHostToDevice, r.st));
+        CUDA_TRY(cudaMemcpyAsync(b + r.offs[1], r.d + (size_t)r.done * D, vb, cudaMemcpyHostToDevice, r.st));
+        tgt.ray_o = (const float *)(b + r.offs[0]);
+        tgt.ray_d = (const float *)(b + r.offs[1]);
+        tgt.accum = (float *)(b + r.offs[2]);
+        tgt.aov = aov_packed(b + r.offs[3], r.aov, cnt, D);
+    } else {
+        tgt.ray_o = r.o + (size_t)r.done * D;
+        tgt.ray_d = r.d + (size_t)r.done * D;
+        tgt.accum = r.rgb + (size_t)r.done * 3;
+        tgt.aov = aov_offset(r.aov, r.done, D);
+    }
+    r.j = FrameJob{(int)cnt, 1, 0, 0, (int)cnt, 1, nullptr, tgt, 0, 1, 0, r.st};
+    r.j.restart_clock = r.done == 0;
+    int rc = frame_submit(sc, r.j);
+    if (!rc) rc = frame_readback(sc, r.j);
+    return rc;
+}
+
+// waits for the launch in flight; once it needs no retry, sums its counters and (host arrays) copies its results out
+static int rays_collect(RaysRun &r, bool *again) {
+    ntr_scene *sc = r.sc;
+    int rc = frame_collect(sc, r.j, again);
+    if (rc || *again) return rc;
+    add_counters(r.sum, sc->counters);
+    r.sum.queue_overflows = sc->counters.queue_overflows;
+    const uint32_t cnt = (uint32_t)r.j.win_w;
+    if (r.host) {
+        const int D = sc->dev.dim;
+        CUDA_TRY(cudaMemcpyAsync(r.rgb + (size_t)r.done * 3, r.j.tgt.accum, (size_t)cnt * 3 * sizeof(float), cudaMemcpyDeviceToHost, r.st));
+        const AovTarget into = aov_offset(r.aov, r.done, D);
+        for (int k = 0; k < 3; ++k)
+            if (into.p[k]) CUDA_TRY(cudaMemcpyAsync(into.p[k], r.j.tgt.aov.p[k], (size_t)cnt * aov_bytes(k, D), cudaMemcpyDeviceToHost, r.st));
+    }
+    r.done += cnt;
+    return NTR_OK;
+}
+
+// waits for the last copies and publishes the counters
+static int rays_finish(RaysRun &r, int rc) {
+    const cudaError_t e = cudaStreamSynchronize(r.st);
+    if (e != cudaSuccess && !rc) rc = fail(NTR_ERR_RUNTIME, "cudaStreamSynchronize failed: %s", cudaGetErrorString(e));
+    if (!rc) r.sc->counters = r.sum;
+    return rc;
+}
+
+static int rays_run(RaysRun &r) {
+    int rc = rays_begin(r);
+    for (int attempt = 0; !rc && r.done < r.n;) {
+        if (++attempt > 8) { rc = fail(NTR_ERR_RUNTIME, "wavefront queue kept overflowing"); break; }
+        bool again = false;
+        if (!(rc = rays_submit(r))) rc = rays_collect(r, &again);
+        if (!again) attempt = 0;
+    }
+    return rays_finish(r, rc);
+}
+
+NTR_API int ntr_render_rays(ntr_scene *sc, uint32_t n, const float *origins, const float *dirs, float *rgb_out,
+                            const ntr_aov_buffers *aovs) {
+    ENTER(sc);
+    AovTarget aov;
+    int rc = check_rays(sc, n, origins, dirs, rgb_out, aovs, &aov);
+    if (rc || !n) return rc;
+    RaysRun r;
+    r.sc = sc; r.n = n; r.o = origins; r.d = dirs; r.rgb = rgb_out; r.aov = aov; r.st = sc->stream; r.host = true;
+    return rays_run(r);
+}
+
+NTR_API int ntr_render_rays_device(ntr_scene *sc, uint32_t n, const float *origins, const float *dirs, float *rgb_out,
+                                   const ntr_aov_buffers *dev_aovs, void *stream) {
+    ENTER(sc);
+    AovTarget aov;
+    int rc = check_rays(sc, n, origins, dirs, rgb_out, dev_aovs, &aov);
+    if (rc || !n) return rc;
+    RaysRun r;
+    r.sc = sc; r.n = n; r.o = origins; r.d = dirs; r.rgb = rgb_out; r.aov = aov;
+    r.st = stream ? (cudaStream_t)stream : sc->stream;
+    const bool passes = sc->dev.kind == NTR_SCENE_COMPOSITE && sc->any_reflective && sc->dev.max_depth > 0;
+    if (passes) return rays_run(r);         // synchronous on the stream, as ntr_render_device with passes
+    // single-pass rays: every launch fully asynchronous on the caller's stream
+    if ((rc = rays_begin(r))) return rc;
+    CUDA_TRY(cudaEventRecord(sc->ev0, r.st));
+    for (; r.done < n; r.done += r.per) {
+        const uint32_t cnt = std::min(r.per, n - r.done);
+        RenderTarget tgt;
+        tgt.out_mode = NTR_OUT_RAYS;
+        tgt.ray_o = origins + (size_t)r.done * sc->dev.dim;
+        tgt.ray_d = dirs + (size_t)r.done * sc->dev.dim;
+        tgt.accum = rgb_out + (size_t)r.done * 3;
+        tgt.aov = aov_offset(aov, r.done, sc->dev.dim);
+        bool p = false;
+        if ((rc = enqueue_frame(sc, r.st, (int)cnt, 1, 0, 0, (int)cnt, 1, nullptr, tgt, 0, 1, 0, &p))) return rc;
+    }
+    CUDA_TRY(cudaEventRecord(sc->ev1, r.st));
+    sc->timing_valid = true;
+    sc->counters = ntr_counters{};
+    sc->counters.primary_rays = n;
+    return NTR_OK;
+}
+
 NTR_API int ntr_abort(ntr_scene *sc) {
     if (!sc) return fail(NTR_ERR_VALUE, "scene is NULL");
     // polled by every warp before it takes the next block of work.  Word 0: a synchronous call in progress, or an
@@ -2449,6 +2640,82 @@ NTR_API int ntr_group_render_views(ntr_group *g, int n, const float *origins, co
 NTR_API int ntr_group_render_views_aovs(ntr_group *g, int n, const float *origins, const float *axes, const ntr_image_format *fmt,
                                         void *dst, size_t dst_len, const ntr_aov_buffers *aovs) {
     return group_render_views(g, n, origins, axes, fmt, dst, dst_len, aovs);
+}
+
+// Rays dealt to the entries in contiguous ranges: entry i traces rays [i * n / G, (i + 1) * n / G) in its own device memory and
+// copies its results straight to their place.  Every round submits the next launch on every entry before it collects any.
+NTR_API int ntr_group_render_rays(ntr_group *g, uint32_t n, const float *origins, const float *dirs, float *rgb_out,
+                                  const ntr_aov_buffers *aovs) {
+    if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
+    const int G = (int)g->sc.size();
+    AovTarget aov;
+    for (ntr_scene *sc : g->sc) { const int rc = check_rays(sc, n, origins, dirs, rgb_out, aovs, &aov); if (rc) return rc; }
+    if (!n) return NTR_OK;
+    if (g->busy.exchange(true)) return fail(NTR_ERR_RUNTIME, "the renderer is already running");
+    struct Unbusy { ntr_group *g; ~Unbusy() { g->busy.store(false); } } unbusy{g};
+    for (int i = 0; i < G; ++i) {
+        ntr_scene *sc = g->sc[i];
+        if (sc->busy.exchange(true)) {
+            for (int k = 0; k < i; ++k) g->sc[k]->busy.store(false);
+            return fail(NTR_ERR_RUNTIME, "the renderer is already running");
+        }
+        sc->h_abort[0] = 0;
+        sc->abort_idx = 0;
+    }
+    struct Release { ntr_group *g; ~Release() { for (ntr_scene *s : g->sc) s->busy.store(false); } } release{g};
+    const int D = g->sc[0]->dev.dim;
+    std::vector<RaysRun> runs(G);
+    std::vector<int> attempts(G, 0);
+    int rc = NTR_OK;
+    CUDA_TRY(cudaSetDevice(g->dev[0]));
+    CUDA_TRY(cudaEventRecord(g->ev0, g->sc[0]->stream));
+    for (int i = 0; i < G && !rc; ++i) {
+        RaysRun &r = runs[i];
+        const uint32_t first = (uint32_t)((uint64_t)i * n / G);
+        r.sc = g->sc[i]; r.n = (uint32_t)((uint64_t)(i + 1) * n / G) - first;
+        r.o = origins + (size_t)first * D; r.d = dirs + (size_t)first * D; r.rgb = rgb_out + (size_t)first * 3;
+        r.aov = aov_offset(aov, first, D); r.st = g->sc[i]->stream; r.host = true;
+        CUDA_TRY(cudaSetDevice(g->dev[i]));
+        if (i) CUDA_TRY(cudaStreamWaitEvent(r.st, g->ev0, 0));      // the call's clock starts on dev[0]
+        rc = rays_begin(r);
+    }
+    for (bool any = true; any && !rc;) {
+        any = false;
+        std::vector<char> sent(G, 0);
+        for (int i = 0; i < G && !rc; ++i) {
+            if (runs[i].done >= runs[i].n) continue;
+            if (++attempts[i] > 8) { rc = fail(NTR_ERR_RUNTIME, "wavefront queue kept overflowing"); break; }
+            cudaSetDevice(g->dev[i]);
+            rc = rays_submit(runs[i]);
+            sent[i] = 1;
+            any = true;
+        }
+        for (int i = 0; i < G; ++i) {
+            if (!sent[i]) continue;
+            cudaSetDevice(g->dev[i]);
+            bool again = false;
+            const int r = rc == NTR_OK ? rays_collect(runs[i], &again) : (cudaStreamSynchronize(runs[i].st), NTR_OK);
+            if (r != NTR_OK && rc == NTR_OK) rc = r;
+            if (!again) attempts[i] = 0;
+        }
+    }
+    for (int i = 0; i < G; ++i) {
+        cudaSetDevice(g->dev[i]);
+        const int r = rays_finish(runs[i], rc);
+        if (r != NTR_OK && rc == NTR_OK) rc = r;
+        if (i) cudaEventRecord(g->done[i], runs[i].st);
+    }
+    CUDA_TRY(cudaSetDevice(g->dev[0]));
+    for (int i = 1; i < G; ++i) CUDA_TRY(cudaStreamWaitEvent(g->sc[0]->stream, g->done[i], 0));
+    CUDA_TRY(cudaEventRecord(g->ev1, g->sc[0]->stream));
+    g->timing_valid = rc == NTR_OK;
+    if (rc) return rc;
+    g->counters = ntr_counters{};
+    for (const RaysRun &r : runs) {
+        add_counters(g->counters, r.sum);
+        g->counters.queue_overflows += r.sum.queue_overflows;
+    }
+    return NTR_OK;
 }
 
 NTR_API int ntr_group_abort(ntr_group *g) {

@@ -86,7 +86,8 @@ struct FormatDev {
 enum : int {
     NTR_OUT_PACKED = 0,     // pack straight into the image format (no secondary passes needed)
     NTR_OUT_ACCUM = 1,      // float RGB accumulator (secondary passes add to it, a pack kernel follows)
-    NTR_OUT_IDS = 2         // primary hit ids + distances (parity hook)
+    NTR_OUT_IDS = 2,        // primary hit ids + distances (parity hook)
+    NTR_OUT_RAYS = 3        // a batch of caller-given rays (ntr_render_rays): float RGB per ray in the accumulator, no packing
 };
 
 struct FrameDev {
@@ -116,8 +117,9 @@ struct FrameDev {
     // words v * npix + pix (npix = win_w * out_rows), and its packed frame starts at packed + v * pitch * win_h
     const CameraDev *views;
     uint32_t n_views;
-    // AOVs of a batch of views (NTR_F_AOV), per pixel slot v * npix + pix, nullptr where not wanted: the flat id of the plain
-    // primary ray's opaque hit (-1: miss), its distance, and dim floats of the hit's normal.  aov_half_w / aov_half_h /
+    // AOVs of a batch of views (NTR_F_AOV), per pixel slot v * npix + pix, or of a batch of rays (render_rays_kernel), per ray;
+    // nullptr where not wanted: the flat id of the plain primary ray's opaque hit (-1: miss), its distance, and dim floats of
+    // the hit's normal.  aov_half_w / aov_half_h /
     // aov_fovI describe the plain (factor-1) view, whose ray a factor that is not a power of two traces separately.
     int32_t *aov_ids;
     float *aov_depth;

@@ -7,6 +7,8 @@
 //                       packing epilogue; secondary passes: the same per-ray code over a wavefront queue of
 //                       reflection bounces written by the previous pass with warp-aggregated atomics.
 //   pack_kernel         float accumulator -> ImageFormat bytes (reference process_pixel, src/render.cpp:396-466)
+//   render_rays_kernel  the primary pass of a batch of caller-given rays (ntr_render_rays); its bounces go to the
+//                       render_pass_kernel bounce passes
 //   trace_rays_kernel / occludes_rays_kernel   KDNode.intersects / KDNode.occludes parity hooks
 #pragma once
 #include <cuda_runtime.h>
@@ -415,6 +417,49 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
     flush_counters(ctl, cnt);
 }
 
+// The primary pass of a batch of caller-given rays (ntr_render_rays): origins / dirs are n x D, ray i takes accumulator slot i
+// and bounce-record pixel word i.  Work is handed out like the list pass: every fetch takes 32 rays, one per lane, and the
+// fetch whose range crosses a multiple of 8192 rays polls the abort flag.  The colour is stored over the slot (the bounce
+// passes add to it).  The AOVs (FrameDev::aov_*) are wanted where their pointer is set: checked at run time, one build.
+template <int DT, int FLAGS>
+__global__ void __launch_bounds__(kCtaThreads, MinCtas<DT, FLAGS>::value)
+render_rays_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ FrameDev f, const __grid_constant__ QueueDev q,
+                   const __grid_constant__ ControlDev ctl, const float *origins, const float *dirs, uint32_t n) {
+    constexpr int CAP = DimCap<DT>::value;
+    const int D = NTR_D(DT, s);
+    const int lane = threadIdx.x & 31;
+    const bool want_aov = f.aov_ids || f.aov_depth || f.aov_normals;
+    Counters cnt;
+    MailboxStore ms;
+    ms.attach((FLAGS & NTR_F_GENERAL) ? s.mb_table : nullptr, s.mb_words, s.mb_threads, blockIdx.x * blockDim.x + threadIdx.x, s.n_simplex, s.mb_shift);
+    for (;;) {
+        uint32_t b = 0;
+        if (lane == 0) b = atomicAdd(ctl.tile_cursor, 32u);
+        b = __shfl_sync(0xFFFFFFFFu, b, 0);
+        if (b >= n) break;
+        if ((b & 8191u) < 32u && *ctl.abort_flag) {
+            if (lane == 0) atomicAdd(ctl.tile_cursor, 0x40000000u);
+            break;
+        }
+        const uint32_t i = b + lane;
+        if (i < n) {
+            float o[CAP], dir[CAP], rgb[3];
+#pragma unroll
+            for (int k = 0; k < CAP; ++k) {
+                if (k < D) { o[k] = __ldg(origins + (size_t)i * D + k); dir[k] = __ldg(dirs + (size_t)i * D + k); }
+            }
+            QueueEmit<DT> emit{q, ctl, i, q.out != nullptr};
+            PrimaryAov<DT> aov;
+            given_ray_color<DT, FLAGS>(s, o, dir, rgb, emit, cnt, &ms, want_aov ? &aov : nullptr);
+            f.accum[(size_t)i * 3 + 0] = rgb[0]; f.accum[(size_t)i * 3 + 1] = rgb[1]; f.accum[(size_t)i * 3 + 2] = rgb[2];
+            if (want_aov) store_aov<DT>(s, f, i, aov);
+        }
+    }
+    __syncwarp();
+    ms.detach();
+    flush_counters(ctl, cnt);
+}
+
 // Next frame's tile schedule: tiles sorted by decreasing cost (rank by counting; n <= a few thousand tiles), costs
 // halved so that the schedule follows a moving camera with some inertia.
 static __global__ void order_tiles_kernel(unsigned long long *cost, uint32_t *order, uint32_t n) {
@@ -502,6 +547,9 @@ struct KernelSet {
     void (*occludes_rays)(dim3, dim3, cudaStream_t, const SceneDev &, uint32_t, const float *, const float *,
                           const float *, const uint32_t *, const int32_t *, int32_t *, int32_t *);
     int (*max_blocks_per_sm)();
+    void (*render_rays)(dim3, dim3, cudaStream_t, const SceneDev &, const FrameDev &, const QueueDev &, const ControlDev &,
+                        const float *, const float *, uint32_t);
+    int (*rays_blocks_per_sm)();
 };
 
 template <int DT, int FLAGS> struct Launch {
@@ -527,15 +575,29 @@ template <int DT, int FLAGS> struct Launch {
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, render_pass_kernel<DT, FLAGS>, kCtaThreads, 0);
         return n;
     }
-    // the ray hooks have no warp form: both render variants share them
+    static void render_rays(dim3 g, dim3 b, cudaStream_t st, const SceneDev &s, const FrameDev &f, const QueueDev &q,
+                            const ControlDev &ctl, const float *o, const float *d, uint32_t n) {
+        // NTR_LAUNCH_LOG=1: a line of its own, which the render_pass_kernel lines' pattern ("ntr launch ...") does not match
+        const char *log = getenv("NTR_LAUNCH_LOG");
+        if (log && atoi(log) != 0) fprintf(stderr, "ntr rays-launch family=%d flags=%d grid=%u\n", DT, FLAGS, g.x);
+        render_rays_kernel<DT, FLAGS><<<g, b, 0, st>>>(s, f, q, ctl, o, d, n);
+    }
+    static int rays_blocks_per_sm() {
+        int n = 0;
+        cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, render_rays_kernel<DT, FLAGS>, kCtaThreads, 0);
+        return n;
+    }
+    // the ray hooks and the ray-fed primary pass have no warp form: every render variant shares them
     static KernelSet get() {
-        return KernelSet{&render_pass, &Launch<DT, FLAGS & 3>::trace_rays, &Launch<DT, FLAGS & 3>::occludes_rays, &max_blocks_per_sm};
+        return KernelSet{&render_pass, &Launch<DT, FLAGS & 3>::trace_rays, &Launch<DT, FLAGS & 3>::occludes_rays, &max_blocks_per_sm,
+                         &Launch<DT, FLAGS & 3>::render_rays, &Launch<DT, FLAGS & 3>::rays_blocks_per_sm};
     }
 };
 
 // defined in kern_d*.cu: variant index = FLAGS (0..255; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
 // everywhere else the index falls back to the build without it; NTR_F_SS, NTR_F_LIST and NTR_F_VIEWS builds exist in the
-// per-lane, non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE; NTR_F_AOV builds exist with NTR_F_VIEWS only)
+// per-lane, non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE; NTR_F_AOV builds exist with NTR_F_VIEWS only).
+// render_rays_kernel is built per lane and non-wide, for FLAGS & 3 only (4 builds per family), like the ray hooks.
 const KernelSet *kernel_set_d3(int flags);
 const KernelSet *kernel_set_d4(int flags);
 const KernelSet *kernel_set_d5(int flags);

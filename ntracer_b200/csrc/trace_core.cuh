@@ -1638,6 +1638,27 @@ NTR_HD void plain_primary_hit(const SceneDev &s, const CameraDev &cam, const Fra
     }
 }
 
+// ---- caller-given primary rays (ntr_render_rays; no counterpart in the reference) -------------------------------------
+// The colour of primary ray (o, dir) into rgb[3], exactly as the plain primary pass colours a camera ray: box_color, or
+// ray_color at depth 0 with no source and weight 1 into a zero accumulator.  The direction is used as given.
+// aov (optional): receives the ray's opaque hit and the normal that shades it (ray_color's miss state and zeros on a miss).
+template <int DT, int FLAGS, typename EMIT>
+NTR_HD void given_ray_color(const SceneDev &s, const float *o, const float *dir, float *rgb, EMIT &emit, Counters &cnt,
+                            MailboxStore *ms, PrimaryAov<DT> *aov) {
+    if (aov) {
+        aov->hit.dist = 0; aov->hit.ref = NTR_NONE_REF; aov->hit.lane = -1;
+        for (int i = 0; i < DimCap<DT>::value; ++i) aov->n[i] = 0.0f;
+    }
+    rgb[0] = 0.0f; rgb[1] = 0.0f; rgb[2] = 0.0f;
+    if (s.kind == NTR_SCENE_BOX) {
+        box_color<DT>(s, o, dir, rgb, aov ? &aov->hit : nullptr, aov ? aov->n : nullptr);
+        return;
+    }
+    const float one[3] = {1.0f, 1.0f, 1.0f};
+    const Skip none = {NTR_NONE_REF, 0};
+    ray_color<DT, FLAGS>(s, true, o, dir, 0, none, one, rgb, emit, cnt, aov ? &aov->hit : nullptr, ms, aov ? aov->n : nullptr);
+}
+
 // ---- adaptive supersampling (ntr_scene_set_supersampling_threshold) -------------------------------------------------
 // Pixel (x, y) is refined -- traced again with ss_pixel_color -- iff, in some channel, the plain 1-spp colours of its
 // corner set {(x, y), (x+1, y), (x, y+1), (x+1, y+1)} intersected with the view span more than the threshold.
