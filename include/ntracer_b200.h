@@ -186,6 +186,33 @@ NTR_API int ntr_scene_set_supersampling_threshold(ntr_scene *scene, float thresh
  * was not adaptively supersampled has an all-zero mask.  NTR_ERR_RUNTIME before the first frame.  Either pointer may be
  * NULL. */
 NTR_API int ntr_last_refine_mask(ntr_scene *scene, uint8_t *mask_or_null, size_t len, uint64_t *count_or_null);
+/* The camera's projection (no counterpart in the reference, whose camera is the pinhole of flat_origin_ray_source,
+ * src/tracer.hpp:60-76).  Host state like the camera and the supersampling factor: read when a frame is enqueued
+ * (ntr_render_begin captures it).  Pixel coordinates stay integers with no half-pixel offset; half_w = W/2 and
+ * half_h = H/2 are those of the traced view (sW x sH at supersampling factor s); right, up, fwd are camera rows 0, 1, 2.
+ *   NTR_PROJ_PERSPECTIVE (the default): the reference's pinhole through fov, byte for byte; param is ignored.
+ *   NTR_PROJ_ORTHOGRAPHIC: param h = half the view's width in scene units (finite, > 0).  k = h / half_w (float),
+ *     origin + right*k*(x - half_w) - up*k*(y - half_h), direction fwd (normalised).  fov is ignored; the rays start on the
+ *     image plane through the camera origin.
+ *   NTR_PROJ_EQUIRECTANGULAR: param alpha = the horizontal field angle in radians, in (0, 2*pi].  a = alpha / (2*half_w),
+ *     theta = a*(x - half_w), phi = a*(y - half_h), direction cos(phi)*(sin(theta)*right + cos(theta)*fwd) - sin(phi)*up
+ *     (normalised) from the camera origin.  fov is ignored.  A W x W/2 frame at alpha = 2*pi is the whole sphere.
+ * Every path that honours the supersampling factor and threshold honours the projection, and so do ntr_primary_hit_ids and
+ * the views AOVs; ntr_trace_rays*, ntr_occludes_rays and ntr_render_rays ignore it as they ignore the camera.  At factors 2,
+ * 4 and 8 sample (0, 0) of a pixel is its plain ray bit for bit.  Counters are those of the perspective frame's definition.
+ * An unknown kind, or a parameter out of range, NaN or infinite -> NTR_ERR_VALUE. */
+#define NTR_PROJ_PERSPECTIVE 0
+#define NTR_PROJ_ORTHOGRAPHIC 1
+#define NTR_PROJ_EQUIRECTANGULAR 2
+NTR_API int ntr_scene_set_projection(ntr_scene *scene, int kind, float param);
+/* The primary rays of the width x height view under the scene's camera, fov and projection, computed on the device by the
+ * function the primary pass calls (the projection's counterpart of the reference's screen_coord_to_ray).  Ray y*width + x
+ * is pixel (x, y); origins_out and dirs_out are width*height x D floats.  Like ntr_primary_hit_ids it ignores the
+ * supersampling factor: (s*W, s*H) gives the samples of factor s.  NTR_ERR_VALUE: a size below 1, width*height >= 2^31 or a
+ * NULL pointer.  NTR_ERR_RUNTIME while a frame of the scene is rendering. */
+NTR_API int ntr_camera_rays(ntr_scene *scene, int width, int height, float *origins_out, float *dirs_out);
+/* The same into DEVICE memory of the scene's device, on a caller-supplied CUDA stream (NULL = the scene's own), asynchronously. */
+NTR_API int ntr_camera_rays_device(ntr_scene *scene, int width, int height, float *origins_out, float *dirs_out, void *stream);
 
 /* ---- the hot path ---------------------------------------------------------------------------- */
 /* Renders one frame into a HOST buffer: replaces worker_draw + process_pixel for all tiles
@@ -331,6 +358,8 @@ NTR_API int ntr_group_set_params(ntr_group *group, const ntr_scene_desc *desc);
 NTR_API int ntr_group_set_supersampling(ntr_group *group, int factor);
 /* ntr_scene_set_supersampling_threshold for every device of the group. */
 NTR_API int ntr_group_set_supersampling_threshold(ntr_group *group, float threshold);
+/* ntr_scene_set_projection for every device of the group. */
+NTR_API int ntr_group_set_projection(ntr_group *group, int kind, float param);
 /* ntr_last_refine_mask of the last group frame: every device writes its tile rows, the count is their sum. */
 NTR_API int ntr_group_last_refine_mask(ntr_group *group, uint8_t *mask_or_null, size_t len, uint64_t *count_or_null);
 /* ntr_render over the group: host destination, same contract (NTR_ERR_ABORTED after ntr_group_abort). */

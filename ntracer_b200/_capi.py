@@ -206,6 +206,9 @@ def load():
         'ntr_scene_set_params': (C.c_int, [vp, C.POINTER(SceneDesc)]),
         'ntr_scene_set_supersampling': (C.c_int, [vp, i32]),
         'ntr_scene_set_supersampling_threshold': (C.c_int, [vp, C.c_float]),
+        'ntr_scene_set_projection': (C.c_int, [vp, i32, C.c_float]),
+        'ntr_camera_rays': (C.c_int, [vp, i32, i32, vp, vp]),
+        'ntr_camera_rays_device': (C.c_int, [vp, i32, i32, vp, vp, vp]),
         'ntr_last_refine_mask': (C.c_int, [vp, vp, C.c_size_t, C.POINTER(C.c_uint64)]),
         'ntr_render': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t]),
         'ntr_render_device': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t, vp, i32, i32, i32]),
@@ -244,6 +247,7 @@ def load():
         'ntr_group_set_params': (C.c_int, [vp, C.POINTER(SceneDesc)]),
         'ntr_group_set_supersampling': (C.c_int, [vp, i32]),
         'ntr_group_set_supersampling_threshold': (C.c_int, [vp, C.c_float]),
+        'ntr_group_set_projection': (C.c_int, [vp, i32, C.c_float]),
         'ntr_group_last_refine_mask': (C.c_int, [vp, vp, C.c_size_t, C.POINTER(C.c_uint64)]),
         'ntr_group_render': (C.c_int, [vp, C.POINTER(ImageFormat), vp, C.c_size_t]),
         'ntr_group_render_device': (C.c_int, [vp, C.POINTER(ImageFormat), C.POINTER(vp)]),
@@ -280,6 +284,7 @@ EXPORTED_SYMBOLS = (
     'ntr_group_create', 'ntr_group_destroy', 'ntr_group_size', 'ntr_group_set_camera', 'ntr_group_set_params',
     'ntr_group_set_supersampling', 'ntr_scene_set_supersampling_threshold', 'ntr_last_refine_mask',
     'ntr_group_set_supersampling_threshold', 'ntr_group_last_refine_mask',
+    'ntr_scene_set_projection', 'ntr_group_set_projection', 'ntr_camera_rays', 'ntr_camera_rays_device',
     'ntr_group_render', 'ntr_group_render_device', 'ntr_group_render_views', 'ntr_group_render_views_aovs', 'ntr_group_render_rays',
     'ntr_group_abort', 'ntr_group_get_counters',
     'ntr_group_last_kernel_ms', 'ntr_group_launch_count',

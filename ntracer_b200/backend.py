@@ -5,6 +5,8 @@ ntracer_b200.tracern / ntracer_b200.render build flat scene dicts and drive this
 bench.py use it directly.  Every method goes through libntracer_b200.so -- there is no CPU path.
 """
 import ctypes as C
+import math
+import numbers
 
 import numpy as np
 
@@ -59,6 +61,37 @@ def _views_dest(dest, n, fmt):
 
 
 AOV_NAMES = ('ids', 'depth', 'normals')
+PROJECTIONS = ('perspective', 'orthographic', 'equirectangular')       # index = NTR_PROJ_*
+
+
+def projection_args(kind, param=None):
+    """The arguments of set_projection -> (kind, param) with param a float, or None for 'perspective' (whose parameter is
+    ignored).  TypeError: kind is not a string or param not a real number; ValueError: an unknown kind, 'orthographic'
+    without param, or param out of range (orthographic: finite and > 0; equirectangular: in (0, 2 pi], default 2 pi)."""
+    if not isinstance(kind, str):
+        raise TypeError('the projection must be one of %s' % ', '.join(map(repr, PROJECTIONS)))
+    if kind not in PROJECTIONS:
+        raise ValueError('unknown projection %r: one of %s' % (kind, ', '.join(map(repr, PROJECTIONS))))
+    if param is not None and (isinstance(param, bool) or not isinstance(param, numbers.Real)):
+        raise TypeError('the projection parameter must be a real number')
+    if kind == 'perspective':
+        return kind, None
+    if kind == 'orthographic':
+        if param is None:
+            raise ValueError('an orthographic projection needs its half width in scene units')
+        if not (math.isfinite(param) and param <= FLT_MAX and np.float32(param) > 0):
+            raise ValueError('the orthographic half width must be finite and > 0')
+        return kind, float(param)
+    param = 2 * math.pi if param is None else param
+    if not (np.float32(param) > 0 and np.float32(param) <= np.float32(2 * math.pi)):
+        raise ValueError('the equirectangular field angle must lie in (0, 2 pi] radians')
+    return kind, float(param)
+
+
+def _set_projection(obj, fn, kind, param):
+    kind, param = projection_args(kind, param)
+    _capi.check(fn(obj._h, PROJECTIONS.index(kind), 0.0 if param is None else param))
+    obj.projection = (kind, param)
 AOV_DTYPES = {'ids': np.int32, 'depth': np.float32, 'normals': np.float32}
 
 
@@ -144,6 +177,7 @@ class DeviceScene:
         self._open = {}
         self.supersampling = 1
         self.supersampling_threshold = None
+        self.projection = ('perspective', None)
         self._window = None                     # (width, height) of the last frame's window: the shape of refine_mask()
         desc, keep = _capi.make_desc(scene)
         _capi.check(self._lib.ntr_scene_create(C.byref(desc), device, C.byref(self._h)))
@@ -193,11 +227,38 @@ class DeviceScene:
         _capi.check(self._lib.ntr_scene_set_supersampling_threshold(self._h, -1.0 if threshold is None else float(threshold)))
         self.supersampling_threshold = None if threshold is None else float(threshold)
 
+    def set_projection(self, kind, param=None):
+        """The camera's projection: 'perspective' (the default), 'orthographic' (param: half the view's width in scene
+        units) or 'equirectangular' (param: the horizontal field angle in radians, default 2 pi); see projection_args."""
+        _set_projection(self, self._lib.ntr_scene_set_projection, kind, param)
+
     def refine_mask(self):
         """-> (mask, count): the refine mask of the last frame as a (height, width) uint8 array over its window (1 =
         refined; rows a sharded render does not own stay 0) and the number of refined pixels."""
         w, h = self._window if self._window else (0, 0)
         return _refine_mask(self._lib.ntr_last_refine_mask, self._h, w, h)
+
+    def camera_rays(self, width, height):
+        """The primary rays of the width x height view under the camera, fov and projection, as the device computes them
+        (the supersampling factor is not used) -> (origins, dirs), float32 (width * height, dim); ray y * width + x is pixel
+        (x, y).  render_rays of them gives render_float's colours."""
+        n = int(width) * int(height)
+        o = np.zeros((n, self.dim), np.float32)
+        d = np.zeros((n, self.dim), np.float32)
+        _capi.check(self._lib.ntr_camera_rays(self._h, int(width), int(height), _p(o), _p(d)))
+        return o, d
+
+    def camera_rays_device(self, width, height, origins, dirs, stream=0):
+        """camera_rays into float32 (width * height, dim) contiguous torch tensors of the scene's device, on a CUDA stream
+        handle (0: the scene's own stream), asynchronously.  TypeError: a wrong dtype or device; ValueError: a wrong shape."""
+        import torch
+        if not isinstance(origins, torch.Tensor):
+            raise TypeError('origins must be a torch tensor')
+        shape = (int(width) * int(height), self.dim)
+        o = _tensor(origins, 'origins', torch.float32, shape, self.device)
+        d = _tensor(dirs, 'dirs', torch.float32, shape, o.device.index)
+        _capi.check(self._lib.ntr_camera_rays_device(self._h, int(width), int(height), C.c_void_p(o.data_ptr()),
+                                                     C.c_void_p(d.data_ptr()), C.c_void_p(stream)))
 
     # ---- the hot path ----
     def render(self, fmt, dest=None):
@@ -414,6 +475,7 @@ class DeviceGroup:
         self.size = int(self._lib.ntr_group_size(self._h))
         self.supersampling = 1
         self.supersampling_threshold = None
+        self.projection = ('perspective', None)
         self._window = None
         if 'cam_origin' in scene and 'cam_axes' in scene:
             self.set_camera(scene['cam_origin'], scene['cam_axes'])
@@ -447,6 +509,10 @@ class DeviceGroup:
     def set_supersampling_threshold(self, threshold):
         _capi.check(self._lib.ntr_group_set_supersampling_threshold(self._h, -1.0 if threshold is None else float(threshold)))
         self.supersampling_threshold = None if threshold is None else float(threshold)
+
+    def set_projection(self, kind, param=None):
+        """DeviceScene.set_projection on every device of the group"""
+        _set_projection(self, self._lib.ntr_group_set_projection, kind, param)
 
     def refine_mask(self):
         """DeviceScene.refine_mask of the last group frame: every device's rows, their refined pixels summed."""

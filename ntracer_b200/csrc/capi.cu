@@ -183,7 +183,7 @@ struct ntr_scene {
     uint32_t *h_ctl = nullptr;              // pinned read-back of the control block and the counters (frame_readback)
     unsigned long long *h_cnt = nullptr;
     uint64_t launches = 0;
-    int grid_blocks[256] = {};         // per variant flags (NTR_F_SS, NTR_F_LIST, NTR_F_VIEWS and NTR_F_AOV included)
+    int grid_blocks[512] = {};         // per variant flags (NTR_F_SS, NTR_F_LIST, NTR_F_VIEWS, NTR_F_AOV and NTR_F_PROJ included)
     // NTR_F_WIDE builds (96 registers, 5 CTAs per SM): for frames sharded over 4 or more GPUs, whose passes all end in a few
     // long rays (measured, config 4: 1/4 share 20.9 -> 19.9 ms, 1/8 share 15.2 -> 14.4 ms; 1/2 share and whole frames lose
     // 2..12 %).  Picking the build per pass from pass times measured on the second and third frame of a view gained another
@@ -206,6 +206,13 @@ struct ntr_scene {
     uint32_t rays_prev_pass_count[kMaxPasses + 2] = {};
     int rays_grid[4] = {};
     uint32_t rays_per_launch = 0;
+    // the projection (ntr_scene_set_projection), read when a frame is enqueued, and the wavefront statistics of projected frames,
+    // kept apart like the views calls' (projected frames keep no tile schedule), so that a perspective frame makes the decisions
+    // it would have made without them
+    int proj = NTR_PROJ_PERSPECTIVE;
+    float proj_param = 0.0f;
+    float proj_pass_ns_per_ray = 0.0f;
+    uint32_t proj_prev_pass_count[kMaxPasses + 2] = {}, proj_prev_pass_count2[kMaxPasses + 2] = {};
     // begin/end frames (ntr_render_begin / ntr_render_end); a views call uses their device buffers, staging buffers, events and
     // copy stream for its double-buffered launches
     FrameSlot slots[NTR_FRAMES_IN_FLIGHT];
@@ -457,6 +464,10 @@ uint64_t count_halo(const FrameDev &f) {
 // A batch of caller-given rays (tgt.out_mode NTR_OUT_RAYS, factor 1) is a win_w x 1 window: render_rays_kernel traces ray i into
 // accumulator slot i, the bounce passes are the single frame's, nothing is packed, no tile schedule is kept and the refine-mask
 // record is left alone.
+// Under a projection other than the perspective one (sc->proj) every primary pass runs an NTR_F_PROJ build: a batch of views
+// its views builds; a single frame the views build too, as one view (FrameDev::n_views = 1, views = nullptr: the kernel's
+// camera) -- a hit-id frame with its ids and depth stored as AOVs -- and the list passes of an adaptive frame the NTR_F_LIST
+// one.  Such frames keep no tile schedule and keep wavefront statistics of their own.
 int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0, int y0, int win_w, int win_h,
                   const ntr_image_format *fmt, const RenderTarget &tgt, int tile_row_first, int tile_row_step,
                   int compact, bool *used_passes, const CameraDev *views = nullptr, uint32_t n_views = 0) {
@@ -481,19 +492,29 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     if (fmt) fill_format(f.fmt, fmt);
     f.views = views; f.n_views = n_views;
     const bool rays = tgt.out_mode == NTR_OUT_RAYS;
-    const bool aov = (n_views || rays) && tgt.aov.any();
+    const bool proj = !rays && sc->proj != NTR_PROJ_PERSPECTIVE;
+    AovTarget aovs = tgt.aov;
+    if (proj && tgt.out_mode == NTR_OUT_IDS) { aovs.p[0] = tgt.ids; aovs.p[1] = tgt.dists; }
+    const bool aov = (n_views || rays || proj) && aovs.any();
+    if (proj) {
+        f.proj = sc->proj;
+        f.proj_k = projection_k(sc->proj, sc->proj_param, f.half_w);
+        if (!n_views) f.n_views = 1;
+    }
     if (aov) {
-        f.aov_ids = static_cast<int32_t *>(tgt.aov.p[0]);
-        f.aov_depth = static_cast<float *>(tgt.aov.p[1]);
-        f.aov_normals = static_cast<float *>(tgt.aov.p[2]);
+        f.aov_ids = static_cast<int32_t *>(aovs.p[0]);
+        f.aov_depth = static_cast<float *>(aovs.p[1]);
+        f.aov_normals = static_cast<float *>(aovs.p[2]);
         // the plain frame's ray parameters, as ntr_primary_hit_ids sets them (factor 1)
         f.aov_half_w = (float)width / 2.0f;
         f.aov_half_h = (float)height / 2.0f;
         f.aov_fovI = tanf(sc->dev.fov / 2) / f.aov_half_w;
+        if (proj) f.aov_proj_k = projection_k(sc->proj, sc->proj_param, f.aov_half_w);
     }
     const size_t nv = n_views ? n_views : 1;
     // wavefront statistics of the previous frame (of the previous views call, for a batch of views)
-    float &pass_ns_per_ray = rays ? sc->rays_pass_ns_per_ray : n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray;
+    float &pass_ns_per_ray = rays ? sc->rays_pass_ns_per_ray : n_views ? sc->views_pass_ns_per_ray
+                             : proj ? sc->proj_pass_ns_per_ray : sc->pass_ns_per_ray;
 
     // Scenes with big leaves: the bounce passes run the warp-synchronous kernels (incoherent rays; lanes that run out of
     // work help the ones parked at big leaves), the primary pass every lane for itself (the 32 rays of an 8x4 pixel block
@@ -541,7 +562,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     // whole frame on one GPU (loss of row-major locality + the cost bookkeeping), so it is used for sharded renders --
     // and for whole frames of scenes with giant leaves, whose few blocks through the centre cost 10-90x the mean
     // (config 4: primary pass 11.2-11.6 -> 10.4 ms, frame 43.3 -> 42.4 ms, calls 17 and 20)
-    const bool use_sched = n_tiles >= 64 && composite && tgt.out_mode != NTR_OUT_IDS && !rays && !sc->no_tile_sched &&
+    const bool use_sched = n_tiles >= 64 && composite && tgt.out_mode != NTR_OUT_IDS && !rays && !proj && !sc->no_tile_sched &&
                            (f.tile_row_step > 1 || sc->force_tile_sched || sc->max_leaf >= 256);
     const int slot = n_views ? kSchedViews : sc->ctl_slot;
     if (use_sched) {
@@ -594,13 +615,13 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     const uint32_t wide_now = wide_ok && (sc->wide_mode == 1 || f.tile_row_step >= 4) ? 0xFFFFFFFFu : 0u;
     auto wide_for = [&](int pass) { return (wide_now >> pass) & 1u ? (int)NTR_F_WIDE : 0; };
     // a supersampled primary pass runs the per-lane, non-wide NTR_F_SS build whatever NTR_WARP / NTR_WIDE say (kernels.cuh)
-    // a batch of views runs the per-lane, non-wide NTR_F_VIEWS build at every factor, 1 included; no more CTAs than the exact
-    // mailbox has columns
-    const int pflags = n_views ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_VIEWS | (aov ? NTR_F_AOV : 0)
+    // a batch of views, and any projected frame, runs the per-lane, non-wide NTR_F_VIEWS build at every factor, 1 included; no
+    // more CTAs than the exact mailbox has columns
+    const int pflags = n_views || proj ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_VIEWS | (aov ? NTR_F_AOV : 0) | (proj ? NTR_F_PROJ : 0)
                        : ss > 1 ? (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_SS : primary_flags | wide_for(0);
     const KernelSet *ks = sc->kset(pflags);
     int grid = grid_for(sc, pflags);
-    if (n_views && sc->dev.mb_table) grid = std::min(grid, (int)(sc->dev.mb_threads / kCtaThreads));
+    if ((n_views || proj) && sc->dev.mb_table) grid = std::min(grid, (int)(sc->dev.mb_threads / kCtaThreads));
     const uint32_t rec4 = 2 + 2 * ((sc->dev.dim + 3) / 4);
     QueueDev q;
     memset(&q, 0, sizeof q);
@@ -650,7 +671,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
     }
     // the list-driven primary passes of an adaptive frame: per-lane, non-wide NTR_F_LIST builds; no more CTAs than the
     // exact mailbox has columns
-    const int lflags = (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_LIST;
+    const int lflags = (flags & (NTR_F_GENERAL | NTR_F_COUNT)) | NTR_F_LIST | (proj ? NTR_F_PROJ : 0);
     auto list_pass = [&](const FrameDev &fl, uint32_t *cursor, QueueDev ql) {
         ControlDev cl = ctl;
         cl.tile_cursor = cursor;
@@ -729,7 +750,8 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         return NTR_OK;
     };
     if (passes) {
-        const int rc = bounces(CTL_COUNT0, CTL_CURSOR0, rays ? sc->rays_prev_pass_count : n_views ? sc->views_prev_pass_count : sc->prev_pass_count);
+        const int rc = bounces(CTL_COUNT0, CTL_CURSOR0, rays ? sc->rays_prev_pass_count : n_views ? sc->views_prev_pass_count
+                                                        : proj ? sc->proj_prev_pass_count : sc->prev_pass_count);
         if (rc) return rc;
     }
     if (adaptive) {
@@ -753,6 +775,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         fr.half_w = (float)fr.width / 2.0f;
         fr.half_h = (float)fr.height / 2.0f;
         fr.fovI = tanf(sc->dev.fov / 2) / fr.half_w;
+        if (proj) fr.proj_k = projection_k(sc->proj, sc->proj_param, fr.half_w);
         fr.list = sc->d_list;
         fr.list_count = d_ctl + CTL_REFINED;
         QueueDev qr;
@@ -762,7 +785,7 @@ int enqueue_frame(ntr_scene *sc, cudaStream_t st, int width, int height, int x0,
         qr.out_count = d_ctl + CTL_COUNT0B + 1;
         list_pass(fr, d_ctl + CTL_LIST_CURSOR, qr);
         mark();
-        if (passes && (rc = bounces(CTL_COUNT0B, CTL_CURSOR0B, sc->prev_pass_count2))) return rc;
+        if (passes && (rc = bounces(CTL_COUNT0B, CTL_CURSOR0B, proj ? sc->proj_prev_pass_count2 : sc->prev_pass_count2))) return rc;
     }
     if ((passes || adaptive) && tgt.out_mode == NTR_OUT_PACKED) {
         f.out_mode = NTR_OUT_PACKED;
@@ -799,10 +822,12 @@ struct FrameJob {
     const CameraDev *views = nullptr;   // a batch of views (device array) and its size; 0: one frame through the scene's camera
     uint32_t n_views = 0;
     bool restart_clock = true;          // false: ev0 keeps marking the start of an earlier launch of the same call
+    bool proj = false;                  // the last submit ran under a projection other than the perspective one
 };
 
 int frame_submit(ntr_scene *sc, FrameJob &j) {
     if (j.restart_clock) CUDA_TRY(cudaEventRecord(sc->ev0, j.st));
+    j.proj = j.tgt.out_mode != NTR_OUT_RAYS && sc->proj != NTR_PROJ_PERSPECTIVE;
     int rc = enqueue_frame(sc, j.st, j.width, j.height, j.x0, j.y0, j.win_w, j.win_h, j.fmt, j.tgt, j.trf, j.trs, j.compact, &j.passes,
                            j.views, j.n_views);
     if (rc) return rc;
@@ -832,14 +857,15 @@ int frame_collect(ntr_scene *sc, FrameJob &j, bool *again) {
         if (adaptive)
             for (int d = 1; d <= sc->dev.max_depth && d <= kMaxPasses; ++d) rays += std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
         if (rays > 0)
-            (j.tgt.out_mode == NTR_OUT_RAYS ? sc->rays_pass_ns_per_ray : j.n_views ? sc->views_pass_ns_per_ray : sc->pass_ns_per_ray) =
-                ms * 1e6f / (float)rays;
+            (j.tgt.out_mode == NTR_OUT_RAYS ? sc->rays_pass_ns_per_ray : j.n_views ? sc->views_pass_ns_per_ray
+             : j.proj ? sc->proj_pass_ns_per_ray : sc->pass_ns_per_ray) = ms * 1e6f / (float)rays;
     }
     uint32_t *const prev = j.tgt.out_mode == NTR_OUT_RAYS ? sc->rays_prev_pass_count
-                           : j.n_views ? sc->views_prev_pass_count : sc->prev_pass_count;
+                           : j.n_views ? sc->views_prev_pass_count : j.proj ? sc->proj_prev_pass_count : sc->prev_pass_count;
+    uint32_t *const prev2 = j.proj ? sc->proj_prev_pass_count2 : sc->prev_pass_count2;
     if (j.passes) for (int d = 1; d <= kMaxPasses; ++d) prev[d] = std::min(h_ctl[CTL_COUNT0 + d], sc->queue_capacity);
     if (j.passes && adaptive)
-        for (int d = 1; d <= kMaxPasses; ++d) sc->prev_pass_count2[d] = std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
+        for (int d = 1; d <= kMaxPasses; ++d) prev2[d] = std::min(h_ctl[CTL_COUNT0B + d], sc->queue_capacity);
     if (sc->pass_timing && sc->n_pass_ev > 1) {
         fprintf(stderr, "ntr pass ms:");
         for (int i = 0; i + 1 < sc->n_pass_ev; ++i) {
@@ -1311,6 +1337,30 @@ NTR_API int ntr_scene_set_supersampling_threshold(ntr_scene *sc, float threshold
     if (isnan(threshold) || threshold == INFINITY) return fail(NTR_ERR_VALUE, "the supersampling threshold must be a finite number (negative: off)");
     if (sc->busy) return fail(NTR_ERR_RUNTIME, "the scene is locked while rendering");
     sc->ss_threshold = threshold < 0.0f ? -1.0f : threshold;
+    return NTR_OK;
+}
+
+static int check_projection(int kind, float param) {
+    if (kind == NTR_PROJ_PERSPECTIVE) return NTR_OK;
+    if (kind == NTR_PROJ_ORTHOGRAPHIC) {
+        if (!(param > 0.0f && param < INFINITY)) return fail(NTR_ERR_VALUE, "the orthographic half width must be finite and positive");
+        return NTR_OK;
+    }
+    if (kind == NTR_PROJ_EQUIRECTANGULAR) {
+        if (!(param > 0.0f && param <= 6.283185307179586f))     // 2 pi, rounded to float
+            return fail(NTR_ERR_VALUE, "the equirectangular field angle must lie in (0, 2*pi] radians");
+        return NTR_OK;
+    }
+    return fail(NTR_ERR_VALUE, "unknown projection kind %d", kind);
+}
+
+NTR_API int ntr_scene_set_projection(ntr_scene *sc, int kind, float param) {
+    if (!sc) return fail(NTR_ERR_VALUE, "scene is NULL");
+    int rc = check_projection(kind, param);
+    if (rc) return rc;
+    if (sc->busy) return fail(NTR_ERR_RUNTIME, "the scene is locked while rendering");
+    sc->proj = kind;
+    sc->proj_param = kind == NTR_PROJ_PERSPECTIVE ? 0.0f : param;
     return NTR_OK;
 }
 
@@ -1963,6 +2013,55 @@ NTR_API int ntr_primary_hit_ids(ntr_scene *sc, int width, int height, int32_t *i
     return NTR_OK;
 }
 
+// ---- the camera's rays (ntr_camera_rays) ------------------------------------------------------------------------------
+static int check_camera_rays(int width, int height, const float *o, const float *d) {
+    if (width < 1 || height < 1 || (uint64_t)width * (uint64_t)height >= (1ull << 31))
+        return fail(NTR_ERR_VALUE, "width and height must be at least 1, and width * height below 2^31");
+    if (!o || !d) return fail(NTR_ERR_VALUE, "NULL argument");
+    return NTR_OK;
+}
+
+// Enqueues camera_rays_kernel for the width x height view at factor 1, with the frame parameters enqueue_frame gives it.
+static int enqueue_camera_rays(ntr_scene *sc, cudaStream_t st, int width, int height, float *o, float *d) {
+    FrameDev f;
+    memset(&f, 0, sizeof f);
+    f.ss = 1;
+    f.width = width; f.height = height;
+    f.half_w = (float)width / 2.0f;
+    f.half_h = (float)height / 2.0f;
+    f.fovI = tanf(sc->dev.fov / 2) / f.half_w;
+    f.proj = sc->proj;
+    if (sc->proj != NTR_PROJ_PERSPECTIVE) f.proj_k = projection_k(sc->proj, sc->proj_param, f.half_w);
+    const uint64_t n = (uint64_t)width * height;
+    const int blocks = (int)std::min<uint64_t>((n + kCtaThreads - 1) / kCtaThreads, (uint64_t)sc->sm_count * 16);
+    sc->kset(0)->camera_rays(dim3(blocks), dim3(kCtaThreads), st, sc->dev, sc->cam, f, o, d);
+    ++sc->launches;
+    CUDA_TRY(cudaGetLastError());
+    return NTR_OK;
+}
+
+NTR_API int ntr_camera_rays(ntr_scene *sc, int width, int height, float *origins_out, float *dirs_out) {
+    ENTER(sc);
+    int rc = check_camera_rays(width, height, origins_out, dirs_out);
+    if (rc) return rc;
+    const size_t bytes = (size_t)width * height * sc->dev.dim * sizeof(float), off = align_up(bytes, 256);
+    if ((rc = ensure(&sc->d_scratch, &sc->scratch_cap, 2 * off))) return rc;
+    float *d_o = static_cast<float *>(sc->d_scratch);
+    float *d_d = reinterpret_cast<float *>(static_cast<unsigned char *>(sc->d_scratch) + off);
+    if ((rc = enqueue_camera_rays(sc, sc->stream, width, height, d_o, d_d))) return rc;
+    CUDA_TRY(cudaMemcpyAsync(origins_out, d_o, bytes, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaMemcpyAsync(dirs_out, d_d, bytes, cudaMemcpyDeviceToHost, sc->stream));
+    CUDA_TRY(cudaStreamSynchronize(sc->stream));
+    return NTR_OK;
+}
+
+NTR_API int ntr_camera_rays_device(ntr_scene *sc, int width, int height, float *origins_out, float *dirs_out, void *stream) {
+    ENTER(sc);
+    int rc = check_camera_rays(width, height, origins_out, dirs_out);
+    if (rc) return rc;
+    return enqueue_camera_rays(sc, stream ? (cudaStream_t)stream : sc->stream, width, height, origins_out, dirs_out);
+}
+
 static int ray_batch_scratch(ntr_scene *sc, uint32_t n, size_t *offs, const size_t *sizes, int count) {
     size_t total = 0;
     for (int i = 0; i < count; ++i) { offs[i] = total; total += align_up(sizes[i], 256); }
@@ -2463,6 +2562,12 @@ NTR_API int ntr_group_set_supersampling(ntr_group *g, int factor) {
 NTR_API int ntr_group_set_supersampling_threshold(ntr_group *g, float threshold) {
     if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
     for (ntr_scene *sc : g->sc) { const int rc = ntr_scene_set_supersampling_threshold(sc, threshold); if (rc) return rc; }
+    return NTR_OK;
+}
+
+NTR_API int ntr_group_set_projection(ntr_group *g, int kind, float param) {
+    if (!g) return fail(NTR_ERR_VALUE, "group is NULL");
+    for (ntr_scene *sc : g->sc) { int rc = ntr_scene_set_projection(sc, kind, param); if (rc) return rc; }
     return NTR_OK;
 }
 

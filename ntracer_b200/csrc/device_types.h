@@ -43,8 +43,11 @@ enum : int {
     NTR_F_VIEWS = 64,       // render_pass_kernel only, per-lane form: the primary pass of a batch of views (ntr_render_views,
                             // FrameDev::views): the blocks of all views in one launch, every lane traces its pixel with
                             // ss_pixel_color at factor FrameDev::ss (1 included) through the camera of its view
-    NTR_F_AOV = 128         // with NTR_F_VIEWS only: the lane also stores the hit id, depth and normal of its pixel's plain
+    NTR_F_AOV = 128,        // with NTR_F_VIEWS only: the lane also stores the hit id, depth and normal of its pixel's plain
                             // (factor-1) primary ray into FrameDev::aov_* (ntr_render_views_aovs)
+    NTR_F_PROJ = 256        // with NTR_F_VIEWS, NTR_F_VIEWS | NTR_F_AOV or NTR_F_LIST only: the ray generator switches at run time on
+                            // FrameDev::proj (ntr_scene_set_projection, trace_core.cuh: primary_ray_at); a frame with views ==
+                            // nullptr traces its one view through the kernel's camera parameter
 };
 
 struct SceneDev {
@@ -125,6 +128,10 @@ struct FrameDev {
     float *aov_depth;
     float *aov_normals;
     float aov_half_w, aov_half_h, aov_fovI;
+    // the projection (ntr_scene_set_projection), read by the NTR_F_PROJ builds and camera_rays_kernel only: the kind
+    // (NTR_PROJ_*), proj_k = k or a of the view f describes, aov_proj_k that of the plain view (trace_core.cuh: projection_k)
+    int proj;
+    float proj_k, aov_proj_k;
 };
 
 // One deferred ray of the wavefront (a reflection bounce): 16-byte aligned record.

@@ -9,6 +9,7 @@
 //   pack_kernel         float accumulator -> ImageFormat bytes (reference process_pixel, src/render.cpp:396-466)
 //   render_rays_kernel  the primary pass of a batch of caller-given rays (ntr_render_rays); its bounces go to the
 //                       render_pass_kernel bounce passes
+//   camera_rays_kernel  the primary rays of a view under the scene's projection (ntr_camera_rays)
 //   trace_rays_kernel / occludes_rays_kernel   KDNode.intersects / KDNode.occludes parity hooks
 #pragma once
 #include <cuda_runtime.h>
@@ -176,7 +177,8 @@ __device__ __forceinline__ void list_pass(const SceneDev &s, const CameraDev &ca
         if (inside) {
             float acc[3];
             QueueEmit<DT> emit{q, ctl, slot, q.out != nullptr};
-            ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT)>(s, cam, f, f.x0 + wx, f.y0 + wy, acc, emit, cnt, &ms);
+            ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, false, (FLAGS & NTR_F_PROJ) != 0>(
+                s, cam, f, f.x0 + wx, f.y0 + wy, acc, emit, cnt, &ms);
             f.accum[(size_t)slot * 3 + 0] = acc[0]; f.accum[(size_t)slot * 3 + 1] = acc[1]; f.accum[(size_t)slot * 3 + 2] = acc[2];
         }
     }
@@ -223,6 +225,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
     // One loop serves both kinds of pass so that the per-ray code (ray_color and everything it inlines) exists
     // exactly once in the kernel: only the work fetch and the epilogue differ.
     constexpr bool VIEWS = (FLAGS & NTR_F_VIEWS) != 0;
+    constexpr bool PROJ = (FLAGS & NTR_F_PROJ) != 0;
     const bool primary = (FLAGS & (NTR_F_SS | NTR_F_VIEWS)) != 0 || q.in == nullptr;   // NTR_F_SS / NTR_F_VIEWS builds only run primary passes
     const int my_rows = f.tile_row_first < f.tiles_y
                             ? (f.tiles_y - f.tile_row_first + f.tile_row_step - 1) / f.tile_row_step : 0;
@@ -309,16 +312,18 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
             if (inside) {
                 if constexpr (VIEWS) {
                     // the view's camera is read from global memory where it is used (by reference), not copied to registers;
-                    // at factor 1 the pixel gets the plain path's bits (ss_pixel_color, EXACT1)
+                    // at factor 1 the pixel gets the plain path's bits (ss_pixel_color, EXACT1).  A projected single frame
+                    // (NTR_F_PROJ, views == nullptr) is one view through the kernel's camera parameter.
                     QueueEmit<DT> emit{q, ctl, pix, f.out_mode == NTR_OUT_ACCUM};
+                    const CameraDev &vcam = PROJ && !f.views ? cam : f.views[view];
                     if constexpr ((FLAGS & NTR_F_AOV) != 0) {
                         PrimaryAov<DT> aov;
-                        ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true>(s, f.views[view], f, f.x0 + px, f.y0 + py,
-                                                                                                        acc, emit, cnt, &ms, &aov);
+                        ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true, PROJ>(s, vcam, f, f.x0 + px, f.y0 + py,
+                                                                                                              acc, emit, cnt, &ms, &aov);
                         store_aov<DT>(s, f, pix, aov);
                     } else {
-                        ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true>(s, f.views[view], f, f.x0 + px, f.y0 + py,
-                                                                                                        acc, emit, cnt, &ms);
+                        ss_pixel_color<DT, FLAGS & (NTR_F_GENERAL | NTR_F_COUNT), QueueEmit<DT>, true, PROJ>(s, vcam, f, f.x0 + px, f.y0 + py,
+                                                                                                              acc, emit, cnt, &ms);
                     }
                 } else if constexpr ((FLAGS & NTR_F_SS) != 0) {
                     // supersampled frame: the lane traces the ss x ss samples of its pixel right here, one after the other
@@ -362,7 +367,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
         // warp-synchronous form (trace_warp.cuh: all 32 lanes enter, `active` says who has a ray; rays park at big leaves
         // and the warp splits them over its lanes when enough lanes are idle) wins where single rays walk leaves of
         // hundreds of items (config 4: 58.4 -> 49.9 ms, its 1/8-frame share 26.3 -> 19.9 ms).
-        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE | NTR_F_SS | NTR_F_VIEWS | NTR_F_AOV);      // the per-ray code knows nothing of the switches
+        constexpr int RF = FLAGS & ~(NTR_F_WARP | NTR_F_WIDE | NTR_F_SS | NTR_F_VIEWS | NTR_F_AOV | NTR_F_PROJ);   // the per-ray code knows nothing of the switches
         if constexpr ((FLAGS & NTR_F_WARP) != 0) {
             if (s.kind != NTR_SCENE_BOX) {          // warp-uniform
                 if (!active) {
@@ -406,7 +411,7 @@ render_pass_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ C
         } else if (inside) {
             if (f.out_mode == NTR_OUT_ACCUM) {
                 f.accum[(size_t)pix * 3 + 0] = acc[0]; f.accum[(size_t)pix * 3 + 1] = acc[1]; f.accum[(size_t)pix * 3 + 2] = acc[2];
-            } else {
+            } else if constexpr (!PROJ) {       // a projected hit-id frame stores its ids and depth as AOVs (NTR_F_AOV)
                 f.ids[pix] = prim.ref == NTR_NONE_REF ? -1 : (s.kind == NTR_SCENE_BOX ? 0 : flat_prim_id(s, prim.ref, prim.lane));
                 if (f.dists) f.dists[pix] = prim.dist;
             }
@@ -458,6 +463,26 @@ render_rays_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ F
     __syncwarp();
     ms.detach();
     flush_counters(ctl, cnt);
+}
+
+// The primary rays of the f.width x f.height view f describes (ntr_camera_rays): ray i = y * width + x is pixel (x, y), its
+// origin and direction D floats each at origins / dirs + i * D.  primary_ray with PROJ is the function the NTR_F_PROJ passes
+// call, and under the perspective projection the plain passes' primary_ray_of.
+template <int DT>
+__global__ void __launch_bounds__(kCtaThreads)
+camera_rays_kernel(const __grid_constant__ SceneDev s, const __grid_constant__ CameraDev cam, const __grid_constant__ FrameDev f,
+                   float *origins, float *dirs) {
+    constexpr int CAP = DimCap<DT>::value;
+    const int D = NTR_D(DT, s);
+    const uint32_t n = (uint32_t)f.width * (uint32_t)f.height;
+    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n; i += gridDim.x * blockDim.x) {
+        float o[CAP], dir[CAP];
+        primary_ray<DT, true>(s, cam, f, (int)(i % (uint32_t)f.width), (int)(i / (uint32_t)f.width), o, dir);
+#pragma unroll
+        for (int k = 0; k < CAP; ++k) {
+            if (k < D) { origins[(size_t)i * D + k] = o[k]; dirs[(size_t)i * D + k] = dir[k]; }
+        }
+    }
 }
 
 // Next frame's tile schedule: tiles sorted by decreasing cost (rank by counting; n <= a few thousand tiles), costs
@@ -550,6 +575,7 @@ struct KernelSet {
     void (*render_rays)(dim3, dim3, cudaStream_t, const SceneDev &, const FrameDev &, const QueueDev &, const ControlDev &,
                         const float *, const float *, uint32_t);
     int (*rays_blocks_per_sm)();
+    void (*camera_rays)(dim3, dim3, cudaStream_t, const SceneDev &, const CameraDev &, const FrameDev &, float *, float *);
 };
 
 template <int DT, int FLAGS> struct Launch {
@@ -587,17 +613,26 @@ template <int DT, int FLAGS> struct Launch {
         cudaOccupancyMaxActiveBlocksPerMultiprocessor(&n, render_rays_kernel<DT, FLAGS>, kCtaThreads, 0);
         return n;
     }
-    // the ray hooks and the ray-fed primary pass have no warp form: every render variant shares them
+    static void camera_rays(dim3 g, dim3 b, cudaStream_t st, const SceneDev &s, const CameraDev &cam, const FrameDev &f, float *o,
+                            float *d) {
+        const char *log = getenv("NTR_LAUNCH_LOG");
+        if (log && atoi(log) != 0) fprintf(stderr, "ntr camrays-launch family=%d grid=%u\n", DT, g.x);
+        camera_rays_kernel<DT><<<g, b, 0, st>>>(s, cam, f, o, d);
+    }
+    // the ray hooks and the ray-fed primary pass have no warp form: every render variant shares them; camera_rays_kernel has
+    // one build per family
     static KernelSet get() {
         return KernelSet{&render_pass, &Launch<DT, FLAGS & 3>::trace_rays, &Launch<DT, FLAGS & 3>::occludes_rays, &max_blocks_per_sm,
-                         &Launch<DT, FLAGS & 3>::render_rays, &Launch<DT, FLAGS & 3>::rays_blocks_per_sm};
+                         &Launch<DT, FLAGS & 3>::render_rays, &Launch<DT, FLAGS & 3>::rays_blocks_per_sm, &Launch<DT, 0>::camera_rays};
     }
 };
 
-// defined in kern_d*.cu: variant index = FLAGS (0..255; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
+// defined in kern_d*.cu: variant index = FLAGS (0..511; NTR_F_WIDE builds exist for the general variant in 3..5 dimensions,
 // everywhere else the index falls back to the build without it; NTR_F_SS, NTR_F_LIST and NTR_F_VIEWS builds exist in the
-// per-lane, non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE; NTR_F_AOV builds exist with NTR_F_VIEWS only).
-// render_rays_kernel is built per lane and non-wide, for FLAGS & 3 only (4 builds per family), like the ray hooks.
+// per-lane, non-wide form only, so they override NTR_F_WARP and NTR_F_WIDE; NTR_F_AOV builds exist with NTR_F_VIEWS only;
+// NTR_F_PROJ builds exist with NTR_F_VIEWS, NTR_F_VIEWS | NTR_F_AOV and NTR_F_LIST only, 12 per family).
+// render_rays_kernel is built per lane and non-wide, for FLAGS & 3 only (4 builds per family), like the ray hooks;
+// camera_rays_kernel once per family.
 const KernelSet *kernel_set_d3(int flags);
 const KernelSet *kernel_set_d4(int flags);
 const KernelSet *kernel_set_d5(int flags);
@@ -609,6 +644,16 @@ const KernelSet *kernel_set_d10(int flags);
 const KernelSet *kernel_set_dn(int flags);
 
 #define NTR_SS_SETS(DT)                                                                                 \
+        static const KernelSet proj_views[4] = {Launch<DT, NTR_F_VIEWS | NTR_F_PROJ>::get(), Launch<DT, 1 | NTR_F_VIEWS | NTR_F_PROJ>::get(), \
+                                                Launch<DT, 2 | NTR_F_VIEWS | NTR_F_PROJ>::get(), Launch<DT, 3 | NTR_F_VIEWS | NTR_F_PROJ>::get()}; \
+        static const KernelSet proj_aovs[4] = {Launch<DT, NTR_F_VIEWS | NTR_F_AOV | NTR_F_PROJ>::get(),            \
+                                               Launch<DT, 1 | NTR_F_VIEWS | NTR_F_AOV | NTR_F_PROJ>::get(),        \
+                                               Launch<DT, 2 | NTR_F_VIEWS | NTR_F_AOV | NTR_F_PROJ>::get(),        \
+                                               Launch<DT, 3 | NTR_F_VIEWS | NTR_F_AOV | NTR_F_PROJ>::get()};       \
+        static const KernelSet proj_list[4] = {Launch<DT, NTR_F_LIST | NTR_F_PROJ>::get(), Launch<DT, 1 | NTR_F_LIST | NTR_F_PROJ>::get(), \
+                                               Launch<DT, 2 | NTR_F_LIST | NTR_F_PROJ>::get(), Launch<DT, 3 | NTR_F_LIST | NTR_F_PROJ>::get()}; \
+        if (flags & NTR_F_PROJ)                                                                         \
+            return (flags & NTR_F_LIST) ? &proj_list[flags & 3] : (flags & NTR_F_AOV) ? &proj_aovs[flags & 3] : &proj_views[flags & 3]; \
         static const KernelSet ss[4] = {Launch<DT, NTR_F_SS>::get(), Launch<DT, 1 | NTR_F_SS>::get(),   \
                                         Launch<DT, 2 | NTR_F_SS>::get(), Launch<DT, 3 | NTR_F_SS>::get()}; \
         if (flags & NTR_F_SS) return &ss[flags & 3];                                                     \

@@ -1489,9 +1489,57 @@ NTR_HD void primary_ray_of(const SceneDev &s, const CameraDev &cam, float fovI, 
     NTR_UNROLL
     for (int i = 0; i < D; ++i) dir[i] /= len;
 }
+
+// ---- projections (ntr_scene_set_projection; no counterpart in the reference) ----------------------------------------
+// The parameter of projection `kind` for a view of half width half_w: k = h / half_w (orthographic: scene units per pixel)
+// or a = alpha / (2 * half_w) (equirectangular: radians per pixel), in float like fovI.  At factor s the view's half_w is
+// s times the plain one, so k and a scale by 1/s exactly when s is a power of two.
+NTR_HD float projection_k(int kind, float param, float half_w) {
+    return kind == NTR_PROJ_ORTHOGRAPHIC ? param / half_w : param / (2.0f * half_w);
+}
+// pixel (x, y) of a view under an orthographic (kind 1) or equirectangular (kind 2) projection with parameter k
 template <int DT>
+NTR_HD void projected_ray_of(const SceneDev &s, const CameraDev &cam, int kind, float k, float half_w, float half_h, int x, int y,
+                             float *o, float *dir) {
+    const int D = NTR_D(DT, s);
+    const float u = k * ((float)x - half_w), v = k * ((float)y - half_h);
+    float sq = 0;
+    if (kind == NTR_PROJ_ORTHOGRAPHIC) {
+    NTR_UNROLL
+        for (int i = 0; i < D; ++i) {
+            o[i] = cam.origin[i] + cam.right[i] * u - cam.up[i] * v;
+            dir[i] = cam.fwd[i];
+            sq += dir[i] * dir[i];
+        }
+    } else {
+        const float st = sinf(u), ct = cosf(u), sp = sinf(v), cp = cosf(v);
+    NTR_UNROLL
+        for (int i = 0; i < D; ++i) {
+            o[i] = cam.origin[i];
+            dir[i] = cp * (st * cam.right[i] + ct * cam.fwd[i]) - sp * cam.up[i];
+            sq += dir[i] * dir[i];
+        }
+    }
+    const float len = sqrtf(sq);
+    NTR_UNROLL
+    for (int i = 0; i < D; ++i) dir[i] /= len;
+}
+// The primary ray of pixel (x, y): PROJ (the NTR_F_PROJ builds and camera_rays_kernel) switches on the projection kind at run
+// time; without it the code is the pinhole's alone.
+template <int DT, bool PROJ>
+NTR_HD void primary_ray_at(const SceneDev &s, const CameraDev &cam, int proj, float proj_k, float fovI, float half_w, float half_h,
+                           int x, int y, float *o, float *dir) {
+    if constexpr (PROJ) {
+        if (proj != NTR_PROJ_PERSPECTIVE) {
+            projected_ray_of<DT>(s, cam, proj, proj_k, half_w, half_h, x, y, o, dir);
+            return;
+        }
+    }
+    primary_ray_of<DT>(s, cam, fovI, half_w, half_h, x, y, o, dir);
+}
+template <int DT, bool PROJ = false>
 NTR_HD void primary_ray(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, float *o, float *dir) {
-    primary_ray_of<DT>(s, cam, f.fovI, f.half_w, f.half_h, x, y, o, dir);
+    primary_ray_at<DT, PROJ>(s, cam, f.proj, f.proj_k, f.fovI, f.half_w, f.half_h, x, y, o, dir);
 }
 
 // box_scene::calculate_color (tracer.hpp:101-114) with hypercube_intersects (:126-152) inlined:
@@ -1563,11 +1611,12 @@ template <int DT> struct PrimaryAov {
     HitRec hit;
     float n[DimCap<DT>::value];     // the normal that shades the hit; zeros on a miss
 };
-template <int DT, int FLAGS>
+template <int DT, int FLAGS, bool PROJ = false>
 NTR_HD void plain_primary_hit(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, PrimaryAov<DT> &a,
                               MailboxStore *ms);
 
-template <int DT, int FLAGS, typename EMIT, bool EXACT1 = false>
+// PROJ: the NTR_F_PROJ builds (primary_ray_at)
+template <int DT, int FLAGS, typename EMIT, bool EXACT1 = false, bool PROJ = false>
 NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, float *sum,
                            EMIT &emit, Counters &cnt, MailboxStore *ms, PrimaryAov<DT> *aov = nullptr) {
     constexpr int CAP = DimCap<DT>::value;
@@ -1585,7 +1634,7 @@ NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameD
         const int j = k / ss, i = k - j * ss;
         float o[CAP], dir[CAP];
         float c[3] = {0.0f, 0.0f, 0.0f};
-        primary_ray<DT>(s, cam, f, ss * x + i, ss * y + j, o, dir);
+        primary_ray<DT, PROJ>(s, cam, f, ss * x + i, ss * y + j, o, dir);
         const bool capture = aov && pow2 && k == 0;
         if (s.kind == NTR_SCENE_BOX) {
             box_color<DT>(s, o, dir, c, capture ? &aov->hit : nullptr, capture ? aov->n : nullptr);   // assigns the colour: weight it here
@@ -1597,19 +1646,19 @@ NTR_HD void ss_pixel_color(const SceneDev &s, const CameraDev &cam, const FrameD
         if (EXACT1 && ss == 1) { sum[0] = c[0]; sum[1] = c[1]; sum[2] = c[2]; }
         else { sum[0] = add_rn(sum[0], c[0]); sum[1] = add_rn(sum[1], c[1]); sum[2] = add_rn(sum[2], c[2]); }
     }
-    if (aov && !pow2) plain_primary_hit<DT, FLAGS>(s, cam, f, x, y, *aov, ms);
+    if (aov && !pow2) plain_primary_hit<DT, FLAGS, PROJ>(s, cam, f, x, y, *aov, ms);
 }
 
 // The hit of output pixel (x, y)'s plain primary ray, with the nearest-hit traversal of ray_color only: no shading, no
 // bounces, no counters.  a must hold ray_color's miss state (ss_pixel_color clears it).
-template <int DT, int FLAGS>
+template <int DT, int FLAGS, bool PROJ>
 NTR_HD void plain_primary_hit(const SceneDev &s, const CameraDev &cam, const FrameDev &f, int x, int y, PrimaryAov<DT> &a,
                               MailboxStore *ms) {
     constexpr int CAP = DimCap<DT>::value;
     constexpr int TF = FLAGS & ~NTR_F_COUNT;
     const int D = NTR_D(DT, s);
     float o[CAP], dir[CAP];
-    primary_ray_of<DT>(s, cam, f.aov_fovI, f.aov_half_w, f.aov_half_h, x, y, o, dir);
+    primary_ray_at<DT, PROJ>(s, cam, f.proj, f.aov_proj_k, f.aov_fovI, f.aov_half_w, f.aov_half_h, x, y, o, dir);
     if (s.kind == NTR_SCENE_BOX) {
         float c[3];
         box_color<DT>(s, o, dir, c, &a.hit, a.n);

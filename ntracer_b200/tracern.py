@@ -14,7 +14,7 @@ import numbers
 import numpy as np
 
 from . import _capi
-from .backend import DeviceGroup, DeviceScene, FLT_MAX
+from .backend import DeviceGroup, DeviceScene, FLT_MAX, projection_args
 from . import render as _render
 from .render import Color, LockedError, Material, Scene, _color_tuple, _encode_floats
 
@@ -968,6 +968,7 @@ class _LightList(list):
 class _SceneBase(Scene):
     supersampling = 1           # class-level default: scenes pickled before the attribute existed load with it
     supersampling_threshold = None      # likewise: off, and a scene that never sets it pickles as before
+    projection = ('perspective', None)  # likewise: the reference's pinhole camera
 
     def __init__(self, dimension):
         self.locked = 0
@@ -1027,6 +1028,20 @@ class _SceneBase(Scene):
         else:
             self.supersampling_threshold = float(threshold)
 
+    def set_projection(self, kind, param=None):
+        """The camera's projection (no counterpart in the reference, whose camera is a pinhole through fov): 'perspective'
+        (the default; param is ignored), 'orthographic' (param: half the view's width in scene units, required; fov is
+        ignored and the rays start on the image plane through the camera origin, so the camera must stand outside what it
+        should see) or 'equirectangular' (param: the horizontal field angle in radians, in (0, 2 pi], default 2 pi; fov is
+        ignored; a W x W/2 frame at 2 pi shows the whole sphere around the camera).  Every renderer and calculate_color
+        honour it, supersampling included.  scene.projection reads it back as (kind, param)."""
+        self._check_unlocked()
+        kind, param = projection_args(kind, param)
+        if kind == 'perspective':
+            self.__dict__.pop('projection', None)
+        else:
+            self.projection = (kind, param)
+
     # ---- backend ----
     def _device_scene(self):
         raise NotImplementedError
@@ -1050,6 +1065,8 @@ class _SceneBase(Scene):
             dev.set_supersampling(self.supersampling)
         if getattr(dev, 'supersampling_threshold', None) != self.supersampling_threshold:
             dev.set_supersampling_threshold(self.supersampling_threshold)
+        if getattr(dev, 'projection', ('perspective', None)) != self.projection:
+            dev.set_projection(*self.projection)
         return dev
 
     def calculate_color(self, x, y, width, height):
